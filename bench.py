@@ -3,6 +3,7 @@
 XYB->linear) on B200, with the roofline of the dominant kernel and the CPU restatement timed beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 8k|batch2048|split16k]
+                    [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one batch of synthetic post-entropy frame state (SURVEY.md 8(d)).
   8k        (default) one 7680x4320 frame per GPU, mixed varblocks DCT8..DCT256+AFV, gab on, EPF 3 iterations; N GPUs
@@ -13,6 +14,11 @@ A "step" = one pass of the hot path over one batch of synthetic post-entropy fra
   split16k  one 16384x16384 frame split by group rows over the N GPUs, 7 halo rows exchanged with NCCL (strong scaling)
 Prints ONE JSON line on rank 0.  Under torchrun one process per GPU; barrier + synchronize around the timed region,
 device time by CUDA events, max over ranks.
+
+--dump-outputs DIR writes the float32 linear planes the last timed step produced (what the caller of the timed entry point
+receives) as DIR/planes.npy, shape (3, rows, width); under torchrun each rank writes DIR/planes_rank<R>.npy.  Inputs are
+drawn from fixed seeds, so two builds run with the same arguments can be compared file for file.  Outputs larger than
+64 MB in all are cut to a sample of whole rows drawn with a fixed seed (the same rows for the same shape).
 """
 import argparse
 import json
@@ -31,6 +37,8 @@ BYTES_PER_PX = 24.35      # SURVEY.md 8(d): 12 coeff + 12 out + 0.1875 LF + 0.15
 BYTES_PER_PX_K2 = 24.13   # stage 2 alone: XYB in, linear out, sigma maps
 METRIC = "reconstructed MP/s (VarDCT dequant->XYB)"
 BATCH_FRAMES = 16         # frames per GPU per step of the batch2048 workload
+DUMP_BYTES = 64 * 10**6   # --dump-outputs: at most this much in all, .npy headers included
+DUMP_SEED = 0x4A584C00    # --dump-outputs: which rows a sample keeps
 
 
 def peaks():
@@ -83,6 +91,24 @@ def make_inputs(W, H, seed, epf_iters, oracle_tables=False, survey_spec=False):
     return p, st, qw, qo
 
 
+def dump_planes(dirname, name, planes, parts=1):
+    """--dump-outputs: planes (3, rows, width), a device tensor or a numpy array, as float32 to dirname/name.npy; when that
+    would pass DUMP_BYTES / parts, a sample of whole rows drawn with DUMP_SEED, kept in increasing order."""
+    rows, width = planes.shape[1], planes.shape[2]
+    keep = min(rows, (DUMP_BYTES // parts - 4096) // (3 * width * 4))     # 4096: room for the .npy header
+    if keep < rows:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rows, keep, replace=False))
+        if isinstance(planes, np.ndarray):
+            planes = planes[:, idx]
+        else:
+            import torch
+            planes = planes[:, torch.from_numpy(idx).to(planes.device)]
+    if not isinstance(planes, np.ndarray):
+        planes = planes.cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(planes, dtype=np.float32))
+
+
 def cpu_baseline(nthreads, sample=(2048, 2048), epf_iters=3, reps=1):
     """The CPU restatement of jxlatte's algorithm (oracle 'port'; not the JVM) on a bounded sample of the workload."""
     from oracle import oracle
@@ -112,8 +138,10 @@ def run_reference(args):
     steps = max(1, args.steps)
     t0 = time.perf_counter()
     for _ in range(steps):
-        oracle.vardct_reconstruct(p, st, nthreads=cores)
+        planes = oracle.vardct_reconstruct(p, st, nthreads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_planes(args.dump_outputs, "planes", planes)
     v = W * H * steps / 1e6 / dt
     t0 = time.perf_counter()
     p1, st1, _, _ = make_inputs(1024, 1024, 0x4A584C00 + 79, iters, oracle_tables=True)
@@ -302,6 +330,9 @@ def run_ours(args):
     if sampler:
         sampler.stop_flag = True
         sampler.join(timeout=3)
+    if args.dump_outputs:       # before the stage timings below write into the same planes
+        out = (wl.stack if wl.stack is not None else wl.first)["out"]
+        dump_planes(args.dump_outputs, "planes" if world == 1 else "planes_rank%d" % rank, out, world)
     value = wl.px_per_step_all * args.steps / 1e6 / (ms_max / 1e3)
 
     # ---- stage timing for the roofline of the dominant kernel (rank 0, same process, CUDA events on the same stream) ----
@@ -545,7 +576,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="8k", choices=["8k", "batch2048", "split16k"])
     ap.add_argument("--no-sub-records", action="store_true", help="skip the batch2048 / split16k sub-records of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the planes of the last timed step to DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
