@@ -84,6 +84,16 @@ SYMBOLS = {
     "jxlb200_lf_dequant": (_i32, [_vp, _i32, _i32, _vp, C.c_float, C.c_float, _i32, _i32, _P3, _vp, _P3]),
     "jxlb200_blend_batch": (_i32, [_vp, _i32, C.POINTER(_vp), _vp, _vp, _vp, _i32, _vp]),
     "jxlb200_blend": (_i32, [_vp, _vp, _i32, _i32, _vp, C.c_int64, _vp, C.c_int64, _vp, C.c_int64, _vp, C.c_int64, _vp, C.c_int64]),
+    "jxlb200_lf_dequant_dev": (_i32, [_vp, _i32, _i32, _vp, C.c_float, C.c_float, _i32, _i32, _P3, _vp, _P3]),
+    "jxlb200_restore_uniform_dev": (_i32, [_vp, _FP, C.c_float, _P3, _P3]),
+    "jxlb200_color_transform_dev": (_i32, [_vp, _FP, _P3, _P3]),
+    "jxlb200_upsample_dev": (_i32, [_vp, _vp, _i32, _i32, _i32, _vp, _vp]),
+    "jxlb200_noise_dev": (_i32, [_vp, _P3, _i32, _i32, _i32, C.c_int64, _vp, C.c_float, C.c_float]),
+    "jxlb200_splines_dev": (_i32, [_vp, _P3, _i32, _i32, _i32, _vp, _vp, _vp, _i32, C.c_float, C.c_float]),
+    "jxlb200_blend_batch_dev": (_i32, [_vp, _i32, C.POINTER(_vp), _vp, _vp, _i32, _vp]),
+    "jxlb200_pack_samples_dev": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
+    "jxlb200_cast_to_float_dev": (_i32, [_vp, _vp, C.c_int64, C.c_float, _vp]),
+    "jxlb200_modular_xyb_dev": (_i32, [_vp, _P3, C.c_int64, _vp, _P3]),
 }
 
 

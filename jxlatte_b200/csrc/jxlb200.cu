@@ -24,6 +24,7 @@
 #include "k6_subsample.cuh"
 #include "k7_blend.cuh"
 #include "k8_features.cuh"
+#include "k9_device.cuh"
 #include "splines_host.cuh"
 #include "qm_tables.cuh"
 #include "split_nccl.cuh"
@@ -84,6 +85,8 @@ struct jxlb200_ctx {
     DevBuf packed;          // interleaved 8/16-bit samples of jxlb200_vardct_reconstruct_packed
     DevBuf blend;           // five compact rectangles of jxlb200_blend
     DevBuf sub, sub_maps;   // chroma-subsampled frames: per-channel planes + scratch, strided block maps
+    DevBuf dtab;            // small host tables of the feature calls (upsampling weights, spline arcs, LF extraPrecision)
+    DevBuf feat;            // scratch of the feature calls (noise samples)
     DevTables tab;
 
     int fail(int code, const char *what, cudaError_t e = cudaSuccess) {
@@ -591,7 +594,7 @@ void jxlb200_destroy(jxlb200_ctx *ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     DevBuf *all[] = {&ctx->sched, &ctx->items, &ctx->gate, &ctx->wraw, &ctx->woff, &ctx->wexp, &ctx->cosbig, &ctx->lut8, &ctx->sigma, &ctx->flags,
-                     &ctx->mid, &ctx->pp[0], &ctx->pp[1], &ctx->in_q, &ctx->in_q16, &ctx->in_lf, &ctx->in_maps, &ctx->out_planes, &ctx->mod, &ctx->sub, &ctx->sub_maps, &ctx->blend, &ctx->packed, &ctx->split_xyb, &ctx->split_maps, &ctx->pack_thr[0], &ctx->pack_thr[1], &ctx->pack_thr[2], &ctx->pack_thr[3]};
+                     &ctx->mid, &ctx->pp[0], &ctx->pp[1], &ctx->in_q, &ctx->in_q16, &ctx->in_lf, &ctx->in_maps, &ctx->out_planes, &ctx->mod, &ctx->sub, &ctx->sub_maps, &ctx->dtab, &ctx->feat, &ctx->blend, &ctx->packed, &ctx->split_xyb, &ctx->split_maps, &ctx->pack_thr[0], &ctx->pack_thr[1], &ctx->pack_thr[2], &ctx->pack_thr[3]};
     for (DevBuf *b : all) b->release();
     if (ctx->comm && nccl_api().ok) nccl_api().CommDestroy(ctx->comm);
     if (ctx->comm_stream) cudaStreamDestroy(ctx->comm_stream);
@@ -1339,17 +1342,23 @@ int32_t jxlb200_vardct_invert(jxlb200_ctx *ctx, const jxlb200_frame_params *p,
     return stage_out_planes(ctx, dout, sizeof(float) * npx, xyb);
 }
 
-// one restoration stage on host planes: mode 0 Gaborish only, 1 EPF only, 2 colour only
+// one restoration stage on device planes: mode 0 Gaborish only, 1 EPF only, 2 colour only (what the host form and the _dev form share)
+static int stage_enqueue(jxlb200_ctx *ctx, const jxlb200_frame_params *p, int mode, const float *const din[3],
+                         const int32_t *hf_mul, const int32_t *sharp, float *const dout[3]) {
+    jxlb200_frame_params q = *p;
+    q.gab = mode == 0 ? 1 : 0;
+    q.epf_iters = mode == 1 ? p->epf_iters : 0;
+    q.color_mode = mode == 2 ? p->color_mode : 0;
+    return restore_dev(ctx, &q, nullptr, din, p->width, hf_mul, sharp, dout);
+}
+
+// one restoration stage on host planes: upload, stage_enqueue, download
 static int host_stage(jxlb200_ctx *ctx, const jxlb200_frame_params *p, int mode, const float *const in[3],
                       const int32_t *hf_mul, const int32_t *sharp, float *const out[3]) {
     int rc = check_params(ctx, p);
     if (rc) return rc;
     if (!in || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    jxlb200_frame_params q = *p;
-    q.gab = mode == 0 ? 1 : 0;
-    q.epf_iters = mode == 1 ? p->epf_iters : 0;
-    q.color_mode = mode == 2 ? p->color_mode : 0;
     const size_t npx = (size_t)p->width * p->height;
     void *din[3];
     if ((rc = stage_in_planes(ctx, ctx->in_q, (const void *const *)in, sizeof(float) * npx, din))) return rc;
@@ -1361,14 +1370,13 @@ static int host_stage(jxlb200_ctx *ctx, const jxlb200_frame_params *p, int mode,
     }
     CUDA_TRY(ctx, ctx->out_planes.ensure(sizeof(float) * 3 * npx));
     float *dout[3] = {ctx->out_planes.as<float>(), ctx->out_planes.as<float>() + npx, ctx->out_planes.as<float>() + 2 * npx};
-    rc = restore_dev(ctx, &q, nullptr, (const float *const *)din, p->width, M.hf, M.sharp, dout);
+    rc = stage_enqueue(ctx, p, mode, (const float *const *)din, M.hf, M.sharp, dout);
     if (rc) return rc;
     return stage_out_planes(ctx, dout, sizeof(float) * npx, out);
 }
 
 // Gaborish + EPF of a Modular-encoded frame (Frame.decodeFrame :457-461 with header.encoding == MODULAR): one sigma for the frame
-int32_t jxlb200_restore_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular,
-    const float *const in[3], float *const out[3]) {
+static int check_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular, const void *in, const void *out) {
     if (!ctx) return JXLB200_E_ARG;
     if (!p || !in || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
     // a Modular frame has its own size, not a multiple of 8; sizes the tile kernel does not take go through the staged kernels
@@ -1377,29 +1385,54 @@ int32_t jxlb200_restore_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p,
         return ctx->fail(JXLB200_E_UNSUPPORTED, "filters on a frame narrower than 4 pixels (mirrorCoordinate reflects more than once)");
     if (p->epf_iters < 0 || p->epf_iters > 3) return ctx->fail(JXLB200_E_ARG, "epf_iters outside 0..3");
     if (!(epf_sigma_for_modular == epf_sigma_for_modular)) return ctx->fail(JXLB200_E_ARG, "sigma is NaN");
-    int rc = 0;
+    return 0;
+}
+
+static int restore_uniform_enqueue(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular,
+                                   const float *const din[3], float *const dout[3]) {
+    const size_t npx = (size_t)p->width * p->height;
+    if (!p->gab && p->epf_iters == 0 && p->color_mode == 0) {
+        for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(dout[c], din[c], sizeof(float) * npx, cudaMemcpyDeviceToDevice, ctx->stream));
+        return 0;
+    }
+    ctx->uniform_sigma = true;
+    ctx->uniform_inv_sigma = 1.0f / epf_sigma_for_modular;        // Frame.java:574
+    // hf_mul / sharpness are not read in this mode; any non-NULL pointers satisfy the argument checks below
+    const int rc = restore_dev(ctx, p, nullptr, din, p->width, (const int32_t *)din[0], (const int32_t *)din[0], dout);
+    ctx->uniform_sigma = false;
+    return rc;
+}
+
+int32_t jxlb200_restore_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular,
+    const float *const in[3], float *const out[3]) {
+    int rc = check_uniform(ctx, p, epf_sigma_for_modular, in, out);
+    if (rc) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t npx = ((size_t)p->width * p->height + 3) & ~(size_t)3;      // planes stay 16-byte aligned
-    void *din[3];
+    const float *din[3];
     CUDA_TRY(ctx, ctx->in_q.ensure(3 * sizeof(float) * npx));
     for (int c = 0; c < 3; c++) {
         if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
         din[c] = ctx->in_q.as<float>() + c * npx;
-        CUDA_TRY(ctx, cudaMemcpyAsync(din[c], in[c], sizeof(float) * (size_t)p->width * p->height, cudaMemcpyHostToDevice, ctx->stream));
+        CUDA_TRY(ctx, cudaMemcpyAsync((void *)din[c], in[c], sizeof(float) * (size_t)p->width * p->height, cudaMemcpyHostToDevice, ctx->stream));
     }
     CUDA_TRY(ctx, ctx->out_planes.ensure(sizeof(float) * 3 * npx));
     float *dout[3] = {ctx->out_planes.as<float>(), ctx->out_planes.as<float>() + npx, ctx->out_planes.as<float>() + 2 * npx};
-    if (!p->gab && p->epf_iters == 0 && p->color_mode == 0) {
-        for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(dout[c], din[c], sizeof(float) * npx, cudaMemcpyDeviceToDevice, ctx->stream));
-    } else {
-        ctx->uniform_sigma = true;
-        ctx->uniform_inv_sigma = 1.0f / epf_sigma_for_modular;        // Frame.java:574
-        // hf_mul / sharpness are not read in this mode; any non-NULL pointers satisfy the argument checks below
-        rc = restore_dev(ctx, p, nullptr, (const float *const *)din, p->width, (const int32_t *)din[0], (const int32_t *)din[0], dout);
-        ctx->uniform_sigma = false;
-        if (rc) return rc;
-    }
+    if ((rc = restore_uniform_enqueue(ctx, p, epf_sigma_for_modular, din, dout))) return rc;
     return stage_out_planes(ctx, dout, sizeof(float) * (size_t)p->width * p->height, out);
+}
+
+int32_t jxlb200_restore_uniform_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular,
+    const float *const in[3], float *const out[3]) {
+    int rc = check_uniform(ctx, p, epf_sigma_for_modular, in, out);
+    if (rc) return rc;
+    for (int c = 0; c < 3; c++) {
+        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+        for (int d = 0; d < 3; d++)
+            if (in[c] == out[d]) return ctx->fail(JXLB200_E_ARG, "in-place restore is not allowed");
+    }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return restore_uniform_enqueue(ctx, p, epf_sigma_for_modular, in, out);
 }
 
 int32_t jxlb200_gaborish(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float *const in[3], float *const out[3]) {
@@ -1411,6 +1444,18 @@ int32_t jxlb200_epf(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float
 }
 int32_t jxlb200_color_transform(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float *const in[3], float *const out[3]) {
     return host_stage(ctx, p, 2, in, nullptr, nullptr, out);
+}
+int32_t jxlb200_color_transform_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float *const in[3], float *const out[3]) {
+    int rc = check_params(ctx, p);
+    if (rc) return rc;
+    if (!in || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
+    for (int c = 0; c < 3; c++) {
+        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+        for (int d = 0; d < 3; d++)
+            if (in[c] == out[d]) return ctx->fail(JXLB200_E_ARG, "in-place colour transform is not allowed");
+    }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return stage_enqueue(ctx, p, 2, in, nullptr, nullptr, out);
 }
 
 // ---- Modular ----
@@ -1585,13 +1630,11 @@ int32_t jxlb200_blend(jxlb200_ctx *ctx, const jxlb200_blend_op *op, int32_t h, i
 // rectangle touches), every rectangle of every channel is blended there in the order given -- later items see what earlier ones
 // wrote, as blendFrame / computePatches do (J/JXLCodestreamDecoder.java:212-254, 415-537) -- and the written planes come back once.
 // patches-lossless.jxl: ~2000 rectangles, two PCIe round trips instead of ~8000. ----
-int32_t jxlb200_blend_batch(jxlb200_ctx *ctx, int32_t n_planes, void *const planes[], const int32_t plane_h[], const int32_t plane_w[],
-    const int32_t writable[], int32_t n_items, const jxlb200_blend_item *items) {
-    if (!ctx) return JXLB200_E_ARG;
-    if (n_planes < 1 || n_planes > 64 || !planes || !plane_h || !plane_w || !writable || n_items < 0 || (n_items > 0 && !items))
-        return ctx->fail(JXLB200_E_ARG, "bad arguments");
-    if (n_items == 0) return 0;
-    std::vector<int> lo(n_planes, 1 << 30), hi(n_planes, -1);
+// Checks the items against the planes and records the rows [lo, hi) of each plane that some rectangle touches.
+static int blend_items_check(jxlb200_ctx *ctx, int32_t n_planes, void *const planes[], const int32_t plane_h[], const int32_t plane_w[],
+    const int32_t writable[], int32_t n_items, const jxlb200_blend_item *items, std::vector<int> &lo, std::vector<int> &hi) {
+    lo.assign(n_planes, 1 << 30);
+    hi.assign(n_planes, -1);
     for (int k = 0; k < n_items; k++) {
         const jxlb200_blend_item &it = items[k];
         if (it.op.mode < 1 || it.op.mode > 4) return ctx->fail(JXLB200_E_STREAM, "Illegal blend mode");
@@ -1609,8 +1652,46 @@ int32_t jxlb200_blend_batch(jxlb200_ctx *ctx, int32_t n_planes, void *const plan
                 return ctx->fail(JXLB200_E_STREAM, "blend rectangle outside its buffer");
             lo[pl] = std::min(lo[pl], it.y[r]); hi[pl] = std::max(hi[pl], it.y[r] + it.h);
         }
-        if (!writable[it.plane[0]]) return ctx->fail(JXLB200_E_ARG, "blend item writes a plane not marked writable");
+        if (writable && !writable[it.plane[0]]) return ctx->fail(JXLB200_E_ARG, "blend item writes a plane not marked writable");
     }
+    return 0;
+}
+
+// One k7_blend launch per item, in order.  row0[pl] is the device address of row 0 of plane pl (plane_w[pl] samples per row); only
+// rows hi[pl] > lo[pl] of a plane are dereferenced.
+static int blend_items_enqueue(jxlb200_ctx *ctx, int32_t n_planes, const std::vector<uintptr_t> &row0, const std::vector<int> &hi,
+    const int32_t plane_w[], int32_t n_items, const jxlb200_blend_item *items) {
+    cudaStream_t st = ctx->stream;
+    for (int k = 0; k < n_items; k++) {
+        const jxlb200_blend_item &it = items[k];
+        BlendArgs A;
+        A.mode = it.op.mode; A.is_int = it.op.is_int; A.is_alpha = it.op.is_alpha; A.has_extra = it.op.has_extra; A.clamp = it.op.clamp; A.premult = it.op.premult;
+        A.h = it.h; A.w = it.w;
+        auto at = [&](int r) -> char * {
+            const int pl = it.plane[r];
+            if (pl < 0 || pl >= n_planes || hi[pl] < 0) return nullptr;
+            return (char *)(row0[pl] + ((size_t)it.y[r] * plane_w[pl] + it.x[r]) * 4);
+        };
+        auto pitch = [&](int r) -> long long { const int pl = it.plane[r]; return (pl < 0 || pl >= n_planes) ? 1 : plane_w[pl]; };
+        A.out = at(0); A.a = at(1); A.b = at(2); A.fa = (const float *)at(3); A.ra = (const float *)at(4);
+        A.pout = pitch(0); A.pa = pitch(1); A.pb = pitch(2); A.pfa = pitch(3); A.pra = pitch(4);
+        const long long n = (long long)it.h * it.w;
+        k7_blend<<<(int)std::min<long long>(ctx->sms * 8, (n + 255) / 256), 256, 0, st>>>(A);
+        ctx->launches++;
+    }
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+
+int32_t jxlb200_blend_batch(jxlb200_ctx *ctx, int32_t n_planes, void *const planes[], const int32_t plane_h[], const int32_t plane_w[],
+    const int32_t writable[], int32_t n_items, const jxlb200_blend_item *items) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (n_planes < 1 || n_planes > 64 || !planes || !plane_h || !plane_w || !writable || n_items < 0 || (n_items > 0 && !items))
+        return ctx->fail(JXLB200_E_ARG, "bad arguments");
+    if (n_items == 0) return 0;
+    std::vector<int> lo, hi;
+    int rc = blend_items_check(ctx, n_planes, planes, plane_h, plane_w, writable, n_items, items, lo, hi);
+    if (rc) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     std::vector<size_t> off(n_planes, 0);
     size_t total = 0;
@@ -1622,28 +1703,14 @@ int32_t jxlb200_blend_batch(jxlb200_ctx *ctx, int32_t n_planes, void *const plan
     CUDA_TRY(ctx, ctx->blend.ensure(total));
     cudaStream_t st = ctx->stream;
     char *base = (char *)ctx->blend.p;
+    std::vector<uintptr_t> row0(n_planes, 0);
     for (int pl = 0; pl < n_planes; pl++)
-        if (hi[pl] >= 0)
+        if (hi[pl] >= 0) {
+            row0[pl] = (uintptr_t)(base + off[pl]) - (uintptr_t)lo[pl] * plane_w[pl] * 4;   // the staged rows start at row lo[pl]
             CUDA_TRY(ctx, cudaMemcpyAsync(base + off[pl], (const char *)planes[pl] + (size_t)lo[pl] * plane_w[pl] * 4,
                                           (size_t)(hi[pl] - lo[pl]) * plane_w[pl] * 4, cudaMemcpyHostToDevice, st));
-    for (int k = 0; k < n_items; k++) {
-        const jxlb200_blend_item &it = items[k];
-        BlendArgs A;
-        A.mode = it.op.mode; A.is_int = it.op.is_int; A.is_alpha = it.op.is_alpha; A.has_extra = it.op.has_extra; A.clamp = it.op.clamp; A.premult = it.op.premult;
-        A.h = it.h; A.w = it.w;
-        auto at = [&](int r) -> char * {
-            const int pl = it.plane[r];
-            if (pl < 0 || pl >= n_planes || hi[pl] < 0) return nullptr;
-            return base + off[pl] + ((size_t)(it.y[r] - lo[pl]) * plane_w[pl] + it.x[r]) * 4;
-        };
-        auto pitch = [&](int r) -> long long { const int pl = it.plane[r]; return (pl < 0 || pl >= n_planes) ? 1 : plane_w[pl]; };
-        A.out = at(0); A.a = at(1); A.b = at(2); A.fa = (const float *)at(3); A.ra = (const float *)at(4);
-        A.pout = pitch(0); A.pa = pitch(1); A.pb = pitch(2); A.pfa = pitch(3); A.pra = pitch(4);
-        const long long n = (long long)it.h * it.w;
-        k7_blend<<<(int)std::min<long long>(ctx->sms * 8, (n + 255) / 256), 256, 0, st>>>(A);
-        ctx->launches++;
-    }
-    CUDA_TRY(ctx, cudaGetLastError());
+        }
+    if ((rc = blend_items_enqueue(ctx, n_planes, row0, hi, plane_w, n_items, items))) return rc;
     for (int pl = 0; pl < n_planes; pl++)
         if (hi[pl] >= 0 && writable[pl])
             CUDA_TRY(ctx, cudaMemcpyAsync((char *)planes[pl] + (size_t)lo[pl] * plane_w[pl] * 4, base + off[pl],
@@ -1652,39 +1719,75 @@ int32_t jxlb200_blend_batch(jxlb200_ctx *ctx, int32_t n_planes, void *const plan
     return 0;
 }
 
+int32_t jxlb200_blend_batch_dev(jxlb200_ctx *ctx, int32_t n_planes, void *const planes[], const int32_t plane_h[], const int32_t plane_w[],
+    int32_t n_items, const jxlb200_blend_item *items) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (n_planes < 1 || n_planes > 64 || !planes || !plane_h || !plane_w || n_items < 0 || (n_items > 0 && !items))
+        return ctx->fail(JXLB200_E_ARG, "bad arguments");
+    if (n_items == 0) return 0;
+    std::vector<int> lo, hi;
+    int rc = blend_items_check(ctx, n_planes, planes, plane_h, plane_w, nullptr, n_items, items, lo, hi);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    std::vector<uintptr_t> row0(n_planes, 0);
+    for (int pl = 0; pl < n_planes; pl++) row0[pl] = (uintptr_t)planes[pl];
+    return blend_items_enqueue(ctx, n_planes, row0, hi, plane_w, n_items, items);
+}
 
-// ---- k x k upsampling of one float channel on host buffers (k8_features.cuh) ----
-int32_t jxlb200_upsample(jxlb200_ctx *ctx, const float *in, int32_t h, int32_t w, int32_t k, const float *weights, float *out) {
+
+// ---- k x k upsampling of one float channel (k8_features.cuh) ----
+static int upsample_check(jxlb200_ctx *ctx, const void *in, int32_t h, int32_t w, int32_t k, const float *weights, const void *out) {
     if (!ctx) return JXLB200_E_ARG;
     if (!in || !weights || !out || h <= 0 || w <= 0) return ctx->fail(JXLB200_E_ARG, "NULL pointer or empty channel");
     if (k != 2 && k != 4 && k != 8) return ctx->fail(JXLB200_E_ARG, "upsampling factor must be 2, 4 or 8 (FrameHeader.java:121-123)");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return 0;
+}
+static int upsample_enqueue(jxlb200_ctx *ctx, const float *d_in, int32_t h, int32_t w, int32_t k, const float *weights, float *d_out) {
     const size_t n = (size_t)h * w, nw = (size_t)k * k * 25;
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * (n + n * k * k + nw)));
-    float *d_in = ctx->blend.as<float>(), *d_out = d_in + n, *d_w = d_out + n * k * k;
+    CUDA_TRY(ctx, ctx->dtab.ensure(sizeof(float) * nw));
+    float *d_w = ctx->dtab.as<float>();
     cudaStream_t st = ctx->stream;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_in, in, sizeof(float) * n, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(d_w, weights, sizeof(float) * nw, cudaMemcpyHostToDevice, st));
     k8_upsample<<<min(ctx->sms * 8, ceil_div((int)std::min<size_t>(n, 1u << 30), 128)), 128, sizeof(float) * nw, st>>>(d_in, h, w, k, d_w, d_out);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+int32_t jxlb200_upsample(jxlb200_ctx *ctx, const float *in, int32_t h, int32_t w, int32_t k, const float *weights, float *out) {
+    int rc = upsample_check(ctx, in, h, w, k, weights, out);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t n = (size_t)h * w;
+    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * (n + n * k * k)));
+    float *d_in = ctx->blend.as<float>(), *d_out = d_in + n;
+    cudaStream_t st = ctx->stream;
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_in, in, sizeof(float) * n, cudaMemcpyHostToDevice, st));
+    if ((rc = upsample_enqueue(ctx, d_in, h, w, k, weights, d_out))) return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, sizeof(float) * n * k * k, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     return 0;
 }
+int32_t jxlb200_upsample_dev(jxlb200_ctx *ctx, const float *in, int32_t h, int32_t w, int32_t k, const float *weights, float *out) {
+    int rc = upsample_check(ctx, in, h, w, k, weights, out);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return upsample_enqueue(ctx, in, h, w, k, weights, out);
+}
 
 
-// ---- noise synthesis on host planes (k8_features.cuh): Frame.initializeNoise + synthesizeNoise ----
-int32_t jxlb200_noise(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t group_dim, int64_t seed0,
-    const float lut[8], float base_corr_x, float base_corr_b) {
+// ---- noise synthesis (k8_features.cuh): Frame.initializeNoise + synthesizeNoise, in place on device planes ----
+static int noise_check(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t group_dim, const float *lut) {
     if (!ctx) return JXLB200_E_ARG;
     if (!planes || !planes[0] || !planes[1] || !planes[2] || !lut || h <= 0 || w <= 0) return ctx->fail(JXLB200_E_ARG, "NULL pointer or empty frame");
     if (group_dim != 128 && group_dim != 256 && group_dim != 512 && group_dim != 1024) return ctx->fail(JXLB200_E_ARG, "group_dim must be 128 << 0..3");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return 0;
+}
+static int noise_enqueue(jxlb200_ctx *ctx, float *const d_planes[3], int32_t h, int32_t w, int32_t group_dim, int64_t seed0,
+    const float lut[8], float base_corr_x, float base_corr_b) {
     const size_t n = (size_t)h * w;
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 6 * n));
+    CUDA_TRY(ctx, ctx->feat.ensure(sizeof(float) * 3 * n));
     NoiseArgs A;
-    for (int c = 0; c < 3; c++) { A.local[c] = ctx->blend.as<float>() + c * n; A.plane[c] = ctx->blend.as<float>() + (3 + c) * n; }
+    for (int c = 0; c < 3; c++) { A.local[c] = ctx->feat.as<float>() + c * n; A.plane[c] = d_planes[c]; }
     A.h = h; A.w = w; A.group_dim = group_dim;
     A.log_dim = group_dim == 128 ? 7 : group_dim == 256 ? 8 : group_dim == 512 ? 9 : 10;
     A.group_cols = ceil_div(w, group_dim);
@@ -1693,20 +1796,40 @@ int32_t jxlb200_noise(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32
     for (int i = 0; i < 8; i++) A.lut[i] = lut[i];
     A.base_x = base_corr_x; A.base_b = base_corr_b;
     cudaStream_t st = ctx->stream;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(A.plane[c], planes[c], sizeof(float) * n, cudaMemcpyHostToDevice, st));
     k8_noise_rng<<<ceil_div(A.num_groups * 8, 64), 64, 0, st>>>(A);
     k8_noise_apply<<<min(ctx->sms * 8, ceil_div((int)std::min<size_t>(n, 1u << 30), 256)), 256, 0, st>>>(A);
     ctx->launches += 2;
     CUDA_TRY(ctx, cudaGetLastError());
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(planes[c], A.plane[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+}
+int32_t jxlb200_noise(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t group_dim, int64_t seed0,
+    const float lut[8], float base_corr_x, float base_corr_b) {
+    int rc = noise_check(ctx, planes, h, w, group_dim, lut);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t n = (size_t)h * w;
+    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 3 * n));
+    float *d[3] = {ctx->blend.as<float>(), ctx->blend.as<float>() + n, ctx->blend.as<float>() + 2 * n};
+    cudaStream_t st = ctx->stream;
+    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(d[c], planes[c], sizeof(float) * n, cudaMemcpyHostToDevice, st));
+    if ((rc = noise_enqueue(ctx, d, h, w, group_dim, seed0, lut, base_corr_x, base_corr_b))) return rc;
+    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(planes[c], d[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     return 0;
 }
+int32_t jxlb200_noise_dev(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t group_dim, int64_t seed0,
+    const float lut[8], float base_corr_x, float base_corr_b) {
+    int rc = noise_check(ctx, planes, h, w, group_dim, lut);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return noise_enqueue(ctx, planes, h, w, group_dim, seed0, lut, base_corr_x, base_corr_b);
+}
 
 
-// ---- splines on host planes (splines_host.cuh + k8_splines): Frame.renderSplines ----
-int32_t jxlb200_splines(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t num_splines, const int32_t *npoints,
-    const int32_t *points, const int32_t *coeff, int32_t quant_adjust, float base_corr_x, float base_corr_b) {
+// ---- splines (splines_host.cuh + k8_splines): Frame.renderSplines, in place ----
+// Spline.computeCoeffs and the arcs of every spline, on the host (both forms)
+static int splines_arcs(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t num_splines, const int32_t *npoints,
+    const int32_t *points, const int32_t *coeff, int32_t quant_adjust, float base_corr_x, float base_corr_b, std::vector<SplineArcDev> &arcs) {
     if (!ctx) return JXLB200_E_ARG;
     if (!planes || !planes[0] || !planes[1] || !planes[2] || !npoints || !points || !coeff || h <= 0 || w <= 0 || num_splines < 0)
         return ctx->fail(JXLB200_E_ARG, "NULL pointer or empty frame");
@@ -1724,89 +1847,185 @@ int32_t jxlb200_splines(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int
             trk[3].c[i] = coeff[96 + i] * sa;
         }
     }
-    std::vector<SplineArcDev> arcs;
     const int32_t *pts = points;
     for (int s = 0; s < num_splines; s++) {
         if (npoints[s] < 1) return ctx->fail(JXLB200_E_ARG, "a spline needs at least one control point");
         splines_host::build(pts, npoints[s], trk, h, w, arcs);
         pts += 2 * npoints[s];
     }
-    if (arcs.empty()) return 0;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)h * w, abytes = sizeof(SplineArcDev) * arcs.size();
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 3 * n + abytes + 64));
-    float *d[3] = {ctx->blend.as<float>(), ctx->blend.as<float>() + n, ctx->blend.as<float>() + 2 * n};
-    SplineArcDev *d_arcs = (SplineArcDev *)(ctx->blend.as<char>() + ((sizeof(float) * 3 * n + 63) & ~(size_t)63));
+    return 0;
+}
+static int splines_enqueue(jxlb200_ctx *ctx, float *const d[3], int32_t h, int32_t w, const std::vector<SplineArcDev> &arcs) {
+    const size_t abytes = sizeof(SplineArcDev) * arcs.size();
+    CUDA_TRY(ctx, ctx->dtab.ensure(abytes));
+    SplineArcDev *d_arcs = ctx->dtab.as<SplineArcDev>();
     cudaStream_t st = ctx->stream;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(d[c], planes[c], sizeof(float) * n, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(d_arcs, arcs.data(), abytes, cudaMemcpyHostToDevice, st));
     k8_splines<<<dim3(ceil_div(w, 32), ceil_div(h, 8)), 256, 0, st>>>(d[0], d[1], d[2], h, w, d_arcs, (int)arcs.size(), (float)sqrt(0.125));
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+int32_t jxlb200_splines(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t num_splines, const int32_t *npoints,
+    const int32_t *points, const int32_t *coeff, int32_t quant_adjust, float base_corr_x, float base_corr_b) {
+    std::vector<SplineArcDev> arcs;
+    int rc = splines_arcs(ctx, planes, h, w, num_splines, npoints, points, coeff, quant_adjust, base_corr_x, base_corr_b, arcs);
+    if (rc || arcs.empty()) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t n = (size_t)h * w;
+    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 3 * n));
+    float *d[3] = {ctx->blend.as<float>(), ctx->blend.as<float>() + n, ctx->blend.as<float>() + 2 * n};
+    cudaStream_t st = ctx->stream;
+    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(d[c], planes[c], sizeof(float) * n, cudaMemcpyHostToDevice, st));
+    if ((rc = splines_enqueue(ctx, d, h, w, arcs))) return rc;
     for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(planes[c], d[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     return 0;
 }
+int32_t jxlb200_splines_dev(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t num_splines, const int32_t *npoints,
+    const int32_t *points, const int32_t *coeff, int32_t quant_adjust, float base_corr_x, float base_corr_b) {
+    std::vector<SplineArcDev> arcs;
+    int rc = splines_arcs(ctx, planes, h, w, num_splines, npoints, points, coeff, quant_adjust, base_corr_x, base_corr_b, arcs);
+    if (rc || arcs.empty()) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return splines_enqueue(ctx, planes, h, w, arcs);
+}
 
 
-// ---- LF coefficients on host planes (k8_lf_dequant): LFCoefficients' dequantisation + LF chroma-from-luma + adaptive smoothing ----
-int32_t jxlb200_lf_dequant(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float scaled_dequant[3], float k_x, float k_b,
-    int32_t cfl, int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, float *const out[3]) {
+// ---- LF coefficients (k8_lf_dequant): LFCoefficients' dequantisation + LF chroma-from-luma + adaptive smoothing ----
+static int lf_check(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float scaled_dequant[3], const int32_t *const lf_quant[3],
+    const uint8_t *extra_precision, float *const out[3]) {
     if (!ctx) return JXLB200_E_ARG;
     if (hb < 1 || wb < 1 || !scaled_dequant || !lf_quant || !extra_precision || !out) return ctx->fail(JXLB200_E_ARG, "bad arguments");
     for (int c = 0; c < 3; c++)
         if (!lf_quant[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)hb * wb;
-    const int gcols = (wb + 255) >> 8, ng = gcols * ((hb + 255) >> 8);
+    const int ng = ((wb + 255) >> 8) * ((hb + 255) >> 8);
     for (int g = 0; g < ng; g++)
         if (extra_precision[g] > 3) return ctx->fail(JXLB200_E_STREAM, "extraPrecision is a 2-bit field");
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 6 * n + ng + 64));
-    LfArgs A;
+    return 0;
+}
+static int lf_enqueue(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float scaled_dequant[3], float k_x, float k_b,
+    int32_t cfl, int32_t adaptive_smoothing, const int32_t *const d_q[3], const uint8_t *extra_precision, float *const d_out[3]) {
+    const size_t n = (size_t)hb * wb;
+    const int gcols = (wb + 255) >> 8, ng = gcols * ((hb + 255) >> 8);
+    CUDA_TRY(ctx, ctx->dtab.ensure(ng));
+    uint8_t *dep = ctx->dtab.as<uint8_t>();
     cudaStream_t st = ctx->stream;
-    for (int c = 0; c < 3; c++) {
-        int32_t *dq = ctx->blend.as<int32_t>() + c * n;
-        A.q[c] = dq;
-        A.out[c] = ctx->blend.as<float>() + (3 + c) * n;
-        A.sd[c] = scaled_dequant[c];
-        CUDA_TRY(ctx, cudaMemcpyAsync(dq, lf_quant[c], sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-    }
-    uint8_t *dep = ctx->blend.as<uint8_t>() + sizeof(float) * 6 * n;
     CUDA_TRY(ctx, cudaMemcpyAsync(dep, extra_precision, ng, cudaMemcpyHostToDevice, st));
+    LfArgs A;
+    for (int c = 0; c < 3; c++) { A.q[c] = d_q[c]; A.out[c] = d_out[c]; A.sd[c] = scaled_dequant[c]; }
     A.ep = dep; A.hb = hb; A.wb = wb; A.gcols = gcols; A.cfl = cfl ? 1 : 0; A.smooth = adaptive_smoothing ? 1 : 0; A.kx = k_x; A.kb = k_b;
     k8_lf_dequant<<<(int)std::min<size_t>((size_t)ctx->sms * 8, (n + 255) / 256), 256, 0, st>>>(A);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(out[c], A.out[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+}
+int32_t jxlb200_lf_dequant(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float scaled_dequant[3], float k_x, float k_b,
+    int32_t cfl, int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, float *const out[3]) {
+    int rc = lf_check(ctx, hb, wb, scaled_dequant, lf_quant, extra_precision, out);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t n = (size_t)hb * wb;
+    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 6 * n));
+    cudaStream_t st = ctx->stream;
+    const int32_t *dq[3];
+    float *dout[3];
+    for (int c = 0; c < 3; c++) {
+        dq[c] = ctx->blend.as<int32_t>() + c * n;
+        dout[c] = ctx->blend.as<float>() + (3 + c) * n;
+        CUDA_TRY(ctx, cudaMemcpyAsync((void *)dq[c], lf_quant[c], sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    }
+    if ((rc = lf_enqueue(ctx, hb, wb, scaled_dequant, k_x, k_b, cfl, adaptive_smoothing, dq, extra_precision, dout))) return rc;
+    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(out[c], dout[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     return 0;
 }
+int32_t jxlb200_lf_dequant_dev(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float scaled_dequant[3], float k_x, float k_b,
+    int32_t cfl, int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, float *const out[3]) {
+    int rc = lf_check(ctx, hb, wb, scaled_dequant, lf_quant, extra_precision, out);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return lf_enqueue(ctx, hb, wb, scaled_dequant, k_x, k_b, cfl, adaptive_smoothing, lf_quant, extra_precision, out);
+}
 
 
-// ---- PNG-ready samples from host planes (k8_pack_samples) ----
-int32_t jxlb200_pack_samples(jxlb200_ctx *ctx, const void *const planes[], const int32_t is_int[], const int32_t depth[],
-    int32_t n_channels, int32_t n_color, int32_t linear, int32_t h, int32_t w, int32_t bits, uint8_t *out) {
+// ---- PNG-ready samples (k8_pack_samples) ----
+static int pack_check(jxlb200_ctx *ctx, const void *const planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t n_channels, int32_t h, int32_t w, int32_t bits, const void *out) {
     if (!ctx) return JXLB200_E_ARG;
     if (!planes || !is_int || !depth || !out || n_channels < 1 || n_channels > 8 || h <= 0 || w <= 0) return ctx->fail(JXLB200_E_ARG, "bad arguments");
     if (bits != 8 && bits != 16) return ctx->fail(JXLB200_E_ARG, "PNG only supports 8 and 16 (PNGWriter.java:57-58)");
+    for (int c = 0; c < n_channels; c++)
+        if (!planes[c] || depth[c] < 1 || depth[c] > 31) return ctx->fail(JXLB200_E_ARG, "NULL plane or bad depth");
+    return 0;
+}
+static int pack_enqueue(jxlb200_ctx *ctx, const void *const d_planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t n_channels, int32_t n_color, int32_t linear, int32_t h, int32_t w, int32_t bits, int32_t layout, uint8_t *d_out) {
+    const size_t n = (size_t)h * w;
+    PackArgs A;
+    for (int c = 0; c < n_channels; c++) { A.plane[c] = d_planes[c]; A.is_int[c] = is_int[c]; A.depth[c] = depth[c]; }
+    A.n_channels = n_channels; A.n_color = n_color; A.linear = linear; A.h = h; A.w = w; A.bits = bits; A.layout = layout;
+    A.out = d_out;
+    k8_pack_samples<<<min(ctx->sms * 8, ceil_div((int)std::min<size_t>(n, 1u << 30), 256)), 256, 0, ctx->stream>>>(A);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+int32_t jxlb200_pack_samples(jxlb200_ctx *ctx, const void *const planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t n_channels, int32_t n_color, int32_t linear, int32_t h, int32_t w, int32_t bits, uint8_t *out) {
+    int rc = pack_check(ctx, planes, is_int, depth, n_channels, h, w, bits, out);
+    if (rc) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)h * w, obytes = n * n_channels * (bits > 8 ? 2 : 1);
     CUDA_TRY(ctx, ctx->blend.ensure(4 * n * n_channels + obytes + 64));
-    PackArgs A;
     cudaStream_t st = ctx->stream;
+    const void *d[8];
     for (int c = 0; c < n_channels; c++) {
-        if (!planes[c] || depth[c] < 1 || depth[c] > 31) return ctx->fail(JXLB200_E_ARG, "NULL plane or bad depth");
-        void *d = ctx->blend.as<char>() + 4 * n * c;
-        CUDA_TRY(ctx, cudaMemcpyAsync(d, planes[c], 4 * n, cudaMemcpyHostToDevice, st));
-        A.plane[c] = d; A.is_int[c] = is_int[c]; A.depth[c] = depth[c];
+        d[c] = ctx->blend.as<char>() + 4 * n * c;
+        CUDA_TRY(ctx, cudaMemcpyAsync((void *)d[c], planes[c], 4 * n, cudaMemcpyHostToDevice, st));
     }
-    A.n_channels = n_channels; A.n_color = n_color; A.linear = linear; A.h = h; A.w = w; A.bits = bits;
-    A.out = (unsigned char *)(ctx->blend.as<char>() + ((4 * n * n_channels + 63) & ~(size_t)63));
-    k8_pack_samples<<<min(ctx->sms * 8, ceil_div((int)std::min<size_t>(n, 1u << 30), 256)), 256, 0, st>>>(A);
+    uint8_t *d_out = (uint8_t *)(ctx->blend.as<char>() + ((4 * n * n_channels + 63) & ~(size_t)63));
+    if ((rc = pack_enqueue(ctx, d, is_int, depth, n_channels, n_color, linear, h, w, bits, 0, d_out))) return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, obytes, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    return 0;
+}
+int32_t jxlb200_pack_samples_dev(jxlb200_ctx *ctx, const void *const planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t n_channels, int32_t n_color, int32_t linear, int32_t h, int32_t w, int32_t bits, int32_t layout, uint8_t *out) {
+    int rc = pack_check(ctx, planes, is_int, depth, n_channels, h, w, bits, out);
+    if (rc) return rc;
+    if (layout != 0 && layout != 1) return ctx->fail(JXLB200_E_ARG, "layout must be 0 (PNG bytes) or 1 (planar samples)");
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return pack_enqueue(ctx, planes, is_int, depth, n_channels, n_color, linear, h, w, bits, layout, out);
+}
+
+
+// ---- glue of the frame loop on device buffers (k9_device.cuh) ----
+int32_t jxlb200_cast_to_float_dev(jxlb200_ctx *ctx, const int32_t *in, int64_t n, float scale, float *out) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!in || !out || n < 0) return ctx->fail(JXLB200_E_ARG, "NULL pointer or negative size");
+    if (n == 0) return 0;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    k9_cast_to_float<<<(int)std::min<long long>((long long)ctx->sms * 8, (n + 255) / 256), 256, 0, ctx->stream>>>(in, n, scale, out);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
-    CUDA_TRY(ctx, cudaMemcpyAsync(out, A.out, obytes, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    return 0;
+}
+
+int32_t jxlb200_modular_xyb_dev(jxlb200_ctx *ctx, const int32_t *const in[3], int64_t n, const float lf_dequant[3], float *const out[3]) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!in || !out || !lf_dequant || n < 0) return ctx->fail(JXLB200_E_ARG, "NULL pointer or negative size");
+    for (int c = 0; c < 3; c++)
+        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+    if (n == 0) return 0;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    XybArgs A;
+    A.y = in[0]; A.x = in[1]; A.b = in[2];
+    for (int c = 0; c < 3; c++) { A.out[c] = out[c]; A.dq[c] = lf_dequant[c]; }
+    A.n = n;
+    k9_modular_xyb<<<(int)std::min<long long>((long long)ctx->sms * 8, (n + 255) / 256), 256, 0, ctx->stream>>>(A);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
     return 0;
 }
 

@@ -207,6 +207,7 @@ struct PackArgs {
     const void *plane[8];
     int is_int[8], depth[8];
     int n_channels, n_color, linear, h, w, bits;
+    int layout;                 // 0: interleaved PNG bytes (big-endian 16 bit); 1: planar [C][h][w] uint8 / native-endian uint16
     unsigned char *out;
 };
 
@@ -237,7 +238,10 @@ __global__ void k8_pack_samples(PackArgs A) {
                 q = java_f2i(__fadd_rn(__fmul_rn(v, (float)maxv), 0.5f));
             }
             q = q < 0 ? 0 : (q > maxv ? maxv : q);
-            if (bytes == 2) { o[2 * c] = (unsigned char)(q >> 8); o[2 * c + 1] = (unsigned char)(q & 255); }
+            if (A.layout == 1) {
+                if (bytes == 2) reinterpret_cast<unsigned short *>(A.out)[c * n + i] = (unsigned short)q;
+                else A.out[c * n + i] = (unsigned char)q;
+            } else if (bytes == 2) { o[2 * c] = (unsigned char)(q >> 8); o[2 * c + 1] = (unsigned char)(q & 255); }
             else o[c] = (unsigned char)q;
         }
     }

@@ -9,8 +9,12 @@ J/io/PFMWriter.java:22-49) for the part of the format this build covers:
 Everything the frame loop of JXLCodestreamDecoder.decode (:588-626) does beyond that -- upsampling, noise, splines,
 patches, the other blend modes, LF frames, chroma subsampling -- raises NotImplementedError (SURVEY.md 8f-2..4).
 
-`engine` is the reconstruction back end.  The default is the CUDA library (jxlatte_b200.host.Reconstructor); there is no
-CPU fallback in this module -- the CPU tests inject the oracle explicitly (tests/test_frontend.py).
+`engine` is the reconstruction back end.  The default is the CUDA library (jxlatte_b200.host.Reconstructor) on host buffers;
+DeviceEngine keeps every buffer of the frame loop on the device and returns the image as CUDA tensors.  There is no CPU fallback
+in this module -- the CPU tests inject the oracle explicitly (tests/test_frontend.py).
+
+The frame loop is written once.  Where it creates, copies or casts a buffer it goes through the engine's `arrays` (NumpyArrays
+for engines that work on host arrays, the DeviceEngine itself for CUDA tensors), so the same loop runs on either.
 """
 import ctypes as C
 import struct
@@ -18,7 +22,7 @@ import zlib
 
 import numpy as np
 
-from . import frontend
+from . import frontend, host
 from .params import FrameParams
 from .upsampling import up_weights
 
@@ -54,6 +58,90 @@ def locate_view(v):
     if y + v.shape[0] > plane.shape[0] or x + v.shape[1] > W:
         return None
     return plane, y, x
+
+
+def locate_tensor_view(v):
+    """locate_view for torch tensors: a 2-D view with unit column stride -> (the rows of its storage at the view's row pitch, as a
+    2-D tensor from storage offset 0; y; x), or None when the view is not such a window.  Slicing keeps the parent's row stride, so
+    the pitch is stride(0) and the origin follows from the storage offset."""
+    if v.dim() != 2 or v.element_size() != 4:
+        return None
+    if v.shape[1] > 1 and v.stride(1) != 1:
+        return None
+    W = v.stride(0)
+    if W < 1 or W < v.shape[1]:
+        return None
+    total = v.untyped_storage().nbytes() // 4
+    y, x = divmod(v.storage_offset(), W)
+    rows = total // W
+    if y + v.shape[0] > rows or x + v.shape[1] > W:
+        return None
+    return v.as_strided((rows, W), (W, 1), 0), y, x
+
+
+class NumpyArrays:
+    """The buffer operations of the frame loop on host numpy arrays (CudaEngine, the oracle engine)."""
+
+    @staticmethod
+    def is_float(a):
+        return a.dtype == np.float32
+
+    @staticmethod
+    def zeros(shape, like=None):
+        return np.zeros(shape, np.float32 if like is None else like.dtype)
+
+    @staticmethod
+    def copy(a):
+        return a.copy()
+
+    @staticmethod
+    def contiguous(a):
+        return np.ascontiguousarray(a)
+
+    @staticmethod
+    def stack(planes):
+        return np.stack(planes)
+
+    @staticmethod
+    def upload(a):
+        return a
+
+    @staticmethod
+    def cast_to_float(a, depth):
+        """ImageBuffer.castToFloat: (float)v * (1f / ((1 << depth) - 1))."""
+        return a.astype(np.float32) * (np.float32(1.0) / np.float32((1 << depth) - 1))
+
+    @staticmethod
+    def modular_xyb(y, x, b, dq):
+        """Frame.decodeFrame :429-447 on the Modular channels Y, X, B - Y -> float X, Y, B."""
+        dq = [np.float32(v) for v in dq]
+        return [dq[0] * x.astype(np.float32), dq[1] * y.astype(np.float32), dq[2] * (y + b).astype(np.float32)]
+
+    @staticmethod
+    def orient(a, o):
+        """JXLCodestreamDecoder.transposeBuffer (:43-112) for orientation o != 1."""
+        if o == 2:
+            a = a[:, ::-1]
+        elif o == 3:
+            a = a[::-1, ::-1]
+        elif o == 4:
+            a = a[::-1, :]
+        elif o == 5:
+            a = a.T
+        elif o == 6:
+            a = a.T[:, ::-1]
+        elif o == 7:
+            a = a[::-1, ::-1].T
+        else:
+            a = a.T[::-1, :]
+        return np.ascontiguousarray(a)
+
+
+_NUMPY = NumpyArrays()
+
+
+def _arrays(engine):
+    return getattr(engine, "arrays", None) or _NUMPY
 
 
 class JXLOptions:
@@ -109,13 +197,16 @@ class CudaEngine:
             self._uploaded = st["qm_weights"]
         # the tolerance kernel is faster only with fewer than three EPF passes (profiles/r2_exact_vs_fast.md)
         if not (self.tolerance_mode and self.allow_tolerance_mode and p.epf_iters < 3 and (p.gab or p.epf_iters)):
-            return self.rec.reconstruct(p, st)
+            return self._reconstruct(p, st)
         from . import _lib
         self.rec.set_option(_lib.OPT_STAGE2, _lib.STAGE2_FUSED)
         try:
-            return self.rec.reconstruct(p, st)
+            return self._reconstruct(p, st)
         finally:
             self.rec.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
+
+    def _reconstruct(self, p, st):
+        return self.rec.reconstruct(p, st)
 
     def modular(self, channels, transforms, bit_depth):
         return self._host.ModularTransforms(self.rec, bit_depth).applyTransforms(channels, transforms)
@@ -181,6 +272,263 @@ class CudaEngine:
         self.rec.close()
 
 
+class DeviceEngine(CudaEngine):
+    """CudaEngine on CUDA tensors: every buffer of the frame loop stays on the device.  The front end's arrays of a frame are
+    uploaded once, each stage runs through the library's _dev entry points on torch's current stream of `device`, and nothing
+    comes back to the host until the image is: JXLImage.channels / planes are CUDA tensors, to_int / packed run the pack kernel on
+    the device.  The decoder synchronises once per displayed image (sync), which is where stream errors of the kernels surface."""
+
+    def __init__(self, device=0, allow_tolerance_mode=False):
+        import torch
+        self._torch = torch
+        super().__init__(device, allow_tolerance_mode)
+        self.device = torch.device("cuda", device)
+        # the legacy default stream is 0 to torch but "the context's own stream" to jxlb200_set_stream: pass cudaStreamLegacy (1)
+        self.stream = torch.cuda.current_stream(self.device)
+        self.rec.set_stream(self.stream.cuda_stream or 1)
+        self.arrays = self
+        self._dtypes = {np.dtype(np.int32): torch.int32, np.dtype(np.float32): torch.float32, np.dtype(np.uint8): torch.uint8}
+
+    def _on_stream(self):
+        """The library's kernels and the frame loop's torch work must share one stream; the library is bound to the stream that was
+        current when the engine was made.  Decoding under another stream would race with it, so that is an error."""
+        if self._torch.cuda.current_stream(self.device) != self.stream:
+            raise RuntimeError("DeviceEngine is bound to %r; decode on that stream (torch.cuda.stream(engine.stream))" % (self.stream,))
+
+    def sync(self):
+        """jxlb200_sync: wait for the decode's work and raise the first stream error it met (the host path's exception classes)."""
+        self._on_stream()
+        self.rec.sync()
+
+    # ---- buffer operations of the frame loop (NumpyArrays on tensors) ----
+    def is_float(self, a):
+        return a.dtype == self._torch.float32
+
+    def zeros(self, shape, like=None):
+        self._on_stream()
+        return self._torch.zeros(tuple(shape), dtype=self._torch.float32 if like is None else like.dtype, device=self.device)
+
+    def empty(self, shape, dtype=None):
+        self._on_stream()
+        return self._torch.empty(tuple(shape), dtype=dtype or self._torch.float32, device=self.device)
+
+    def copy(self, a):
+        self._on_stream()
+        return a.clone(memory_format=self._torch.contiguous_format)
+
+    def contiguous(self, a):
+        return a.contiguous()
+
+    def stack(self, planes):
+        self._on_stream()
+        return self._torch.stack(list(planes))
+
+    def upload(self, a, dtype=None):
+        """A front-end (numpy) array -> a contiguous tensor on the device; tensors pass through (made contiguous).  Host arrays are
+        copied into pinned memory from torch's caching host allocator (the front end may free its arrays as soon as this returns)
+        and sent with a non-blocking copy, so the host runs ahead of the device instead of waiting for each upload."""
+        torch = self._torch
+        self._on_stream()
+        if isinstance(a, torch.Tensor):
+            t = a.to(self.device)
+        else:
+            a = np.ascontiguousarray(a, dtype)
+            t = torch.from_numpy(a).pin_memory().to(self.device, non_blocking=True)
+        if dtype is not None and t.dtype != self._dtypes[np.dtype(dtype)]:
+            raise ValueError("device array has dtype %s, expected %s" % (t.dtype, np.dtype(dtype)))
+        return t.contiguous()
+
+    def cast_to_float(self, a, depth):
+        a = a.contiguous()
+        out = self.empty(a.shape)
+        self.rec.cast_to_float_dev(a.data_ptr(), a.numel(), np.float32(1.0) / np.float32((1 << depth) - 1), out.data_ptr())
+        return out
+
+    def modular_xyb(self, y, x, b, dq):
+        y, x, b = y.contiguous(), x.contiguous(), b.contiguous()
+        out = self.empty((3,) + tuple(y.shape))
+        self.rec.modular_xyb_dev([y.data_ptr(), x.data_ptr(), b.data_ptr()], y.numel(), dq, [out[c].data_ptr() for c in range(3)])
+        return [out[0], out[1], out[2]]
+
+    def orient(self, a, o):
+        torch = self._torch
+        if o == 2:
+            a = torch.flip(a, (1,))
+        elif o == 3:
+            a = torch.flip(a, (0, 1))
+        elif o == 4:
+            a = torch.flip(a, (0,))
+        elif o == 5:
+            a = a.t()
+        elif o == 6:
+            a = torch.flip(a.t(), (1,))
+        elif o == 7:
+            a = torch.flip(a, (0, 1)).t()
+        else:
+            a = torch.flip(a.t(), (0,))
+        return a.contiguous()
+
+    # ---- stages ----
+    def _reconstruct(self, p, st):
+        H, W = p.height, p.width
+        hb, wb, th, tw = H // 8, W // 8, (H + 63) // 64, (W + 63) // 64
+        q = [self.upload(st["qcoeff"][c], np.int32) for c in range(3)]
+        lf = [self.upload(st["lf"][c], np.float32) for c in range(3)]
+        for c in range(3):      # chroma-subsampled channels carry their own (H >> sy) x (W >> sx) planes
+            sy, sx = p.shift_y[c], p.shift_x[c]
+            if tuple(q[c].shape) != (H >> sy, W >> sx) or tuple(lf[c].shape) != (hb >> sy, wb >> sx):
+                raise ValueError("qcoeff[%d] / lf[%d] have shapes %s / %s, expected %s / %s" % (
+                    c, c, tuple(q[c].shape), tuple(lf[c].shape), (H >> sy, W >> sx), (hb >> sy, wb >> sx)))
+        maps = {}
+        for k, dt, shp in (("dct_select", np.uint8, (hb, wb)), ("block_origin", np.uint8, (hb, wb)), ("hf_mul", np.int32, (hb, wb)),
+                           ("x_from_y", np.int32, (th, tw)), ("b_from_y", np.int32, (th, tw)), ("sharpness", np.int32, (hb, wb))):
+            maps[k] = self.upload(st[k], dt)
+            if tuple(maps[k].shape) != shp:
+                raise ValueError("%s has shape %s, expected %s" % (k, tuple(maps[k].shape), shp))
+        out = self.empty((3, H, W))
+        self.rec.reconstruct_dev(p, [a.data_ptr() for a in q], [a.data_ptr() for a in lf],
+                                 *[maps[k].data_ptr() for k in ("dct_select", "block_origin", "hf_mul", "x_from_y", "b_from_y", "sharpness")],
+                                 [out[c].data_ptr() for c in range(3)])
+        return out
+
+    def lf_dequant(self, q, ep, scaled_dequant, kx, kb, smooth):
+        qd = [self.upload(q[c], np.int32) for c in range(3)]
+        hb, wb = qd[0].shape
+        if any(tuple(a.shape) != (hb, wb) for a in qd):
+            raise ValueError("lf_quant planes must share a shape")
+        out = self.empty((3, hb, wb))
+        self.rec.lf_dequant_dev(hb, wb, scaled_dequant, kx, kb, True, smooth, [a.data_ptr() for a in qd], ep, [out[c].data_ptr() for c in range(3)])
+        return out
+
+    def modular(self, channels, transforms, bit_depth):
+        return _DeviceModularTransforms(_DeviceModularOps(self), bit_depth).applyTransforms([self.upload(c, np.int32) for c in channels], transforms)
+
+    def _planes3(self, p, planes):
+        inp = [self.upload(planes[c], np.float32) for c in range(3)]
+        if any(tuple(a.shape) != (p.height, p.width) for a in inp):
+            raise ValueError("planes have shape %s, expected %s" % (tuple(inp[0].shape), (p.height, p.width)))
+        return inp
+
+    def color(self, p, planes):
+        inp = self._planes3(p, planes)
+        out = self.empty((3, p.height, p.width))
+        self.rec.color_transform_dev(p, [a.data_ptr() for a in inp], [out[c].data_ptr() for c in range(3)])
+        return out
+
+    def restore_modular(self, p, planes, sigma):
+        inp = self._planes3(p, planes)
+        out = self.empty((3, p.height, p.width))
+        self.rec.restore_uniform_dev(p, sigma, [a.data_ptr() for a in inp], [out[c].data_ptr() for c in range(3)])
+        return out
+
+    def upsample(self, plane, k, weights):
+        a = self.upload(plane, np.float32)
+        if a.dim() != 2:
+            raise ValueError("plane must be 2-D")
+        h, w = a.shape
+        out = self.empty((h * k, w * k))
+        self.rec.upsample_dev(a.data_ptr(), h, w, k, weights, out.data_ptr())
+        return out
+
+    def noise(self, planes, group_dim, seed0, lut, base_x, base_b):
+        buf = self.upload(planes, np.float32).clone()       # the argument is left as it is, as CudaEngine.noise does
+        h, w = buf.shape[1:]
+        self.rec.noise_dev([buf[c].data_ptr() for c in range(3)], h, w, group_dim, seed0, lut, base_x, base_b)
+        return buf
+
+    def splines(self, planes, splines, quant_adjust, base_x, base_b):
+        buf = self.upload(planes, np.float32).clone()       # the argument is left as it is, as CudaEngine.splines does
+        h, w = buf.shape[1:]
+        self.rec.splines_dev([buf[c].data_ptr() for c in range(3)], h, w, splines, quant_adjust, base_x, base_b)
+        return buf
+
+    def pack(self, channels, depths, n_color, linear, bits, layout=0):
+        """layout 0: uint8 [h, w, C * bits/8] PNG bytes (big-endian 16 bit); 1: [C, h, w] uint8 / uint16 samples."""
+        torch = self._torch
+        self._on_stream()
+        ch = [c.contiguous() for c in channels]
+        h, w = ch[0].shape
+        n = len(ch)
+        if layout == 1:
+            out = torch.empty((n, h, w), dtype=torch.uint16 if bits > 8 else torch.uint8, device=self.device)
+        else:
+            out = torch.empty((h, w, n * (2 if bits > 8 else 1)), dtype=torch.uint8, device=self.device)
+        self.rec.pack_samples_dev([c.data_ptr() for c in ch], [not self.is_float(c) for c in ch], depths, n_color, linear, h, w, bits, layout,
+                                  out.data_ptr())
+        return out
+
+    # ---- compositing: the rectangles of a frame are queued and blended in one call on the device planes ----
+    def _locate(self, v):
+        loc = locate_tensor_view(v)
+        if loc is None:
+            return None
+        plane, y, x = loc
+        key = (plane.data_ptr(), plane.shape[1])
+        if key not in self._batch_index:
+            self._batch_index[key] = len(self._batch_planes)
+            self._batch_planes.append(plane)
+        return self._batch_index[key], y, x
+
+    def blend(self, op, canvas, a, b, fa, ra):
+        refs = [self._locate(v) if v is not None else None for v in (canvas, a, b, fa, ra)]
+        if any(r is None and v is not None for r, v in zip(refs, (canvas, a, b, fa, ra))):
+            raise ValueError("blend operands must be 2-D windows of device planes with contiguous rows")
+        self._batch_items.append((dict(op), tuple(canvas.shape), refs))
+
+    def flush_blends(self):
+        planes, items = self._batch_planes, self._batch_items
+        self._batch_planes, self._batch_writable, self._batch_items, self._batch_index = [], [], [], {}
+        if items:
+            self._on_stream()
+            self.rec.blend_batch_dev([(pl.data_ptr(), pl.shape[0], pl.shape[1]) for pl in planes], items)
+
+
+class _DeviceModularOps:
+    """ModularStream's inverse transforms on device channels (int32 CUDA tensors) through the _dev entry points."""
+
+    def __init__(self, engine):
+        self.e = engine
+
+    def inverseRCT(self, channels, rct_type):
+        v = [c.clone(memory_format=self.e._torch.contiguous_format) for c in channels[:3]]
+        if not (v[0].shape == v[1].shape == v[2].shape):
+            raise host.InvalidBitstreamError("RCT must be performed on three equal size channels")
+        h, w = v[0].shape
+        self.e.rec.modular_rct_dev([a.data_ptr() for a in v], h, w, rct_type)
+        return v
+
+    def inversePalette(self, index_channel, palette, nb_deltas, d_pred, bit_depth):
+        idx, pal = index_channel.contiguous(), palette.contiguous()
+        num_c, nb_colors = pal.shape
+        h, w = idx.shape
+        out = [self.e.zeros((h, w), idx) for _ in range(num_c)]       # zero-initialised, as the host form's outputs
+        self.e.rec.modular_palette_dev(idx.data_ptr(), pal.data_ptr() if pal.numel() else 0, h, w, num_c, nb_colors, nb_deltas, d_pred,
+                                       bit_depth, [a.data_ptr() for a in out])
+        return out
+
+    def inverseHorizontalSqueeze(self, orig, res):
+        return self._squeeze(orig, res, True)
+
+    def inverseVerticalSqueeze(self, orig, res):
+        return self._squeeze(orig, res, False)
+
+    def _squeeze(self, orig, res, horizontal):
+        a, r = orig.contiguous(), res.contiguous()
+        ha, wa = a.shape
+        hr, wr = r.shape
+        out = self.e.zeros((ha, wa + wr) if horizontal else (ha + hr, wa), a)
+        self.e.rec.modular_squeeze_dev(a.data_ptr(), r.data_ptr() if r.numel() else 0, ha, wa, hr, wr, horizontal, out.data_ptr())
+        return out
+
+
+class _DeviceModularTransforms(host.ModularTransforms):
+    """ModularStream.applyTransforms, unchanged, over channels DeviceEngine.modular has already uploaded as int32 tensors."""
+
+    @staticmethod
+    def own(c):
+        return c            # fresh uploads of the front end's channels: nobody else holds them
+
+
 def _f32(x):
     return np.float32(x)
 
@@ -216,39 +564,47 @@ def _conversion_matrix(color):
 
 class _Buf:
     """ImageBuffer (J/util/ImageBuffer.java): one channel, int32 or float32, type changed in place by castToFloat so that
-    every alias (canvas, reference slots) sees it."""
+    every alias (canvas, reference slots) sees it.  `xp`: the array operations of the engine that owns the buffer."""
 
-    def __init__(self, a):
+    def __init__(self, a, xp=_NUMPY):
         self.a = a
+        self.xp = xp
 
     @property
     def is_int(self):
-        return self.a.dtype != np.float32
+        return not self.xp.is_float(self.a)
 
     before_mutation = staticmethod(lambda: None)     # set by the decoder: queued device blends must land before a buffer changes
 
     def cast_to_float(self, depth):
         if self.is_int:
             _Buf.before_mutation()
-            scale = np.float32(1.0) / np.float32((1 << depth) - 1)
-            self.a = self.a.astype(np.float32) * scale
+            self.a = self.xp.cast_to_float(self.a, depth)
 
 
 class JXLImage:
     """Decoded image.  `channels`: one 2-D array per channel (colour first, then extra channels): float32 linear light in
     the tagged primaries for XYB images (what PFMWriter writes), float32 in [0, 1] for other lossy images, int32 samples for
-    lossless Modular images.  `planes` stacks them (cast to float when the types are mixed)."""
+    lossless Modular images.  `planes` stacks them (cast to float when the types are mixed).
 
-    def __init__(self, channels, info, linear):
+    With `engine` (a DeviceEngine) the channels are CUDA tensors of the same dtypes and shapes; `planes`, `to_int` and `packed`
+    then stay on the device, and write_png / write_pfm copy to the host once."""
+
+    def __init__(self, channels, info, linear, engine=None):
         self.channels = list(channels)
         self.info = info
         self.linear = linear
+        self.engine = engine
+        self._xp = _arrays(engine)
 
     @property
     def planes(self):
         if len({c.dtype for c in self.channels}) == 1:
-            return np.stack(self.channels)
-        return np.stack([self._as_float(i) for i in range(len(self.channels))])
+            return self._xp.stack(self.channels)
+        return self._xp.stack([self._as_float(i) for i in range(len(self.channels))])
+
+    def _depths(self):
+        return [self._depth(i) for i in range(len(self.channels))]
 
     def _depth(self, i):
         ncol = self.info["color_channels"]
@@ -256,9 +612,9 @@ class JXLImage:
 
     def _as_float(self, i):
         c = self.channels[i]
-        if c.dtype == np.float32:
+        if self._xp.is_float(c):
             return c
-        return c.astype(np.float32) * (np.float32(1.0) / np.float32((1 << self._depth(i)) - 1))
+        return self._xp.cast_to_float(c, self._depth(i))
 
     @property
     def width(self):
@@ -271,7 +627,9 @@ class JXLImage:
     def to_int(self, bits=8):
         """PNGWriter's sample pipeline: TF_SRGB.fromLinearF for linear images, then (int)(v * max + 0.5f) clamped
         (J/color/TransferFunction.java:39-43, J/util/ImageBuffer.java:129-145).  Integer channels whose depth already is
-        `bits` are only clamped."""
+        `bits` are only clamped.  Device images: a CUDA [C, H, W] uint8 / uint16 tensor from the pack kernel."""
+        if self.engine is not None:
+            return self.engine.pack(self.channels, self._depths(), self.info["color_channels"], self.linear, bits, layout=1)
         if all(c.dtype != np.float32 and self._depth(i) == bits for i, c in enumerate(self.channels)):
             return np.clip(np.stack(self.channels), 0, (1 << bits) - 1).astype(np.uint16 if bits > 8 else np.uint8)
         v = np.stack([self._as_float(i) for i in range(len(self.channels))])
@@ -289,10 +647,12 @@ class JXLImage:
 
     def packed(self, bits=8, engine=None):
         """uint8 [h, w, C * bits/8] in PNG sample order (big-endian for 16 bit).  With an engine the transfer function,
-        quantisation and interleave run on the GPU (jxlb200_pack_samples); without one, in numpy (the PNGWriter mirror)."""
+        quantisation and interleave run on the GPU (jxlb200_pack_samples); without one, in numpy (the PNGWriter mirror).  Device
+        images: the same bytes as a CUDA uint8 tensor, from the pack kernel on the device planes."""
+        if self.engine is not None:
+            return self.engine.pack(self.channels, self._depths(), self.info["color_channels"], self.linear, bits)
         if engine is not None:
-            depths = [self._depth(i) for i in range(len(self.channels))]
-            return engine.pack(self.channels, depths, self.info["color_channels"], self.linear, bits)
+            return engine.pack(self.channels, self._depths(), self.info["color_channels"], self.linear, bits)
         rows = np.moveaxis(self.to_int(bits), 0, 2)
         if bits > 8:
             rows = rows.astype(">u2")
@@ -300,6 +660,8 @@ class JXLImage:
 
     def write_png(self, path, bits=8, engine=None):
         rows = self.packed(bits, engine)
+        if self.engine is not None:
+            rows = rows.cpu().numpy()
         c = len(self.channels)
         ctype = {1: 0, 2: 4, 3: 2, 4: 6}[c]
         raw = b"".join(b"\x00" + rows[y].tobytes() for y in range(rows.shape[0]))
@@ -312,7 +674,9 @@ class JXLImage:
 
     def write_pfm(self, path):
         v = [self._as_float(i) for i in range(len(self.channels))]
-        p = np.stack(v[:3] if len(v) >= 3 else v[:1])
+        p = self._xp.stack(v[:3] if len(v) >= 3 else v[:1])
+        if self.engine is not None:
+            p = p.cpu().numpy()
         with open(path, "wb") as f:
             f.write(("PF\n" if p.shape[0] == 3 else "Pf\n").encode() + ("%d %d\n1.0\n" % (self.width, self.height)).encode())
             f.write(np.moveaxis(p, 0, 2)[::-1].astype(">f4").tobytes())
@@ -339,6 +703,13 @@ class JXLDecoder:
         if self._own and self.engine is not None:
             self.engine.close()
             self.engine = None
+
+    @property
+    def _xp(self):
+        return _arrays(self.engine)
+
+    def _buf(self, a):
+        return _Buf(a, self._xp)
 
     # ---- frame-level pieces ----
     def frame_params(self, info, f):
@@ -394,6 +765,7 @@ class JXLDecoder:
     def decode_frame(self, parsed, k, lf_store=None):
         """-> (list of _Buf of frame size: colour channels then extra channels, colour transform still pending?, params)."""
         info, f = parsed.info, parsed.frames[k]
+        xp, buf = self._xp, self._buf
         h, w = f["height"], f["width"]
         bits = info["bits_per_sample"]
         mod = None
@@ -413,7 +785,7 @@ class JXLDecoder:
                 if src is None:
                     raise frontend.InvalidBitstreamError("LF Level too large")
                 bh, bw = f["padded_height"] // 8, f["padded_width"] // 8
-                lf = np.zeros((3, bh, bw), np.float32)
+                lf = xp.zeros((3, bh, bw))
                 for c in range(3):
                     src[c].cast_to_float(info["bits_per_sample"])
                     a = src[c].a[:bh, :bw]
@@ -439,7 +811,7 @@ class JXLDecoder:
                 rec = self.engine.reconstruct(q, st)
             else:
                 rec = self.engine.reconstruct(p, st)
-            bufs = [_Buf(np.ascontiguousarray(rec[c][:h, :w])) for c in range(3)]
+            bufs = [buf(xp.contiguous(rec[c][:h, :w])) for c in range(3)]
             first = 0
         else:
             if f["do_ycbcr"]:
@@ -447,21 +819,19 @@ class JXLDecoder:
             if info["xyb_encoded"]:
                 # lossy Modular: channels are Y, X, B - Y in integers; Frame.decodeFrame :429-447 scales them by LFGlobal.lfDequant
                 # (X, Y, B order) into float XYB planes, which then take the same colour transform as VarDCT frames
-                dq = [np.float32(v) for v in f["lf_dequant"]]
-                y, x, b = (np.ascontiguousarray(mod[c][:h, :w]) for c in range(3))
-                planes = [dq[0] * x.astype(np.float32), dq[1] * y.astype(np.float32), dq[2] * (y + b).astype(np.float32)]
-                bufs = [_Buf(np.ascontiguousarray(pl, np.float32)) for pl in planes]
+                y, x, b = (xp.contiguous(mod[c][:h, :w]) for c in range(3))
+                bufs = [buf(xp.contiguous(pl)) for pl in xp.modular_xyb(y, x, b, f["lf_dequant"])]
                 p = self.frame_params(info, dict(f, padded_width=-(-w // 8) * 8, padded_height=-(-h // 8) * 8, global_scale=1))
                 pending = True
                 first = 3
             else:
                 ncol = info["color_channels"]
-                bufs = [_Buf(np.ascontiguousarray(mod[c][:h, :w])) for c in range(ncol)]          # int32 samples (Frame.java:452-455)
+                bufs = [buf(xp.contiguous(mod[c][:h, :w])) for c in range(ncol)]          # int32 samples (Frame.java:452-455)
                 first = ncol
             if f["gab"] or f["epf_iters"] > 0:
                 bufs = self._restore_modular(info, f, bufs, first, h, w)
         for e in range(len(info["extra_channels"])):
-            bufs.append(_Buf(np.ascontiguousarray(mod[first + e][:h, :w])))
+            bufs.append(buf(xp.contiguous(mod[first + e][:h, :w])))
         return bufs, pending, p
 
     def _restore_modular(self, info, f, bufs, ncol, h, w):
@@ -481,7 +851,7 @@ class JXLDecoder:
             planes = [bufs[c].a for c in range(3)]
         out = self.engine.restore_modular(p, planes, f["epf_sigma_for_modular"])
         for c in range(ncol):
-            bufs[c] = _Buf(np.ascontiguousarray(out[c]))
+            bufs[c] = self._buf(self._xp.contiguous(out[c]))
         return bufs
 
     # ---- JXLCodestreamDecoder.blendBuffers (:415-497) ----
@@ -513,7 +883,7 @@ class JXLDecoder:
         if ref_bufs is None:
             raise frontend.InvalidBitstreamError("blending against a reference frame that was never stored")
         if ref_bufs[idx] is None:
-            ref_bufs[idx] = _Buf(np.zeros(canvas.a.shape, canvas.a.dtype))
+            ref_bufs[idx] = self._buf(self._xp.zeros(canvas.a.shape, canvas.a))
         ref_buf = ref_bufs[idx]
         ref_alpha = ref_bufs[colors + alpha_ch] if has_extra else None
         frame_alpha = frame_bufs[frame_colors + alpha_ch] if has_extra else None
@@ -521,7 +891,7 @@ class JXLDecoder:
             adepth = alpha_info["bits_per_sample"]
             if mode == 2:
                 if ref_alpha is None:
-                    ref_alpha = _Buf(np.zeros(canvas.a.shape, np.float32))
+                    ref_alpha = self._buf(self._xp.zeros(canvas.a.shape))
                     ref_bufs[colors + alpha_ch] = ref_alpha
                 ref_alpha.cast_to_float(adepth)
             frame_alpha.cast_to_float(adepth)
@@ -620,6 +990,8 @@ class JXLDecoder:
         if self.engine is None:
             self.engine = CudaEngine()
         info = parsed.info
+        xp, buf = self._xp, self._buf
+        sync = getattr(self.engine, "sync", None)
         _Buf.before_mutation = staticmethod(self._flush_blends)
         if hasattr(self.engine, "tolerance_mode"):
             self.engine.tolerance_mode = self.options.quantises_to_8_bits(info["bits_per_sample"])
@@ -654,32 +1026,32 @@ class JXLDecoder:
             fr = dict(f, height=fh, width=fw, y0=fy0, x0=fx0)
             has_noise = bool(f["flags"] & FLAG_NOISE)
             if save and f["save_before_ct"]:
-                reference[f["save_as_reference"]] = [_Buf(b.a.copy()) for b in bufs]
+                reference[f["save_as_reference"]] = [buf(xp.copy(b.a)) for b in bufs]
             self._compute_patches(info, fr, bufs, frame_colors, reference)
             if f["flags"] & FLAG_SPLINES and f["splines"]:
                 for c in range(3):
                     bufs[c].cast_to_float(info["bits_per_sample"])
-                xyb = self.engine.splines(np.stack([bufs[c].a for c in range(3)]), f["splines"], f["spline_quant_adjust"], f["base_corr_x"], f["base_corr_b"])
+                xyb = self.engine.splines(xp.stack([bufs[c].a for c in range(3)]), f["splines"], f["spline_quant_adjust"], f["base_corr_x"], f["base_corr_b"])
                 for c in range(3):
-                    bufs[c].a = np.ascontiguousarray(xyb[c])
+                    bufs[c].a = xp.contiguous(xyb[c])
             if has_noise:
                 for c in range(3):
                     bufs[c].cast_to_float(info["bits_per_sample"])
                 seed0 = (visible_frames << 32) | invisible_frames
-                xyb = self.engine.noise(np.stack([bufs[c].a for c in range(3)]), f["group_dim"], seed0, f["noise"], f["base_corr_x"], f["base_corr_b"])
+                xyb = self.engine.noise(xp.stack([bufs[c].a for c in range(3)]), f["group_dim"], seed0, f["noise"], f["base_corr_x"], f["base_corr_b"])
                 for c in range(3):
-                    bufs[c].a = np.ascontiguousarray(xyb[c])
+                    bufs[c].a = xp.contiguous(xyb[c])
             if pending:
                 hh, ww = bufs[0].a.shape
                 ph, pw = -(-hh // 8) * 8, -(-ww // 8) * 8          # the ABI takes padded planes; the transform is per pixel
                 q = p.copy()
                 q.width, q.height = pw, ph
-                xyb = np.zeros((3, ph, pw), np.float32)
+                xyb = xp.zeros((3, ph, pw))
                 for c in range(3):
                     xyb[c, :hh, :ww] = bufs[c].a
                 rgb = self.engine.color(q, xyb)
                 for c in range(3):
-                    bufs[c] = _Buf(np.ascontiguousarray(rgb[c, :hh, :ww]))
+                    bufs[c] = buf(xp.contiguous(rgb[c, :hh, :ww]))
             adopt = False
             if canvas is None:
                 # The usual still image: ONE VarDCT frame that covers the image and REPLACEs.  copyToCanvas would copy every
@@ -691,12 +1063,11 @@ class JXLDecoder:
                 if adopt:
                     canvas = list(bufs)
                 else:
-                    dt = bufs[0].a.dtype
-                    canvas = [_Buf(np.zeros((info["height"], info["width"]), dt)) for _ in range(colors + nextra)]
+                    canvas = [buf(xp.zeros((info["height"], info["width"]), bufs[0].a)) for _ in range(colors + nextra)]
             if f["type"] in (0, 3) and not adopt:
                 aliased = any(reference[i] is canvas and i != f["save_as_reference"] for i in range(4))
                 if aliased:
-                    canvas = [_Buf(b.a.copy()) for b in canvas]
+                    canvas = [buf(xp.copy(b.a)) for b in canvas]
                 # blendFrame (:499-523)
                 ih, iw = info["height"], info["width"]
                 ps = (min(max(fy0, 0), ih), min(max(fx0, 0), iw))
@@ -713,32 +1084,23 @@ class JXLDecoder:
             if save and not f["save_before_ct"]:
                 reference[f["save_as_reference"]] = canvas
             if f["is_last"] or f["duration"] != 0:
-                self.timings["reconstruct_s"] = time.perf_counter() - t1
-                yield self._finish(canvas, info, linear, copy=not f["is_last"])
+                if sync is None:
+                    self.timings["reconstruct_s"] = time.perf_counter() - t1
+                img = self._finish(canvas, info, linear, copy=not f["is_last"], xp=xp, engine=self.engine if xp is not _NUMPY else None)
+                if sync is not None:
+                    sync()                  # device engines: the image is complete, and stream errors surface here
+                    self.timings["reconstruct_s"] = time.perf_counter() - t1
+                yield img
                 t1 = time.perf_counter()
         parsed.close()
 
     @staticmethod
-    def _finish(canvas, info, linear, copy):
+    def _finish(canvas, info, linear, copy, xp=_NUMPY, engine=None):
         o = info["orientation"]
         out = []
         for b in canvas:
-            a = b.a.copy() if copy else b.a
+            a = xp.copy(b.a) if copy else b.a
             if o != 1:                    # JXLCodestreamDecoder.transposeBuffer (:43-112)
-                if o == 2:
-                    a = a[:, ::-1]
-                elif o == 3:
-                    a = a[::-1, ::-1]
-                elif o == 4:
-                    a = a[::-1, :]
-                elif o == 5:
-                    a = a.T
-                elif o == 6:
-                    a = a.T[:, ::-1]
-                elif o == 7:
-                    a = a[::-1, ::-1].T
-                else:
-                    a = a.T[::-1, :]
-                a = np.ascontiguousarray(a)
+                a = xp.orient(a, o)
             out.append(a)
-        return JXLImage(out, info, linear)
+        return JXLImage(out, info, linear, engine=engine)

@@ -87,6 +87,21 @@ def qm_generate(prm=None):
     return w, off
 
 
+def _blend_items(items):
+    """(op dict, (h, w), [(plane index, y, x) or None] * 5) tuples -> jxlb200_blend_item array."""
+    arr = (_lib.BlendItem * len(items))()
+    for k, (op, (h, w), refs) in enumerate(items):
+        it = arr[k]
+        it.op = _lib.BlendOp(int(op["mode"]), int(op["is_int"]), int(op["is_alpha"]), int(op["has_extra"]), int(op["clamp"]), int(op["premult"]))
+        it.h, it.w = int(h), int(w)
+        for r in range(5):
+            if refs[r] is None:
+                it.plane[r], it.y[r], it.x[r] = -1, 0, 0
+            else:
+                it.plane[r], it.y[r], it.x[r] = int(refs[r][0]), int(refs[r][1]), int(refs[r][2])
+    return arr
+
+
 class Reconstructor:
     """One per decoder instance (JXLDecoder ctor / close(), J/JXLDecoder.java:17-46).  Not thread-safe, like the reference."""
 
@@ -405,17 +420,78 @@ class Reconstructor:
         ph = np.array([a.shape[0] for a in planes], np.int32)
         pw = np.array([a.shape[1] for a in planes], np.int32)
         wr = np.array([1 if w else 0 for w in writable], np.int32)
-        arr = (_lib.BlendItem * len(items))()
-        for k, (op, (h, w), refs) in enumerate(items):
-            it = arr[k]
-            it.op = _lib.BlendOp(int(op["mode"]), int(op["is_int"]), int(op["is_alpha"]), int(op["has_extra"]), int(op["clamp"]), int(op["premult"]))
-            it.h, it.w = int(h), int(w)
-            for r in range(5):
-                if refs[r] is None:
-                    it.plane[r], it.y[r], it.x[r] = -1, 0, 0
-                else:
-                    it.plane[r], it.y[r], it.x[r] = int(refs[r][0]), int(refs[r][1]), int(refs[r][2])
+        arr = _blend_items(items)
         self._check(self._L.jxlb200_blend_batch(self._h, n, ptrs, _ptr(ph), _ptr(pw), _ptr(wr), len(items), C.byref(arr) if len(items) else None))
+
+    # -- device-resident frame loop (jxlatte_b200.decoder.DeviceEngine): integers are CUdeviceptr values; enqueued, not synchronised --
+    def lf_dequant_dev(self, hb, wb, scaled_dequant, kx, kb, cfl, smooth, lf_quant, extra_precision, out):
+        """jxlb200_lf_dequant_dev: lf_quant / out are three device pointers each; extra_precision a host array (one byte per LF group)."""
+        ep = _c(np.asarray(extra_precision).reshape(-1), np.uint8)
+        if ep.size != ((hb + 255) // 256) * ((wb + 255) // 256):
+            raise ValueError("extra_precision must hold one byte per LF group")
+        sd = (C.c_float * 3)(*[float(v) for v in scaled_dequant])
+        self._check(self._L.jxlb200_lf_dequant_dev(self._h, int(hb), int(wb), sd, C.c_float(float(kx)), C.c_float(float(kb)), 1 if cfl else 0,
+                                                   1 if smooth else 0, _lib.planes(lf_quant), _ptr(ep), _lib.planes(out)))
+
+    def restore_uniform_dev(self, p, epf_sigma_for_modular, planes_in, out):
+        self._check(self._L.jxlb200_restore_uniform_dev(self._h, C.byref(p), C.c_float(float(epf_sigma_for_modular)), _lib.planes(planes_in),
+                                                        _lib.planes(out)))
+
+    def color_transform_dev(self, p, planes_in, out):
+        self._check(self._L.jxlb200_color_transform_dev(self._h, C.byref(p), _lib.planes(planes_in), _lib.planes(out)))
+
+    def upsample_dev(self, plane, h, w, k, weights, out):
+        wt = _c(weights, np.float32)
+        if wt.shape != (k, k, 5, 5):
+            raise ValueError("weights must be [k][k][5][5]")
+        self._check(self._L.jxlb200_upsample_dev(self._h, plane, int(h), int(w), int(k), _ptr(wt), out))
+
+    def noise_dev(self, planes, h, w, group_dim, seed0, lut, base_corr_x, base_corr_b):
+        lt = _c(lut, np.float32)
+        self._check(self._L.jxlb200_noise_dev(self._h, _lib.planes(planes), int(h), int(w), int(group_dim), int(seed0), _ptr(lt),
+                                              float(base_corr_x), float(base_corr_b)))
+
+    def splines_dev(self, planes, h, w, splines, quant_adjust, base_corr_x, base_corr_b):
+        npts = np.array([len(s["points"]) // 2 for s in splines], np.int32)
+        pts = np.array([v for s in splines for v in s["points"]], np.int32)
+        cf = np.array([v for s in splines for v in s["coeff"]], np.int32)
+        self._check(self._L.jxlb200_splines_dev(self._h, _lib.planes(planes), int(h), int(w), len(splines), _ptr(npts), _ptr(pts), _ptr(cf),
+                                                int(quant_adjust), float(base_corr_x), float(base_corr_b)))
+
+    def blend_batch_dev(self, planes, items):
+        """planes: [(device pointer, h, w)] of 4-byte samples, pitch == w; items as for blend_batch.  Blended in place, in order."""
+        n = len(planes)
+        ptrs = (C.c_void_p * n)(*[int(p) for p, _, _ in planes])
+        ph = np.array([h for _, h, _ in planes], np.int32)
+        pw = np.array([w for _, _, w in planes], np.int32)
+        arr = _blend_items(items)
+        self._check(self._L.jxlb200_blend_batch_dev(self._h, n, ptrs, _ptr(ph), _ptr(pw), len(items), C.byref(arr) if len(items) else None))
+
+    def pack_samples_dev(self, planes, is_int, depths, n_color, linear, h, w, bits, layout, out):
+        n = len(planes)
+        ptrs = (C.c_void_p * n)(*[int(p) for p in planes])
+        ii = np.array([1 if v else 0 for v in is_int], np.int32)
+        dep = np.array(depths, np.int32)
+        self._check(self._L.jxlb200_pack_samples_dev(self._h, ptrs, _ptr(ii), _ptr(dep), n, int(n_color), int(bool(linear)), int(h), int(w),
+                                                     int(bits), int(layout), out))
+
+    def cast_to_float_dev(self, src, n, scale, out):
+        self._check(self._L.jxlb200_cast_to_float_dev(self._h, src, int(n), C.c_float(float(scale)), out))
+
+    def modular_xyb_dev(self, channels, n, lf_dequant, out):
+        dq = np.array([np.float32(v) for v in lf_dequant], np.float32)
+        self._check(self._L.jxlb200_modular_xyb_dev(self._h, _lib.planes(channels), int(n), _ptr(dq), _lib.planes(out)))
+
+    def modular_rct_dev(self, channels, h, w, rct_type):
+        self._check(self._L.jxlb200_modular_rct_dev(self._h, _lib.planes(channels), int(h), int(w), int(rct_type)))
+
+    def modular_palette_dev(self, idx, palette, h, w, num_c, nb_colors, nb_deltas, d_pred, bit_depth, out):
+        self._check(self._L.jxlb200_modular_palette_dev(self._h, idx, palette or None, int(h), int(w), int(num_c), int(nb_colors), int(nb_deltas),
+                                                        int(d_pred), int(bit_depth), _lib.planes(out)))
+
+    def modular_squeeze_dev(self, avg, res, h_avg, w_avg, h_res, w_res, horizontal, out):
+        self._check(self._L.jxlb200_modular_squeeze_dev(self._h, avg, res or None, int(h_avg), int(w_avg), int(h_res), int(w_res),
+                                                        1 if horizontal else 0, out))
 
     # -- Modular --
     def inverseRCT(self, channels, rct_type):
@@ -518,8 +594,13 @@ class ModularTransforms:
         self.r = reconstructor
         self.bit_depth = bit_depth
 
+    @staticmethod
+    def own(c):
+        """The channel list is edited in place: each channel becomes an int32 C-contiguous array of the transforms' own."""
+        return np.array(c, dtype=np.int32, order="C")
+
     def applyTransforms(self, channels, transforms):
-        ch = [np.array(c, dtype=np.int32, order="C") for c in channels]
+        ch = [self.own(c) for c in channels]
         for tr in reversed(transforms):
             if tr["tr"] == SQUEEZE:
                 for (horizontal, in_place, begin, num_c) in reversed(tr["sp"]):

@@ -2,7 +2,9 @@
 front end + the CUDA reconstruction and writes PNG (8/16 bit) or PFM.  Prints the host front-end time (entropy decoding,
 headers) and the reconstruction time separately, as the north star asks.
 
-    python tools/decode_sample.py input.jxl [output.png|output.pfm] [--bits 8|16] [--repeat N]
+    python tools/decode_sample.py input.jxl [output.png|output.pfm] [--bits 8|16] [--repeat N] [--device]
+
+--device decodes through DeviceEngine: the image stays on the GPU until the output file is written from it.
 
 There is no CPU engine here: the checker's decode of the same file is tests/tools/decode_with_oracle.py."""
 import argparse
@@ -20,9 +22,10 @@ def main():
     ap.add_argument("output", nargs="?")
     ap.add_argument("--bits", type=int, default=8)
     ap.add_argument("--repeat", type=int, default=1)
+    ap.add_argument("--device", action="store_true", help="keep the frame loop and the image on the GPU (DeviceEngine)")
     a = ap.parse_args()
-    from jxlatte_b200.decoder import CudaEngine, JXLDecoder
-    engine = CudaEngine()
+    from jxlatte_b200.decoder import CudaEngine, DeviceEngine, JXLDecoder
+    engine = DeviceEngine() if a.device else CudaEngine()
     best = None
     for _ in range(a.repeat):
         d = JXLDecoder(a.input, engine=engine)
@@ -32,8 +35,8 @@ def main():
         if best is None or total < best[0]:
             best = (total, dict(d.timings))
     mp = img.width * img.height / 1e6
-    print("%s: %dx%d, %d channel(s), engine=cuda: front end %.1f ms, reconstruction + glue %.1f ms, total %.1f ms (%.1f MP/s end to end)" % (
-        os.path.basename(a.input), img.width, img.height, img.planes.shape[0], best[1]["front_end_s"] * 1e3,
+    print("%s: %dx%d, %d channel(s), engine=%s: front end %.1f ms, reconstruction + glue %.1f ms, total %.1f ms (%.1f MP/s end to end)" % (
+        os.path.basename(a.input), img.width, img.height, len(img.channels), "device" if a.device else "cuda", best[1]["front_end_s"] * 1e3,
         best[1]["reconstruct_s"] * 1e3, best[0] * 1e3, mp / best[0]))
     if a.output:
         if a.output.endswith(".pfm"):
