@@ -6,6 +6,7 @@
 #include <string.h>
 #include <new>
 #include <algorithm>
+#include <array>
 #include <string>
 #include <vector>
 
@@ -69,6 +70,7 @@ struct jxlb200_ctx {
     std::vector<cudaEvent_t> ev_pool;
 
     DevBuf sched, items, gate, wraw, woff, wexp, cosbig, lut8, sigma, flags;
+    bool flags_pending = false;         // a kernel that may raise an error flag was enqueued since check_flags last read them
     float lut8_host[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // what lut8 holds on the device, and the stream that put it there
     cudaStream_t lut8_stream = nullptr;
     bool lut8_valid = false;
@@ -204,6 +206,13 @@ template <int N, int PASS> void launch_big(jxlb200_ctx *ctx, const K1Params &P, 
     ctx->launches++;
 }
 
+// the device error flags (check_flags), allocated and zeroed on first use
+cudaError_t ensure_flags(jxlb200_ctx *ctx, cudaStream_t st) {
+    if (ctx->flags.p) return cudaSuccess;
+    cudaError_t e = ctx->flags.ensure(sizeof(int) * 4);
+    return e == cudaSuccess ? cudaMemsetAsync(ctx->flags.p, 0, sizeof(int) * 4, st) : e;
+}
+
 bool is_subsampled(const jxlb200_frame_params *p) {
     for (int c = 0; c < 3; c++)
         if (p->shift_x[c] || p->shift_y[c]) return true;
@@ -220,10 +229,7 @@ int invert_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const int32_t *c
     CUDA_TRY(ctx, ctx->sched.ensure(sizeof(Sched)));
     CUDA_TRY(ctx, ctx->items.ensure(sizeof(int) * (size_t)wb * hb));
     CUDA_TRY(ctx, ctx->gate.ensure(sizeof(int) * (size_t)tw * th));
-    if (!ctx->flags.p) {
-        CUDA_TRY(ctx, ctx->flags.ensure(sizeof(int) * 4));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->flags.p, 0, sizeof(int) * 4, ctx->stream));
-    }
+    CUDA_TRY(ctx, ensure_flags(ctx, ctx->stream));
     cudaStream_t st = ctx->stream;
     Sched *S = ctx->sched.as<Sched>();
     CUDA_TRY(ctx, cudaMemsetAsync(S, 0, sizeof(Sched), st));
@@ -231,6 +237,7 @@ int invert_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const int32_t *c
     const int g0 = min(ctx->sms * 4, ceil_div(ncells, 256));
     const int fhb = frame_rows > 0 ? frame_rows >> 3 : hb;      // block rows of one frame (a batch is a vertical stack)
     k0_count<<<g0, 256, 0, st>>>(ds, bo, ncells, wb, fhb, S, ctx->flags.as<int>() + 2);
+    ctx->flags_pending = true;
     k0_plan<<<1, 32, 0, st>>>(S);
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->gate.p, 0x7f, sizeof(int) * (size_t)tw * th, st));
     k0_scatter<<<g0, 256, 0, st>>>(ds, bo, hb, wb, fhb, S, ctx->items.as<int>(), ctx->gate.as<int>(), tw);
@@ -302,10 +309,7 @@ int invert_subsampled_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const
     CUDA_TRY(ctx, ctx->sub.ensure(sizeof(float) * 4 * npx));
     const size_t nb4 = (nb + 3) & ~(size_t)3;
     CUDA_TRY(ctx, ctx->sub_maps.ensure(2 * nb4 + sizeof(int32_t) * (nb + 2 * nt)));
-    if (!ctx->flags.p) {
-        CUDA_TRY(ctx, ctx->flags.ensure(sizeof(int) * 4));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->flags.p, 0, sizeof(int) * 4, ctx->stream));
-    }
+    CUDA_TRY(ctx, ensure_flags(ctx, ctx->stream));
     cudaStream_t st = ctx->stream;
     char *mb = (char *)ctx->sub_maps.p;
     uint8_t *ds_c = (uint8_t *)mb, *bo_c = (uint8_t *)(mb + nb4);
@@ -317,6 +321,7 @@ int invert_subsampled_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const
         const int sy = p->shift_y[c], sx = p->shift_x[c];
         const int Hc = H >> sy, Wc = W >> sx, hbc = hb >> sy, wbc = wb >> sx;
         k6_submap<<<min(ctx->sms * 4, ceil_div(hbc * wbc, 256)), 256, 0, st>>>(ds, hf_mul, wb, hbc, wbc, sy, sx, ds_c, bo_c, hf_c, ctx->flags.as<int>() + 3);
+        ctx->flags_pending = true;
         ctx->launches++;
         jxlb200_frame_params pc = *p;
         pc.width = Wc; pc.height = Hc;
@@ -394,10 +399,7 @@ int restore_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const jxlb200_s
     if (K.iters > 0) {
         CUDA_TRY(ctx, ctx->sigma.ensure(sizeof(float) * (size_t)wb * ((size_t)((rows + 7) / 8) * n_frames + 2)));
         CUDA_TRY(ctx, ctx->lut8.ensure(sizeof(float) * 8));
-        if (!ctx->flags.p) {
-            CUDA_TRY(ctx, ctx->flags.ensure(sizeof(int) * 4));
-            CUDA_TRY(ctx, cudaMemsetAsync(ctx->flags.p, 0, sizeof(int) * 4, st));
-        }
+        CUDA_TRY(ctx, ensure_flags(ctx, st));
         // K.sharp_lut lives in pageable memory, and an asynchronous copy from pageable memory first waits for everything
         // enqueued on its stream: once per slab that stalled the host behind stage 1 and left the upload engine idle meanwhile.
         // The table rarely changes (RestorationFilter.java:18-44), so it goes up only when it differs from the device's copy.
@@ -411,9 +413,11 @@ int restore_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const jxlb200_s
         const int br0 = K.has_top ? -1 : 0, br1 = ((rows + 7) / 8) * n_frames + (K.has_bottom ? 1 : 0);
         if (ctx->uniform_sigma)
             k2_sigma_fill<<<min(ctx->sms * 2, ceil_div((br1 - br0) * wb, 256)), 256, 0, st>>>(ctx->uniform_inv_sigma, (long long)br0 * wb, (long long)(br1 - br0) * wb, inv_sigma);
-        else
+        else {
             k2_sigma<<<min(ctx->sms * 2, ceil_div((br1 - br0) * wb, 256)), 256, 0, st>>>(hf_mul, sharp, wb, br0, br1, K.gscale,
                                                                                          ctx->lut8.as<float>(), inv_sigma, ctx->flags.as<int>());
+            ctx->flags_pending = true;
+        }
         ctx->launches++;
     }
     // Two bit-exact fused kernels.  Default: the stream kernel where it is the faster one -- at least 0.6 MP, and Gaborish on or three EPF
@@ -519,9 +523,11 @@ int restore_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const jxlb200_s
     return 0;
 }
 
-// device error flags -> status: [0] sharpness outside 0..7, [1] palette scratch, [2] dct_select out of range
+// device error flags -> status: [0] sharpness outside 0..7, [1] palette scratch, [2] dct_select out of range, [3] subsampling with
+// large varblocks.  Read (a synchronous round trip) only when a kernel that raises them ran since the last read.
 int check_flags(jxlb200_ctx *ctx) {
-    if (!ctx->flags.p) return 0;
+    if (!ctx->flags_pending) return 0;
+    ctx->flags_pending = false;
     int e[4] = {0, 0, 0, 0};
     CUDA_TRY(ctx, cudaMemcpy(e, ctx->flags.p, sizeof(e), cudaMemcpyDeviceToHost));
     if (!e[0] && !e[2] && !e[3]) return 0;
@@ -554,6 +560,57 @@ int upload_maps(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const uint8_t *
     if (bfy) CUDA_TRY(ctx, cudaMemcpyAsync(M.bfy, bfy, sizeof(int32_t) * nt, cudaMemcpyHostToDevice, st));
     return 0;
 }
+
+// One host array of a host entry point and the device region it is staged in: `in` is uploaded before the call's kernels,
+// `out` downloaded after them (the same pointer for an array changed in place).  Every region is copied at least one way, so
+// a region of non-zero size with neither pointer is a NULL argument.
+struct Staged {
+    DevBuf *buf;
+    const void *in;
+    void *out;
+    size_t bytes;
+    void *dev = nullptr;
+};
+
+size_t staged_bytes(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
+
+// Checks every host pointer and carves the regions out of their buffers on the context's device, then uploads the inputs.
+// The regions of one buffer must be consecutive in r[]: they share one allocation (each region 256-byte aligned), and a later
+// group of the same buffer would reallocate it under the earlier one.
+int stage_in(jxlb200_ctx *ctx, Staged *r, int n) {
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    for (int i = 0; i < n;) {
+        size_t total = 0;
+        int end = i;
+        for (; end < n && r[end].buf == r[i].buf; end++) {
+            if (r[end].bytes && !r[end].in && !r[end].out) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+            total += staged_bytes(r[end].bytes);
+        }
+        CUDA_TRY(ctx, r[i].buf->ensure(total));
+        for (char *at = (char *)r[i].buf->p; i < end; at += staged_bytes(r[i++].bytes)) r[i].dev = at;
+    }
+    for (int i = 0; i < n; i++)
+        if (r[i].in && r[i].bytes) CUDA_TRY(ctx, cudaMemcpyAsync(r[i].dev, r[i].in, r[i].bytes, cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+}
+
+// Downloads the outputs, then synchronises and reports device errors as jxlb200_sync does.
+int stage_out(jxlb200_ctx *ctx, const Staged *r, int n) {
+    for (int i = 0; i < n; i++)
+        if (r[i].out && r[i].bytes) CUDA_TRY(ctx, cudaMemcpyAsync(r[i].out, r[i].dev, r[i].bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    return jxlb200_sync(ctx);
+}
+
+// r[0..2]: three input planes staged in `bin`, r[3..5]: three output planes staged in `bout`, `bytes` each
+template <class I, class O> void stage_planes(Staged *r, DevBuf &bin, I *const in[3], DevBuf &bout, O *const out[3], size_t bytes) {
+    for (int c = 0; c < 3; c++) {
+        r[c] = {&bin, in[c], nullptr, bytes};
+        r[3 + c] = {&bout, nullptr, out[c], bytes};
+    }
+}
+
+// the device pointers of three staged planes (.data() is the `T *const [3]` argument of an enqueue routine)
+template <class T> std::array<T *, 3> planes_of(const Staged *r) { return {(T *)r[0].dev, (T *)r[1].dev, (T *)r[2].dev}; }
 
 }  // namespace
 
@@ -992,25 +1049,6 @@ int32_t jxlb200_vardct_reconstruct_split_dev(jxlb200_ctx *ctx, const jxlb200_fra
 }
 
 // host-buffer entry points ------------------------------------------------------------------------------------
-static int stage_in_planes(jxlb200_ctx *ctx, DevBuf &buf, const void *const src[3], size_t bytes_per_plane, void *dst[3]) {
-    CUDA_TRY(ctx, buf.ensure(3 * bytes_per_plane));
-    for (int c = 0; c < 3; c++) {
-        dst[c] = (char *)buf.p + c * bytes_per_plane;
-        if (!src[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
-        CUDA_TRY(ctx, cudaMemcpyAsync(dst[c], src[c], bytes_per_plane, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    return 0;
-}
-
-static int stage_out_planes(jxlb200_ctx *ctx, const float *const dev[3], size_t bytes_per_plane, float *const out[3]) {
-    for (int c = 0; c < 3; c++) {
-        if (!out[c]) return ctx->fail(JXLB200_E_ARG, "NULL output plane pointer");
-        CUDA_TRY(ctx, cudaMemcpyAsync(out[c], dev[c], bytes_per_plane, cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return check_flags(ctx);
-}
-
 // Whole path on host buffers.  Frames taller than one slab are pipelined by group rows over three streams: while slab i
 // is uploaded (copy engine 1), stage 1 and stage 2 of slab i-1 run, and slab i-2's pixels go back (copy engine 2) -- PCIe
 // is full duplex, so the call costs about max(upload, download, compute) instead of their sum.  Stage 2 needs HALO rows
@@ -1174,7 +1212,9 @@ static int reconstruct_host(jxlb200_ctx *ctx, const jxlb200_frame_params *p, con
             CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
             return check_flags(ctx);
         }
-        return stage_out_planes(ctx, dout, sizeof(float) * npx, out);
+        Staged r[3];
+        for (int c = 0; c < 3; c++) r[c] = {&ctx->out_planes, nullptr, out[c], sizeof(float) * npx, dout[c]};
+        return stage_out(ctx, r, 3);
     }
     // stage 2 of one slab and stage 1 of the next touch disjoint rows and disjoint context buffers, so they run on two
     // streams: on slab-sized pieces stage 1 is a chain of short latency-bound launches, which hide under the issue-bound k2
@@ -1328,18 +1368,17 @@ int32_t jxlb200_vardct_invert(jxlb200_ctx *ctx, const jxlb200_frame_params *p,
     if (rc) return rc;
     if (!qcoeff || !lf || !dct_select || !block_origin || !hf_mul || !x_from_y || !b_from_y || !xyb)
         return ctx->fail(JXLB200_E_ARG, "NULL pointer");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t npx = (size_t)p->width * p->height, nb = npx / 64;
-    void *dq[3], *dlf[3];
-    if ((rc = stage_in_planes(ctx, ctx->in_q, (const void *const *)qcoeff, sizeof(int32_t) * npx, dq))) return rc;
-    if ((rc = stage_in_planes(ctx, ctx->in_lf, (const void *const *)lf, sizeof(float) * nb, dlf))) return rc;
+    Staged r[9];
+    stage_planes(r, ctx->in_q, qcoeff, ctx->out_planes, xyb, sizeof(float) * npx);
+    for (int c = 0; c < 3; c++) r[6 + c] = {&ctx->in_lf, lf[c], nullptr, sizeof(float) * nb};
+    if ((rc = stage_in(ctx, r, 9))) return rc;
     HostMaps M;
     if ((rc = upload_maps(ctx, p, dct_select, block_origin, hf_mul, x_from_y, b_from_y, nullptr, M))) return rc;
-    CUDA_TRY(ctx, ctx->out_planes.ensure(sizeof(float) * 3 * npx));
-    float *dout[3] = {ctx->out_planes.as<float>(), ctx->out_planes.as<float>() + npx, ctx->out_planes.as<float>() + 2 * npx};
-    rc = invert_dev(ctx, p, (const int32_t *const *)dq, (const float *const *)dlf, M.ds, M.bo, M.hf, M.xfy, M.bfy, dout, p->width);
-    if (rc) return rc;
-    return stage_out_planes(ctx, dout, sizeof(float) * npx, xyb);
+    if ((rc = invert_dev(ctx, p, planes_of<const int32_t>(r).data(), planes_of<const float>(r + 6).data(), M.ds, M.bo, M.hf, M.xfy, M.bfy,
+                         planes_of<float>(r + 3).data(), p->width)))
+        return rc;
+    return stage_out(ctx, r, 9);
 }
 
 // one restoration stage on device planes: mode 0 Gaborish only, 1 EPF only, 2 colour only (what the host form and the _dev form share)
@@ -1352,33 +1391,38 @@ static int stage_enqueue(jxlb200_ctx *ctx, const jxlb200_frame_params *p, int mo
     return restore_dev(ctx, &q, nullptr, din, p->width, hf_mul, sharp, dout);
 }
 
-// one restoration stage on host planes: upload, stage_enqueue, download
-static int host_stage(jxlb200_ctx *ctx, const jxlb200_frame_params *p, int mode, const float *const in[3],
-                      const int32_t *hf_mul, const int32_t *sharp, float *const out[3]) {
+// frame params and three input and three output planes (the restoration stages)
+static int check_planes(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float *const in[3], float *const out[3]) {
     int rc = check_params(ctx, p);
     if (rc) return rc;
     if (!in || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t npx = (size_t)p->width * p->height;
-    void *din[3];
-    if ((rc = stage_in_planes(ctx, ctx->in_q, (const void *const *)in, sizeof(float) * npx, din))) return rc;
-    HostMaps M;
-    memset(&M, 0, sizeof(M));
-    if (mode == 1) {
-        if (!hf_mul || !sharp) return ctx->fail(JXLB200_E_ARG, "EPF needs hf_mul and sharpness");
-        if ((rc = upload_maps(ctx, p, nullptr, nullptr, hf_mul, nullptr, nullptr, sharp, M))) return rc;
-    }
-    CUDA_TRY(ctx, ctx->out_planes.ensure(sizeof(float) * 3 * npx));
-    float *dout[3] = {ctx->out_planes.as<float>(), ctx->out_planes.as<float>() + npx, ctx->out_planes.as<float>() + 2 * npx};
-    rc = stage_enqueue(ctx, p, mode, (const float *const *)din, M.hf, M.sharp, dout);
+    for (int c = 0; c < 3; c++)
+        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+    return 0;
+}
+
+// one restoration stage on host planes: stage in, stage_enqueue, stage out
+static int host_stage(jxlb200_ctx *ctx, const jxlb200_frame_params *p, int mode, const float *const in[3],
+                      const int32_t *hf_mul, const int32_t *sharp, float *const out[3]) {
+    int rc = check_planes(ctx, p, in, out);
     if (rc) return rc;
-    return stage_out_planes(ctx, dout, sizeof(float) * npx, out);
+    if (mode == 1 && (!hf_mul || !sharp)) return ctx->fail(JXLB200_E_ARG, "EPF needs hf_mul and sharpness");
+    Staged r[6];
+    stage_planes(r, ctx->in_q, in, ctx->out_planes, out, sizeof(float) * p->width * p->height);
+    if ((rc = stage_in(ctx, r, 6))) return rc;
+    HostMaps M{};
+    if (mode == 1 && (rc = upload_maps(ctx, p, nullptr, nullptr, hf_mul, nullptr, nullptr, sharp, M))) return rc;
+    if ((rc = stage_enqueue(ctx, p, mode, planes_of<const float>(r).data(), M.hf, M.sharp, planes_of<float>(r + 3).data()))) return rc;
+    return stage_out(ctx, r, 6);
 }
 
 // Gaborish + EPF of a Modular-encoded frame (Frame.decodeFrame :457-461 with header.encoding == MODULAR): one sigma for the frame
-static int check_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular, const void *in, const void *out) {
+static int check_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular, const float *const in[3],
+                         float *const out[3]) {
     if (!ctx) return JXLB200_E_ARG;
     if (!p || !in || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
+    for (int c = 0; c < 3; c++)
+        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
     // a Modular frame has its own size, not a multiple of 8; sizes the tile kernel does not take go through the staged kernels
     if (p->width <= 0 || p->height <= 0 || p->width > 65535 * 8 || p->height > 65535 * 8) return ctx->fail(JXLB200_E_ARG, "bad frame size");
     if ((p->gab || p->epf_iters) && (p->width < 4 || p->height < 4))
@@ -1407,30 +1451,20 @@ int32_t jxlb200_restore_uniform(jxlb200_ctx *ctx, const jxlb200_frame_params *p,
     const float *const in[3], float *const out[3]) {
     int rc = check_uniform(ctx, p, epf_sigma_for_modular, in, out);
     if (rc) return rc;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t npx = ((size_t)p->width * p->height + 3) & ~(size_t)3;      // planes stay 16-byte aligned
-    const float *din[3];
-    CUDA_TRY(ctx, ctx->in_q.ensure(3 * sizeof(float) * npx));
-    for (int c = 0; c < 3; c++) {
-        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
-        din[c] = ctx->in_q.as<float>() + c * npx;
-        CUDA_TRY(ctx, cudaMemcpyAsync((void *)din[c], in[c], sizeof(float) * (size_t)p->width * p->height, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    CUDA_TRY(ctx, ctx->out_planes.ensure(sizeof(float) * 3 * npx));
-    float *dout[3] = {ctx->out_planes.as<float>(), ctx->out_planes.as<float>() + npx, ctx->out_planes.as<float>() + 2 * npx};
-    if ((rc = restore_uniform_enqueue(ctx, p, epf_sigma_for_modular, din, dout))) return rc;
-    return stage_out_planes(ctx, dout, sizeof(float) * (size_t)p->width * p->height, out);
+    Staged r[6];
+    stage_planes(r, ctx->in_q, in, ctx->out_planes, out, sizeof(float) * p->width * p->height);
+    if ((rc = stage_in(ctx, r, 6))) return rc;
+    if ((rc = restore_uniform_enqueue(ctx, p, epf_sigma_for_modular, planes_of<const float>(r).data(), planes_of<float>(r + 3).data()))) return rc;
+    return stage_out(ctx, r, 6);
 }
 
 int32_t jxlb200_restore_uniform_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, float epf_sigma_for_modular,
     const float *const in[3], float *const out[3]) {
     int rc = check_uniform(ctx, p, epf_sigma_for_modular, in, out);
     if (rc) return rc;
-    for (int c = 0; c < 3; c++) {
-        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+    for (int c = 0; c < 3; c++)
         for (int d = 0; d < 3; d++)
             if (in[c] == out[d]) return ctx->fail(JXLB200_E_ARG, "in-place restore is not allowed");
-    }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     return restore_uniform_enqueue(ctx, p, epf_sigma_for_modular, in, out);
 }
@@ -1446,24 +1480,51 @@ int32_t jxlb200_color_transform(jxlb200_ctx *ctx, const jxlb200_frame_params *p,
     return host_stage(ctx, p, 2, in, nullptr, nullptr, out);
 }
 int32_t jxlb200_color_transform_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float *const in[3], float *const out[3]) {
-    int rc = check_params(ctx, p);
+    int rc = check_planes(ctx, p, in, out);
     if (rc) return rc;
-    if (!in || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
-    for (int c = 0; c < 3; c++) {
-        if (!in[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+    for (int c = 0; c < 3; c++)
         for (int d = 0; d < 3; d++)
             if (in[c] == out[d]) return ctx->fail(JXLB200_E_ARG, "in-place colour transform is not allowed");
-    }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     return stage_enqueue(ctx, p, 2, in, nullptr, nullptr, out);
 }
 
-// ---- Modular ----
-int32_t jxlb200_modular_rct_dev(jxlb200_ctx *ctx, int32_t *const ch[3], int32_t h, int32_t w, int32_t rct_type) {
+// ---- Modular: each host form stages its arrays around the _dev form ----
+static int rct_check(jxlb200_ctx *ctx, int32_t *const ch[3], int32_t h, int32_t w, int32_t rct_type) {
     if (!ctx) return JXLB200_E_ARG;
     if (!ch || !ch[0] || !ch[1] || !ch[2] || h < 0 || w < 0) return ctx->fail(JXLB200_E_ARG, "bad RCT arguments");
     if (rct_type < 0 || rct_type >= 42) return ctx->fail(JXLB200_E_ARG, "rct_type outside 0..41");
-    if (h == 0 || w == 0) return 0;
+    return 0;
+}
+
+static int squeeze_check(jxlb200_ctx *ctx, const int32_t *avg, const int32_t *res, int32_t h_avg, int32_t w_avg, int32_t h_res,
+                         int32_t w_res, int32_t horizontal, const int32_t *out) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!avg || !out || h_avg < 0 || w_avg < 0 || h_res < 0 || w_res < 0) return ctx->fail(JXLB200_E_ARG, "bad squeeze arguments");
+    if (horizontal) {
+        if ((w_avg != w_res && w_avg != 1 + w_res) || h_res != h_avg) return ctx->fail(JXLB200_E_ARG, "Corrupted squeeze transform");
+    } else {
+        if ((h_avg != h_res && h_avg != 1 + h_res) || w_res != w_avg) return ctx->fail(JXLB200_E_ARG, "Corrupted squeeze transform");
+    }
+    if (!res && h_res > 0 && w_res > 0) return ctx->fail(JXLB200_E_ARG, "bad squeeze arguments");
+    return 0;
+}
+
+static int palette_check(jxlb200_ctx *ctx, const int32_t *idx, const int32_t *palette, int32_t h, int32_t w, int32_t num_c,
+                         int32_t nb_colors, int32_t d_pred, int32_t *const out[]) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!idx || !out || h < 0 || w < 0 || num_c < 1 || nb_colors < 0 || (nb_colors > 0 && !palette))
+        return ctx->fail(JXLB200_E_ARG, "bad palette arguments");
+    if (d_pred < 0 || d_pred > 13) return ctx->fail(JXLB200_E_ARG, "d_pred outside 0..13");
+    if (d_pred == 6) return ctx->fail(JXLB200_E_UNSUPPORTED, "palette delta with the weighted predictor (reference dereferences null pred[][])");
+    for (int c = 0; c < num_c; c++)
+        if (!out[c]) return ctx->fail(JXLB200_E_ARG, "NULL palette output channel");
+    return 0;
+}
+
+int32_t jxlb200_modular_rct_dev(jxlb200_ctx *ctx, int32_t *const ch[3], int32_t h, int32_t w, int32_t rct_type) {
+    int rc = rct_check(ctx, ch, h, w, rct_type);
+    if (rc || h == 0 || w == 0) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const long long n = (long long)h * w;
     const int grid = (int)min((long long)ctx->sms * 8, (n + 255) / 256);
@@ -1475,15 +1536,8 @@ int32_t jxlb200_modular_rct_dev(jxlb200_ctx *ctx, int32_t *const ch[3], int32_t 
 
 int32_t jxlb200_modular_squeeze_dev(jxlb200_ctx *ctx, const int32_t *avg, const int32_t *res, int32_t h_avg, int32_t w_avg,
     int32_t h_res, int32_t w_res, int32_t horizontal, int32_t *out) {
-    if (!ctx) return JXLB200_E_ARG;
-    if (!avg || !out || h_avg < 0 || w_avg < 0 || h_res < 0 || w_res < 0) return ctx->fail(JXLB200_E_ARG, "bad squeeze arguments");
-    if (horizontal) {
-        if ((w_avg != w_res && w_avg != 1 + w_res) || h_res != h_avg) return ctx->fail(JXLB200_E_ARG, "Corrupted squeeze transform");
-    } else {
-        if ((h_avg != h_res && h_avg != 1 + h_res) || w_res != w_avg) return ctx->fail(JXLB200_E_ARG, "Corrupted squeeze transform");
-    }
-    if (h_avg == 0 || w_avg == 0) return 0;
-    if (!res && h_res > 0 && w_res > 0) return ctx->fail(JXLB200_E_ARG, "bad squeeze arguments");
+    int rc = squeeze_check(ctx, avg, res, h_avg, w_avg, h_res, w_res, horizontal, out);
+    if (rc || h_avg == 0 || w_avg == 0) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     if (horizontal) k5_squeeze_h<<<ceil_div(h_avg, 32), 32, 0, ctx->stream>>>(avg, res, h_avg, w_avg, w_res, out);
     else k5_squeeze_v<<<ceil_div(w_avg, 128), 128, 0, ctx->stream>>>(avg, res, h_avg, h_res, w_avg, out);
@@ -1494,24 +1548,16 @@ int32_t jxlb200_modular_squeeze_dev(jxlb200_ctx *ctx, const int32_t *avg, const 
 
 int32_t jxlb200_modular_palette_dev(jxlb200_ctx *ctx, const int32_t *idx, const int32_t *palette, int32_t h, int32_t w,
     int32_t num_c, int32_t nb_colors, int32_t nb_deltas, int32_t d_pred, int32_t bit_depth, int32_t *const out[]) {
-    if (!ctx) return JXLB200_E_ARG;
-    if (!idx || !out || h < 0 || w < 0 || num_c < 1 || nb_colors < 0 || (nb_colors > 0 && !palette))
-        return ctx->fail(JXLB200_E_ARG, "bad palette arguments");
-    if (d_pred < 0 || d_pred > 13) return ctx->fail(JXLB200_E_ARG, "d_pred outside 0..13");
-    if (d_pred == 6) return ctx->fail(JXLB200_E_UNSUPPORTED, "palette delta with the weighted predictor (reference dereferences null pred[][])");
-    if (h == 0 || w == 0) return 0;
+    int rc = palette_check(ctx, idx, palette, h, w, num_c, nb_colors, d_pred, out);
+    if (rc || h == 0 || w == 0) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    if (!ctx->flags.p) {
-        CUDA_TRY(ctx, ctx->flags.ensure(sizeof(int) * 4));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->flags.p, 0, sizeof(int) * 4, ctx->stream));
-    }
+    CUDA_TRY(ctx, ensure_flags(ctx, ctx->stream));
     int *any = ctx->flags.as<int>() + 1;
     PalArgs A{idx, palette, h, w, num_c, nb_colors, nb_deltas, d_pred, bit_depth};
     const long long n = (long long)h * w;
     const int grid = (int)min((long long)ctx->sms * 8, (n + 255) / 256);
     CUDA_TRY(ctx, cudaMemsetAsync(any, 0, sizeof(int), ctx->stream));
     for (int c = 0; c < num_c; c++) {
-        if (!out[c]) return ctx->fail(JXLB200_E_ARG, "NULL palette output channel");
         k4_palette_gather<<<grid, 256, 0, ctx->stream>>>(A, c, out[c], any);
         ctx->launches++;
     }
@@ -1525,67 +1571,46 @@ int32_t jxlb200_modular_palette_dev(jxlb200_ctx *ctx, const int32_t *idx, const 
 }
 
 int32_t jxlb200_modular_rct(jxlb200_ctx *ctx, int32_t *const ch[3], int32_t h, int32_t w, int32_t rct_type) {
-    if (!ctx) return JXLB200_E_ARG;
-    if (!ch || !ch[0] || !ch[1] || !ch[2] || h < 0 || w < 0) return ctx->fail(JXLB200_E_ARG, "bad RCT arguments");
-    if (h == 0 || w == 0) return (rct_type < 0 || rct_type >= 42) ? ctx->fail(JXLB200_E_ARG, "rct_type outside 0..41") : 0;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t bytes = sizeof(int32_t) * (size_t)h * w;
-    CUDA_TRY(ctx, ctx->mod.ensure(3 * bytes));
-    int32_t *d[3];
-    for (int c = 0; c < 3; c++) {
-        d[c] = (int32_t *)((char *)ctx->mod.p + c * bytes);
-        CUDA_TRY(ctx, cudaMemcpyAsync(d[c], ch[c], bytes, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    int rc = jxlb200_modular_rct_dev(ctx, d, h, w, rct_type);
-    if (rc) return rc;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(ch[c], d[c], bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return 0;
+    int rc = rct_check(ctx, ch, h, w, rct_type);
+    if (rc || h == 0 || w == 0) return rc;
+    Staged r[3];
+    for (int c = 0; c < 3; c++) r[c] = {&ctx->mod, ch[c], ch[c], sizeof(int32_t) * h * w};
+    if ((rc = stage_in(ctx, r, 3))) return rc;
+    if ((rc = jxlb200_modular_rct_dev(ctx, planes_of<int32_t>(r).data(), h, w, rct_type))) return rc;
+    return stage_out(ctx, r, 3);
 }
 
 int32_t jxlb200_modular_squeeze(jxlb200_ctx *ctx, const int32_t *avg, const int32_t *res, int32_t h_avg, int32_t w_avg,
     int32_t h_res, int32_t w_res, int32_t horizontal, int32_t *out) {
-    if (!ctx) return JXLB200_E_ARG;
-    if (!avg || !out || h_avg < 0 || w_avg < 0 || h_res < 0 || w_res < 0) return ctx->fail(JXLB200_E_ARG, "bad squeeze arguments");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t na = (size_t)h_avg * w_avg, nr = (size_t)h_res * w_res, no = na + nr;
-    if (na == 0) return jxlb200_modular_squeeze_dev(ctx, avg, res, h_avg, w_avg, h_res, w_res, horizontal, out);
-    CUDA_TRY(ctx, ctx->mod.ensure(sizeof(int32_t) * (na + nr + no + 4)));
-    int32_t *da = ctx->mod.as<int32_t>(), *dr = da + na, *dout = dr + nr;
-    CUDA_TRY(ctx, cudaMemcpyAsync(da, avg, sizeof(int32_t) * na, cudaMemcpyHostToDevice, ctx->stream));
-    if (nr) CUDA_TRY(ctx, cudaMemcpyAsync(dr, res, sizeof(int32_t) * nr, cudaMemcpyHostToDevice, ctx->stream));
-    int rc = jxlb200_modular_squeeze_dev(ctx, da, dr, h_avg, w_avg, h_res, w_res, horizontal, dout);
-    if (rc) return rc;
-    CUDA_TRY(ctx, cudaMemcpyAsync(out, dout, sizeof(int32_t) * no, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return 0;
+    int rc = squeeze_check(ctx, avg, res, h_avg, w_avg, h_res, w_res, horizontal, out);
+    if (rc || h_avg == 0 || w_avg == 0) return rc;
+    const size_t na = (size_t)h_avg * w_avg, nr = (size_t)h_res * w_res;
+    Staged r[3] = {{&ctx->mod, avg, nullptr, sizeof(int32_t) * na}, {&ctx->mod, res, nullptr, sizeof(int32_t) * nr},
+                   {&ctx->mod, nullptr, out, sizeof(int32_t) * (na + nr)}};
+    if ((rc = stage_in(ctx, r, 3))) return rc;
+    if ((rc = jxlb200_modular_squeeze_dev(ctx, (const int32_t *)r[0].dev, (const int32_t *)r[1].dev, h_avg, w_avg, h_res, w_res,
+                                          horizontal, (int32_t *)r[2].dev)))
+        return rc;
+    return stage_out(ctx, r, 3);
 }
 
 int32_t jxlb200_modular_palette(jxlb200_ctx *ctx, const int32_t *idx, const int32_t *palette, int32_t h, int32_t w,
     int32_t num_c, int32_t nb_colors, int32_t nb_deltas, int32_t d_pred, int32_t bit_depth, int32_t *const out[]) {
-    if (!ctx) return JXLB200_E_ARG;
-    if (!idx || !out || h < 0 || w < 0 || num_c < 1 || num_c > 4096 || nb_colors < 0 || (nb_colors > 0 && !palette))
-        return ctx->fail(JXLB200_E_ARG, "bad palette arguments");
-    if (h == 0 || w == 0) return 0;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)h * w, np = (size_t)num_c * nb_colors;
-    CUDA_TRY(ctx, ctx->mod.ensure(sizeof(int32_t) * (n + np + (size_t)num_c * n + 4)));
-    int32_t *di = ctx->mod.as<int32_t>(), *dp = di + n, *dout = dp + np;
-    CUDA_TRY(ctx, cudaMemcpyAsync(di, idx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, ctx->stream));
-    if (np) CUDA_TRY(ctx, cudaMemcpyAsync(dp, palette, sizeof(int32_t) * np, cudaMemcpyHostToDevice, ctx->stream));
-    int32_t **outs = (int32_t **)malloc(sizeof(int32_t *) * num_c);
-    for (int c = 0; c < num_c; c++) outs[c] = dout + (size_t)c * n;
-    int rc = jxlb200_modular_palette_dev(ctx, di, dp, h, w, num_c, nb_colors, nb_deltas, d_pred, bit_depth, outs);
-    if (!rc)
-        for (int c = 0; c < num_c && !rc; c++) {
-            if (!out[c]) { rc = ctx->fail(JXLB200_E_ARG, "NULL palette output channel"); break; }
-            cudaError_t e = cudaMemcpyAsync(out[c], outs[c], sizeof(int32_t) * n, cudaMemcpyDeviceToHost, ctx->stream);
-            if (e != cudaSuccess) rc = ctx->fail(JXLB200_E_CUDA, "cudaMemcpyAsync", e);
-        }
-    free(outs);
-    if (rc) return rc;
-    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return 0;
+    if (ctx && num_c > 4096) return ctx->fail(JXLB200_E_ARG, "bad palette arguments");   // before palette_check reads out[0 .. num_c)
+    int rc = palette_check(ctx, idx, palette, h, w, num_c, nb_colors, d_pred, out);
+    if (rc || h == 0 || w == 0) return rc;
+    const size_t n = (size_t)h * w;
+    std::vector<Staged> r(2 + num_c);
+    r[0] = {&ctx->mod, idx, nullptr, sizeof(int32_t) * n};
+    r[1] = {&ctx->mod, palette, nullptr, sizeof(int32_t) * num_c * nb_colors};
+    for (int c = 0; c < num_c; c++) r[2 + c] = {&ctx->mod, nullptr, out[c], sizeof(int32_t) * n};
+    if ((rc = stage_in(ctx, r.data(), 2 + num_c))) return rc;
+    std::vector<int32_t *> dout(num_c);
+    for (int c = 0; c < num_c; c++) dout[c] = (int32_t *)r[2 + c].dev;
+    if ((rc = jxlb200_modular_palette_dev(ctx, (const int32_t *)r[0].dev, (const int32_t *)r[1].dev, h, w, num_c, nb_colors, nb_deltas,
+                                          d_pred, bit_depth, dout.data())))
+        return rc;
+    return stage_out(ctx, r.data(), 2 + num_c);
 }
 
 
@@ -1756,16 +1781,11 @@ static int upsample_enqueue(jxlb200_ctx *ctx, const float *d_in, int32_t h, int3
 int32_t jxlb200_upsample(jxlb200_ctx *ctx, const float *in, int32_t h, int32_t w, int32_t k, const float *weights, float *out) {
     int rc = upsample_check(ctx, in, h, w, k, weights, out);
     if (rc) return rc;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)h * w;
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * (n + n * k * k)));
-    float *d_in = ctx->blend.as<float>(), *d_out = d_in + n;
-    cudaStream_t st = ctx->stream;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_in, in, sizeof(float) * n, cudaMemcpyHostToDevice, st));
-    if ((rc = upsample_enqueue(ctx, d_in, h, w, k, weights, d_out))) return rc;
-    CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, sizeof(float) * n * k * k, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    return 0;
+    Staged r[2] = {{&ctx->blend, in, nullptr, sizeof(float) * n}, {&ctx->blend, nullptr, out, sizeof(float) * n * k * k}};
+    if ((rc = stage_in(ctx, r, 2))) return rc;
+    if ((rc = upsample_enqueue(ctx, (const float *)r[0].dev, h, w, k, weights, (float *)r[1].dev))) return rc;
+    return stage_out(ctx, r, 2);
 }
 int32_t jxlb200_upsample_dev(jxlb200_ctx *ctx, const float *in, int32_t h, int32_t w, int32_t k, const float *weights, float *out) {
     int rc = upsample_check(ctx, in, h, w, k, weights, out);
@@ -1806,16 +1826,11 @@ int32_t jxlb200_noise(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32
     const float lut[8], float base_corr_x, float base_corr_b) {
     int rc = noise_check(ctx, planes, h, w, group_dim, lut);
     if (rc) return rc;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)h * w;
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 3 * n));
-    float *d[3] = {ctx->blend.as<float>(), ctx->blend.as<float>() + n, ctx->blend.as<float>() + 2 * n};
-    cudaStream_t st = ctx->stream;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(d[c], planes[c], sizeof(float) * n, cudaMemcpyHostToDevice, st));
-    if ((rc = noise_enqueue(ctx, d, h, w, group_dim, seed0, lut, base_corr_x, base_corr_b))) return rc;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(planes[c], d[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    return 0;
+    Staged r[3];
+    for (int c = 0; c < 3; c++) r[c] = {&ctx->blend, planes[c], planes[c], sizeof(float) * h * w};
+    if ((rc = stage_in(ctx, r, 3))) return rc;
+    if ((rc = noise_enqueue(ctx, planes_of<float>(r).data(), h, w, group_dim, seed0, lut, base_corr_x, base_corr_b))) return rc;
+    return stage_out(ctx, r, 3);
 }
 int32_t jxlb200_noise_dev(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t group_dim, int64_t seed0,
     const float lut[8], float base_corr_x, float base_corr_b) {
@@ -1871,16 +1886,11 @@ int32_t jxlb200_splines(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int
     std::vector<SplineArcDev> arcs;
     int rc = splines_arcs(ctx, planes, h, w, num_splines, npoints, points, coeff, quant_adjust, base_corr_x, base_corr_b, arcs);
     if (rc || arcs.empty()) return rc;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)h * w;
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 3 * n));
-    float *d[3] = {ctx->blend.as<float>(), ctx->blend.as<float>() + n, ctx->blend.as<float>() + 2 * n};
-    cudaStream_t st = ctx->stream;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(d[c], planes[c], sizeof(float) * n, cudaMemcpyHostToDevice, st));
-    if ((rc = splines_enqueue(ctx, d, h, w, arcs))) return rc;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(planes[c], d[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    return 0;
+    Staged r[3];
+    for (int c = 0; c < 3; c++) r[c] = {&ctx->blend, planes[c], planes[c], sizeof(float) * h * w};
+    if ((rc = stage_in(ctx, r, 3))) return rc;
+    if ((rc = splines_enqueue(ctx, planes_of<float>(r).data(), h, w, arcs))) return rc;
+    return stage_out(ctx, r, 3);
 }
 int32_t jxlb200_splines_dev(jxlb200_ctx *ctx, float *const planes[3], int32_t h, int32_t w, int32_t num_splines, const int32_t *npoints,
     const int32_t *points, const int32_t *coeff, int32_t quant_adjust, float base_corr_x, float base_corr_b) {
@@ -1924,21 +1934,13 @@ int32_t jxlb200_lf_dequant(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float
     int32_t cfl, int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, float *const out[3]) {
     int rc = lf_check(ctx, hb, wb, scaled_dequant, lf_quant, extra_precision, out);
     if (rc) return rc;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)hb * wb;
-    CUDA_TRY(ctx, ctx->blend.ensure(sizeof(float) * 6 * n));
-    cudaStream_t st = ctx->stream;
-    const int32_t *dq[3];
-    float *dout[3];
-    for (int c = 0; c < 3; c++) {
-        dq[c] = ctx->blend.as<int32_t>() + c * n;
-        dout[c] = ctx->blend.as<float>() + (3 + c) * n;
-        CUDA_TRY(ctx, cudaMemcpyAsync((void *)dq[c], lf_quant[c], sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-    }
-    if ((rc = lf_enqueue(ctx, hb, wb, scaled_dequant, k_x, k_b, cfl, adaptive_smoothing, dq, extra_precision, dout))) return rc;
-    for (int c = 0; c < 3; c++) CUDA_TRY(ctx, cudaMemcpyAsync(out[c], dout[c], sizeof(float) * n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    return 0;
+    Staged r[6];
+    stage_planes(r, ctx->blend, lf_quant, ctx->blend, out, sizeof(float) * hb * wb);
+    if ((rc = stage_in(ctx, r, 6))) return rc;
+    if ((rc = lf_enqueue(ctx, hb, wb, scaled_dequant, k_x, k_b, cfl, adaptive_smoothing, planes_of<const int32_t>(r).data(), extra_precision,
+                         planes_of<float>(r + 3).data())))
+        return rc;
+    return stage_out(ctx, r, 6);
 }
 int32_t jxlb200_lf_dequant_dev(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const float scaled_dequant[3], float k_x, float k_b,
     int32_t cfl, int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, float *const out[3]) {
@@ -1975,20 +1977,15 @@ int32_t jxlb200_pack_samples(jxlb200_ctx *ctx, const void *const planes[], const
     int32_t n_channels, int32_t n_color, int32_t linear, int32_t h, int32_t w, int32_t bits, uint8_t *out) {
     int rc = pack_check(ctx, planes, is_int, depth, n_channels, h, w, bits, out);
     if (rc) return rc;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)h * w, obytes = n * n_channels * (bits > 8 ? 2 : 1);
-    CUDA_TRY(ctx, ctx->blend.ensure(4 * n * n_channels + obytes + 64));
-    cudaStream_t st = ctx->stream;
+    const size_t n = (size_t)h * w;
+    Staged r[9];
+    for (int c = 0; c < n_channels; c++) r[c] = {&ctx->blend, planes[c], nullptr, 4 * n};
+    r[n_channels] = {&ctx->blend, nullptr, out, n * n_channels * (bits > 8 ? 2 : 1)};
+    if ((rc = stage_in(ctx, r, n_channels + 1))) return rc;
     const void *d[8];
-    for (int c = 0; c < n_channels; c++) {
-        d[c] = ctx->blend.as<char>() + 4 * n * c;
-        CUDA_TRY(ctx, cudaMemcpyAsync((void *)d[c], planes[c], 4 * n, cudaMemcpyHostToDevice, st));
-    }
-    uint8_t *d_out = (uint8_t *)(ctx->blend.as<char>() + ((4 * n * n_channels + 63) & ~(size_t)63));
-    if ((rc = pack_enqueue(ctx, d, is_int, depth, n_channels, n_color, linear, h, w, bits, 0, d_out))) return rc;
-    CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, obytes, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    return 0;
+    for (int c = 0; c < n_channels; c++) d[c] = r[c].dev;
+    if ((rc = pack_enqueue(ctx, d, is_int, depth, n_channels, n_color, linear, h, w, bits, 0, (uint8_t *)r[n_channels].dev))) return rc;
+    return stage_out(ctx, r, n_channels + 1);
 }
 int32_t jxlb200_pack_samples_dev(jxlb200_ctx *ctx, const void *const planes[], const int32_t is_int[], const int32_t depth[],
     int32_t n_channels, int32_t n_color, int32_t linear, int32_t h, int32_t w, int32_t bits, int32_t layout, uint8_t *out) {

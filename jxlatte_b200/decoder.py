@@ -23,7 +23,7 @@ import zlib
 import numpy as np
 
 from . import frontend, host
-from .params import FrameParams
+from .params import STATE_MAPS, FrameParams, check_planes, check_state_shapes
 from .upsampling import up_weights
 
 ENC_VARDCT, ENC_MODULAR = 0, 1
@@ -370,24 +370,11 @@ class DeviceEngine(CudaEngine):
 
     # ---- stages ----
     def _reconstruct(self, p, st):
-        H, W = p.height, p.width
-        hb, wb, th, tw = H // 8, W // 8, (H + 63) // 64, (W + 63) // 64
-        q = [self.upload(st["qcoeff"][c], np.int32) for c in range(3)]
-        lf = [self.upload(st["lf"][c], np.float32) for c in range(3)]
-        for c in range(3):      # chroma-subsampled channels carry their own (H >> sy) x (W >> sx) planes
-            sy, sx = p.shift_y[c], p.shift_x[c]
-            if tuple(q[c].shape) != (H >> sy, W >> sx) or tuple(lf[c].shape) != (hb >> sy, wb >> sx):
-                raise ValueError("qcoeff[%d] / lf[%d] have shapes %s / %s, expected %s / %s" % (
-                    c, c, tuple(q[c].shape), tuple(lf[c].shape), (H >> sy, W >> sx), (hb >> sy, wb >> sx)))
-        maps = {}
-        for k, dt, shp in (("dct_select", np.uint8, (hb, wb)), ("block_origin", np.uint8, (hb, wb)), ("hf_mul", np.int32, (hb, wb)),
-                           ("x_from_y", np.int32, (th, tw)), ("b_from_y", np.int32, (th, tw)), ("sharpness", np.int32, (hb, wb))):
-            maps[k] = self.upload(st[k], dt)
-            if tuple(maps[k].shape) != shp:
-                raise ValueError("%s has shape %s, expected %s" % (k, tuple(maps[k].shape), shp))
-        out = self.empty((3, H, W))
-        self.rec.reconstruct_dev(p, [a.data_ptr() for a in q], [a.data_ptr() for a in lf],
-                                 *[maps[k].data_ptr() for k in ("dct_select", "block_origin", "hf_mul", "x_from_y", "b_from_y", "sharpness")],
+        a = dict(qcoeff=[self.upload(st["qcoeff"][c], np.int32) for c in range(3)], lf=[self.upload(st["lf"][c], np.float32) for c in range(3)])
+        a.update((k, self.upload(st[k], dt)) for k, dt in STATE_MAPS)
+        check_state_shapes(p, a)
+        out = self.empty((3, p.height, p.width))
+        self.rec.reconstruct_dev(p, [t.data_ptr() for t in a["qcoeff"]], [t.data_ptr() for t in a["lf"]], *[a[k].data_ptr() for k, _ in STATE_MAPS],
                                  [out[c].data_ptr() for c in range(3)])
         return out
 
@@ -404,10 +391,7 @@ class DeviceEngine(CudaEngine):
         return _DeviceModularTransforms(_DeviceModularOps(self), bit_depth).applyTransforms([self.upload(c, np.int32) for c in channels], transforms)
 
     def _planes3(self, p, planes):
-        inp = [self.upload(planes[c], np.float32) for c in range(3)]
-        if any(tuple(a.shape) != (p.height, p.width) for a in inp):
-            raise ValueError("planes have shape %s, expected %s" % (tuple(inp[0].shape), (p.height, p.width)))
-        return inp
+        return check_planes(p, [self.upload(planes[c], np.float32) for c in range(3)])
 
     def color(self, p, planes):
         inp = self._planes3(p, planes)

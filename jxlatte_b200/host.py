@@ -21,7 +21,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import QmParams, Slab  # noqa: F401
-from .params import FrameParams
+from .params import STATE_MAPS, FrameParams, check_planes, check_state_shapes
 
 
 class InvalidBitstreamError(IOError):
@@ -61,6 +61,32 @@ def narrow_coefficients(qcoeff):
             a = a.astype(np.int16)
         out.append(np.ascontiguousarray(a))
     return out
+
+
+def _spline_arrays(splines):
+    npts = np.array([len(s["points"]) // 2 for s in splines], np.int32)
+    pts = np.array([v for s in splines for v in s["points"]], np.int32)
+    cf = np.array([v for s in splines for v in s["coeff"]], np.int32)
+    return npts, pts, cf
+
+
+def _extra_precision(extra_precision, hb, wb):
+    ep = _c(np.asarray(extra_precision).reshape(-1), np.uint8)
+    if ep.size != ((hb + 255) // 256) * ((wb + 255) // 256):
+        raise ValueError("extra_precision must hold one byte per LF group")
+    return ep
+
+
+def _upsampling_weights(weights, k):
+    wt = _c(weights, np.float32)
+    if wt.shape != (k, k, 5, 5):
+        raise ValueError("weights must be [k][k][5][5]")
+    return wt
+
+
+def _pack_args(ptrs, is_int, depths):
+    """The plane pointer, is_int and depth arrays of jxlb200_pack_samples[_dev]."""
+    return (C.c_void_p * len(ptrs))(*ptrs), np.array([1 if v else 0 for v in is_int], np.int32), np.array(depths, np.int32)
 
 
 def qm_default_params():
@@ -180,45 +206,27 @@ class Reconstructor:
         self._weights = (w, off)
 
     # -- VarDCT --
-    def _state_args(self, st, H, W, with_sharp, qdtype=np.int32):
-        hb, wb, th, tw = H // 8, W // 8, (H + 63) // 64, (W + 63) // 64
-        q = [_c(st["qcoeff"][c], qdtype) for c in range(3)]
-        lf = [_c(st["lf"][c], np.float32) for c in range(3)]
-        ds, bo = _c(st["dct_select"], np.uint8), _c(st["block_origin"], np.uint8)
-        hm = _c(st["hf_mul"], np.int32)
-        xf, bf = _c(st["x_from_y"], np.int32), _c(st["b_from_y"], np.int32)
-        p = getattr(self, "_p_for_shapes", None)
-        for c in range(3):      # chroma-subsampled channels carry their own (H >> sy) x (W >> sx) planes
-            sy, sx = (p.shift_y[c], p.shift_x[c]) if p is not None else (0, 0)
-            if q[c].shape != (H >> sy, W >> sx) or lf[c].shape != (hb >> sy, wb >> sx):
-                raise ValueError("qcoeff[%d] / lf[%d] have shapes %s / %s, expected %s / %s" % (
-                    c, c, q[c].shape, lf[c].shape, (H >> sy, W >> sx), (hb >> sy, wb >> sx)))
-        for a, shp, nm in ((ds, (hb, wb), "dct_select"),
-                           (bo, (hb, wb), "block_origin"), (hm, (hb, wb), "hf_mul"), (xf, (th, tw), "x_from_y"),
-                           (bf, (th, tw), "b_from_y")):
-            if a.shape != shp:
-                raise ValueError("%s has shape %s, expected %s" % (nm, a.shape, shp))
-        sh = None
-        if with_sharp:
-            sh = _c(st["sharpness"], np.int32)
-            if sh.shape != (hb, wb):
-                raise ValueError("sharpness has shape %s, expected %s" % (sh.shape, (hb, wb)))
-        return q, lf, ds, bo, hm, xf, bf, sh
+    def _state_args(self, st, p, with_sharp, narrow=False, subsampled=True):
+        """qcoeff (int16 through narrow_coefficients when narrow), lf, then the STATE_MAPS (sharpness when with_sharp) as contiguous
+        arrays of their shapes."""
+        q = narrow_coefficients(st["qcoeff"]) if narrow else [_c(st["qcoeff"][c], np.int32) for c in range(3)]
+        a = dict(qcoeff=q, lf=[_c(st["lf"][c], np.float32) for c in range(3)])
+        a.update((k, _c(st[k], dt)) for k, dt in STATE_MAPS if with_sharp or k != "sharpness")
+        check_state_shapes(p, a, subsampled)
+        return tuple(a.values())
 
     def invertVarDCT(self, p, st):
         """bakeDequantizedCoeffs + invertVarDCT for every pass group of the frame -> XYB planes f32[3,H,W]."""
-        H, W = p.height, p.width
-        q, lf, ds, bo, hm, xf, bf, _ = self._state_args(st, H, W, False)
-        out = np.empty((3, H, W), np.float32)
+        # full-size planes only: stage 1 alone refuses chroma-subsampled frames (NotImplementedError from the library)
+        q, lf, ds, bo, hm, xf, bf = self._state_args(st, p, False, subsampled=False)
+        out = np.empty((3, p.height, p.width), np.float32)
         self._check(self._L.jxlb200_vardct_invert(
             self._h, C.byref(p), _lib.planes([_ptr(a) for a in q]), _lib.planes([_ptr(a) for a in lf]),
             _ptr(ds), _ptr(bo), _ptr(hm), _ptr(xf), _ptr(bf), _lib.planes([_ptr(out[c]) for c in range(3)])))
         return out
 
     def _stage(self, fn, p, planes_in, *extra):
-        inp = [_c(planes_in[c], np.float32) for c in range(3)]
-        if inp[0].shape != (p.height, p.width):
-            raise ValueError("planes have shape %s, expected %s" % (inp[0].shape, (p.height, p.width)))
+        inp = check_planes(p, [_c(planes_in[c], np.float32) for c in range(3)])
         out = np.empty((3, p.height, p.width), np.float32)
         self._check(fn(self._h, C.byref(p), _lib.planes([_ptr(a) for a in inp]), *extra,
                        _lib.planes([_ptr(out[c]) for c in range(3)])))
@@ -236,13 +244,8 @@ class Reconstructor:
 
     def restoreModularFrame(self, p, planes_in, epf_sigma_for_modular):
         """Gaborish + EPF (+ p.color_mode) of a Modular-encoded frame: one sigma for the frame (jxlb200_restore_uniform)."""
-        inp = [_c(planes_in[c], np.float32) for c in range(3)]
-        if inp[0].shape != (p.height, p.width):
-            raise ValueError("planes have shape %s, expected %s" % (inp[0].shape, (p.height, p.width)))
-        out = np.empty((3, p.height, p.width), np.float32)
-        self._check(self._L.jxlb200_restore_uniform(self._h, C.byref(p), C.c_float(float(epf_sigma_for_modular)),
-                                                    _lib.planes([_ptr(a) for a in inp]), _lib.planes([_ptr(out[c]) for c in range(3)])))
-        return out
+        sigma = C.c_float(float(epf_sigma_for_modular))
+        return self._stage(lambda h, pp, inp, out: self._L.jxlb200_restore_uniform(h, pp, sigma, inp, out), p, planes_in)
 
     def performColorTransforms(self, p, planes_in):
         return self._stage(self._L.jxlb200_color_transform, p, planes_in)
@@ -252,17 +255,9 @@ class Reconstructor:
 
         narrow=True sends the coefficients as int16 (jxlb200_vardct_reconstruct_i16: half the upload, same result);
         planes that already are int16 go as they are, int32 planes are range-checked and narrowed here."""
-        H, W = p.height, p.width
-        self._p_for_shapes = p
-        try:
-            if narrow:
-                st = dict(st)
-                st["qcoeff"] = narrow_coefficients(st["qcoeff"])
-            q, lf, ds, bo, hm, xf, bf, sh = self._state_args(st, H, W, True, np.int16 if narrow else np.int32)
-        finally:
-            self._p_for_shapes = None
+        q, lf, ds, bo, hm, xf, bf, sh = self._state_args(st, p, True, narrow)
         if out is None:
-            out = np.empty((3, H, W), np.float32)
+            out = np.empty((3, p.height, p.width), np.float32)
         fn = self._L.jxlb200_vardct_reconstruct_i16 if narrow else self._L.jxlb200_vardct_reconstruct
         self._check(fn(
             self._h, C.byref(p), _lib.planes([_ptr(a) for a in q]), _lib.planes([_ptr(a) for a in lf]),
@@ -273,16 +268,8 @@ class Reconstructor:
         """The whole path ending in PNG-ready samples (jxlb200_vardct_reconstruct_packed): sRGB transfer (when `linear`),
         8/16-bit quantisation and R,G,B interleave on the device; returns uint8 [crop_h, crop_w, 3 * bits/8] (16-bit samples big
         endian, as PNGWriter writes them).  crop = (width, height) of the image inside the padded frame."""
-        H, W = p.height, p.width
-        cw, ch = crop if crop is not None else (W, H)
-        self._p_for_shapes = p
-        try:
-            if narrow:
-                st = dict(st)
-                st["qcoeff"] = narrow_coefficients(st["qcoeff"])
-            q, lf, ds, bo, hm, xf, bf, sh = self._state_args(st, H, W, True, np.int16 if narrow else np.int32)
-        finally:
-            self._p_for_shapes = None
+        cw, ch = crop if crop is not None else (p.width, p.height)
+        q, lf, ds, bo, hm, xf, bf, sh = self._state_args(st, p, True, narrow)
         nb = 3 * (2 if bits > 8 else 1)
         if out is None:
             out = np.empty((ch, cw, nb), np.uint8)
@@ -336,9 +323,10 @@ class Reconstructor:
     # -- upsampling (Frame.performUpsampling) --
     def performUpsampling(self, plane, k, weights):
         """One float32 channel h x w -> (h*k) x (w*k); weights float32 [k][k][5][5] (jxlatte_b200.upsampling.up_weights)."""
-        a, wt = _c(plane, np.float32), _c(weights, np.float32)
-        if a.ndim != 2 or wt.shape != (k, k, 5, 5):
-            raise ValueError("plane must be 2-D and weights [k][k][5][5]")
+        a = _c(plane, np.float32)
+        if a.ndim != 2:
+            raise ValueError("plane must be 2-D")
+        wt = _upsampling_weights(weights, k)
         out = np.empty((a.shape[0] * k, a.shape[1] * k), np.float32)
         self._check(self._L.jxlb200_upsample(self._h, _ptr(a), a.shape[0], a.shape[1], int(k), _ptr(wt), _ptr(out)))
         return out
@@ -358,9 +346,7 @@ class Reconstructor:
         """X, Y, B planes [3, h, w] -> planes with the splines drawn.  splines: [{"points": [x0, y0, ...], "coeff": 128 ints}]."""
         buf = [np.array(planes[c], dtype=np.float32, order="C", copy=True) for c in range(3)]
         h, w = buf[0].shape
-        npts = np.array([len(s["points"]) // 2 for s in splines], np.int32)
-        pts = np.array([v for s in splines for v in s["points"]], np.int32)
-        cf = np.array([v for s in splines for v in s["coeff"]], np.int32)
+        npts, pts, cf = _spline_arrays(splines)
         self._check(self._L.jxlb200_splines(self._h, _lib.planes([_ptr(a) for a in buf]), h, w, len(splines), _ptr(npts), _ptr(pts),
                                             _ptr(cf), int(quant_adjust), float(base_corr_x), float(base_corr_b)))
         return np.stack(buf)
@@ -371,9 +357,7 @@ class Reconstructor:
         ch = [np.ascontiguousarray(c if c.dtype == np.float32 else c.astype(np.int32)) for c in channels]
         h, w = ch[0].shape
         n = len(ch)
-        ptrs = (C.c_void_p * n)(*[c.ctypes.data for c in ch])
-        is_int = np.array([c.dtype != np.float32 for c in ch], np.int32)
-        dep = np.array(depths, np.int32)
+        ptrs, is_int, dep = _pack_args([c.ctypes.data for c in ch], [c.dtype != np.float32 for c in ch], depths)
         out = np.empty((h, w, n * (2 if bits > 8 else 1)), np.uint8)
         self._check(self._L.jxlb200_pack_samples(self._h, ptrs, _ptr(is_int), _ptr(dep), n, int(n_color), int(bool(linear)), h, w, int(bits), _ptr(out)))
         return out
@@ -399,9 +383,9 @@ class Reconstructor:
         order + extraPrecision per LF group -> the dequantised, smoothed `lf` planes of the reconstruction call."""
         q = [_c(lf_quant[c], np.int32) for c in range(3)]
         hb, wb = q[0].shape
-        ep = _c(np.asarray(extra_precision).reshape(-1), np.uint8)
-        if ep.size != ((hb + 255) // 256) * ((wb + 255) // 256) or any(a.shape != (hb, wb) for a in q):
-            raise ValueError("lf_quant planes must share a shape and extra_precision hold one byte per LF group")
+        if any(a.shape != (hb, wb) for a in q):
+            raise ValueError("lf_quant planes must share a shape")
+        ep = _extra_precision(extra_precision, hb, wb)
         sd = (C.c_float * 3)(*[float(v) for v in scaled_dequant])
         out = np.empty((3, hb, wb), np.float32)
         self._check(self._L.jxlb200_lf_dequant(self._h, hb, wb, sd, C.c_float(float(kx)), C.c_float(float(kb)), 1 if cfl else 0, 1 if smooth else 0,
@@ -426,9 +410,7 @@ class Reconstructor:
     # -- device-resident frame loop (jxlatte_b200.decoder.DeviceEngine): integers are CUdeviceptr values; enqueued, not synchronised --
     def lf_dequant_dev(self, hb, wb, scaled_dequant, kx, kb, cfl, smooth, lf_quant, extra_precision, out):
         """jxlb200_lf_dequant_dev: lf_quant / out are three device pointers each; extra_precision a host array (one byte per LF group)."""
-        ep = _c(np.asarray(extra_precision).reshape(-1), np.uint8)
-        if ep.size != ((hb + 255) // 256) * ((wb + 255) // 256):
-            raise ValueError("extra_precision must hold one byte per LF group")
+        ep = _extra_precision(extra_precision, hb, wb)
         sd = (C.c_float * 3)(*[float(v) for v in scaled_dequant])
         self._check(self._L.jxlb200_lf_dequant_dev(self._h, int(hb), int(wb), sd, C.c_float(float(kx)), C.c_float(float(kb)), 1 if cfl else 0,
                                                    1 if smooth else 0, _lib.planes(lf_quant), _ptr(ep), _lib.planes(out)))
@@ -441,9 +423,7 @@ class Reconstructor:
         self._check(self._L.jxlb200_color_transform_dev(self._h, C.byref(p), _lib.planes(planes_in), _lib.planes(out)))
 
     def upsample_dev(self, plane, h, w, k, weights, out):
-        wt = _c(weights, np.float32)
-        if wt.shape != (k, k, 5, 5):
-            raise ValueError("weights must be [k][k][5][5]")
+        wt = _upsampling_weights(weights, k)
         self._check(self._L.jxlb200_upsample_dev(self._h, plane, int(h), int(w), int(k), _ptr(wt), out))
 
     def noise_dev(self, planes, h, w, group_dim, seed0, lut, base_corr_x, base_corr_b):
@@ -452,9 +432,7 @@ class Reconstructor:
                                               float(base_corr_x), float(base_corr_b)))
 
     def splines_dev(self, planes, h, w, splines, quant_adjust, base_corr_x, base_corr_b):
-        npts = np.array([len(s["points"]) // 2 for s in splines], np.int32)
-        pts = np.array([v for s in splines for v in s["points"]], np.int32)
-        cf = np.array([v for s in splines for v in s["coeff"]], np.int32)
+        npts, pts, cf = _spline_arrays(splines)
         self._check(self._L.jxlb200_splines_dev(self._h, _lib.planes(planes), int(h), int(w), len(splines), _ptr(npts), _ptr(pts), _ptr(cf),
                                                 int(quant_adjust), float(base_corr_x), float(base_corr_b)))
 
@@ -469,9 +447,7 @@ class Reconstructor:
 
     def pack_samples_dev(self, planes, is_int, depths, n_color, linear, h, w, bits, layout, out):
         n = len(planes)
-        ptrs = (C.c_void_p * n)(*[int(p) for p in planes])
-        ii = np.array([1 if v else 0 for v in is_int], np.int32)
-        dep = np.array(depths, np.int32)
+        ptrs, ii, dep = _pack_args([int(p) for p in planes], is_int, depths)
         self._check(self._L.jxlb200_pack_samples_dev(self._h, ptrs, _ptr(ii), _ptr(dep), n, int(n_color), int(bool(linear)), int(h), int(w),
                                                      int(bits), int(layout), out))
 

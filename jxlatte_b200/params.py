@@ -80,3 +80,38 @@ def default_frame_params(width, height, *, epf_iters=3, gab=True, color_mode=COL
     p.opsin_bias[:] = [-0.0037930732552754493] * 3
     p.intensity_target = intensity_target
     return p
+
+
+# the per-block / per-tile maps of the VarDCT state, in the C ABI's argument order, and their dtypes
+STATE_MAPS = (("dct_select", np.uint8), ("block_origin", np.uint8), ("hf_mul", np.int32), ("x_from_y", np.int32), ("b_from_y", np.int32),
+              ("sharpness", np.int32))
+
+
+def state_shapes(p, subsampled=True):
+    """Expected shape of each VarDCT state array of a frame with params p: "qcoeff" and "lf" hold one shape per channel (a
+    chroma-subsampled channel is smaller by its shifts unless subsampled=False), the STATE_MAPS one shape each."""
+    H, W = p.height, p.width
+    hb, wb, th, tw = H // 8, W // 8, (H + 63) // 64, (W + 63) // 64
+    shifts = [(p.shift_y[c], p.shift_x[c]) if subsampled else (0, 0) for c in range(3)]
+    return dict(qcoeff=[(H >> sy, W >> sx) for sy, sx in shifts], lf=[(hb >> sy, wb >> sx) for sy, sx in shifts],
+                dct_select=(hb, wb), block_origin=(hb, wb), hf_mul=(hb, wb), x_from_y=(th, tw), b_from_y=(th, tw), sharpness=(hb, wb))
+
+
+def check_state_shapes(p, arrays, subsampled=True):
+    """ValueError unless every array of `arrays` (numpy or torch, keyed as in the state dict) has its state_shapes(p) shape."""
+    want = state_shapes(p, subsampled)
+    for c in range(3):
+        q, lf = tuple(arrays["qcoeff"][c].shape), tuple(arrays["lf"][c].shape)
+        if q != want["qcoeff"][c] or lf != want["lf"][c]:
+            raise ValueError("qcoeff[%d] / lf[%d] have shapes %s / %s, expected %s / %s" % (c, c, q, lf, want["qcoeff"][c], want["lf"][c]))
+    for k, a in arrays.items():
+        if k not in ("qcoeff", "lf") and tuple(a.shape) != want[k]:
+            raise ValueError("%s has shape %s, expected %s" % (k, tuple(a.shape), want[k]))
+
+
+def check_planes(p, planes):
+    """The three colour planes of a frame, each p.height x p.width (numpy or torch); ValueError otherwise."""
+    for a in planes:
+        if tuple(a.shape) != (p.height, p.width):
+            raise ValueError("planes have shape %s, expected %s" % (tuple(a.shape), (p.height, p.width)))
+    return planes
