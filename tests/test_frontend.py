@@ -234,7 +234,7 @@ def test_upsampling_kernel_exact(recon, k):
     from oracle import oracle as orc
     from jxlatte_b200.upsampling import up_weights
     rng = np.random.default_rng(k)
-    for shape in ((37, 61), (2, 3), (1, 1), (64, 5)):
+    for shape in ((37, 61), (2, 3), (1, 1), (64, 5), (1, 2), (2, 1), (1, 45), (45, 1)):
         a = rng.uniform(-1.0, 1.5, shape).astype(np.float32)
         wts = up_weights(k)
         assert np.array_equal(recon.performUpsampling(a, k, wts), orc.upsample(a, k, wts))
@@ -265,6 +265,28 @@ def test_spline_rendering_matches_oracle(recon):
           {"points": [10, 190, 310, 10], "coeff": [1] * 128}]
     got, want = recon.renderSplines(pl, sp, 2, 0.0, 1.0), orc.splines(pl, sp, 2, 0.0, 1.0)
     assert float(np.abs(want - pl).max()) > 0.05                       # something was drawn
+    assert float(np.abs(got - want).max()) <= 1e-6
+    assert float((got != want).mean()) < 1e-4
+
+
+@pytest.mark.gpu
+def test_spline_rendering_edges_match_oracle(recon):
+    """More than K8_ARC_CHUNK (128) arcs in one call, so k8_splines stages several chunks; arcs whose boxes straddle 32 x 8 tile
+    edges and the canvas edge; control points off the canvas on every side."""
+    from oracle import oracle as orc
+    rng = np.random.default_rng(6)
+    h, w = 70, 100
+    pl = rng.uniform(0, 0.5, (3, h, w)).astype(np.float32)
+    coeff = [0] * 128
+    coeff[0], coeff[32], coeff[64], coeff[96], coeff[34], coeff[98] = 40, 700, 250, 10, 60, -2
+    sp = [{"points": [-30, 12, 40, 8, 96, 31, 130, 64], "coeff": coeff},                  # enters on the left, leaves on the right
+          {"points": [31, -20, 33, 40, 64, 90], "coeff": coeff},                          # runs along the tile column edge x = 32
+          {"points": [0, 0, 99, 69], "coeff": coeff},                                     # corner to corner
+          {"points": [-5, 75, 105, -6], "coeff": coeff},                                  # both ends off the canvas
+          {"points": [50, 7], "coeff": coeff}]                                            # one point on a tile row edge
+    got, want = recon.renderSplines(pl, sp, 1, 0.0, 1.0), orc.splines(pl, sp, 1, 0.0, 1.0)
+    assert float(np.abs(want - pl).max()) > 0.05
+    assert (np.abs(want - pl).max(axis=0)[[0, -1]] > 1e-3).any() and (np.abs(want - pl).max(axis=0)[:, [0, -1]] > 1e-3).any()
     assert float(np.abs(got - want).max()) <= 1e-6
     assert float((got != want).mean()) < 1e-4
 

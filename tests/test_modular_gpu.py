@@ -61,6 +61,25 @@ def test_palette_with_deltas_every_predictor(recon, orc, d_pred, bit_depth):
     assert np.array_equal(got, ref)
 
 
+@pytest.mark.parametrize("d_pred", [0, 1, 2, 3, 4, 5, 7, 8, 9, 10, 11, 12, 13])
+def test_palette_with_deltas_across_row_bands(recon, orc, d_pred):
+    """k4_palette_delta runs as one 1024-thread CTA sweeping bands of 1024 rows: heights at, one past and two bands past the band
+    size, and widths of 1, 2, 3 and 61 columns, where the predictors' north / west fallbacks decide most samples."""
+    rng = np.random.default_rng(1000 + d_pred)
+    num_c, nb_colors, nb_deltas = 3, 20, 6
+    palette = _rand(rng, (num_c, nb_colors), 0, 256)
+    for h in (1024, 1025, 2100):
+        for w in (1, 2, 3, 61):
+            idx = rng.integers(0, nb_colors, size=(h, w)).astype(np.int32)
+            m = rng.random((h, w))
+            idx[m < 0.3] = rng.integers(0, nb_deltas, size=int((m < 0.3).sum()))          # delta entries: predicted + palette
+            idx[(m >= 0.3) & (m < 0.35)] = rng.integers(nb_colors, nb_colors + 64, size=int(((m >= 0.3) & (m < 0.35)).sum()))
+            idx[(m >= 0.35) & (m < 0.4)] = -rng.integers(1, 300, size=int(((m >= 0.35) & (m < 0.4)).sum()))
+            ref = orc.modular_palette(idx, palette, nb_deltas, d_pred, 8)
+            got = np.stack(recon.inversePalette(idx, palette, nb_deltas, d_pred, 8))
+            assert np.array_equal(got, ref), "%dx%d: first difference at %s" % (h, w, np.argwhere(got != ref)[:1].tolist())
+
+
 def test_palette_without_deltas_is_a_gather(recon, orc):
     rng = np.random.default_rng(2)
     palette = _rand(rng, (4, 256), 0, 256)

@@ -7,9 +7,11 @@ import pytest
 from jxlatte_b200 import synth, default_frame_params, _lib
 from jxlatte_b200.host import qm_generate, Slab
 from jxlatte_b200.multigpu import slab_rows, split_state
+from kernel_trace import assert_stage2_kernel, launched_kernels
 
 pytestmark = pytest.mark.gpu
 HALO = _lib.HALO_ROWS
+FORCED = {_lib.STAGE2_STREAM: "stream", _lib.STAGE2_TILE: "tile", _lib.STAGE2_STAGED: "staged"}
 
 
 @pytest.mark.parametrize("cfg", [dict(W=328, H=776, parts=3, iters=3, gab=True), dict(W=512, H=512, parts=2, iters=1, gab=True),
@@ -23,7 +25,9 @@ def test_slabs_match_whole_frame(recon, cfg, stage2):
     st = synth.make_state(W, H, seed=5 + W, params=p, qm_weights=qw, qm_offsets=qo)
     recon.set_option(_lib.OPT_STAGE2, stage2)
     try:
-        whole = recon.reconstruct(p, st)
+        whole, kernels = launched_kernels(lambda: recon.reconstruct(p, st))
+        if stage2 in FORCED:
+            assert_stage2_kernel(kernels, FORCED[stage2], p)
         dev = torch.device("cuda", 0)
         spans = [slab_rows(H, parts, r) for r in range(parts)]
         wb = W // 8
@@ -59,9 +63,11 @@ def test_slabs_match_whole_frame(recon, cfg, stage2):
             out = torch.empty((3, rows, W), dtype=torch.float32, device=dev)
             slab = Slab(y0, rows, H, 1 if i > 0 else 0, 1 if i < parts - 1 else 0)
             base = [xybs[i][c].data_ptr() + HALO * W * 4 for c in range(3)]
-            recon.restore_dev(ps[i], slab, base, W, maps[i][0].data_ptr() + wb * 4, maps[i][1].data_ptr() + wb * 4,
-                              [out[c].data_ptr() for c in range(3)])
-            recon.sync()
+            _, kernels = launched_kernels(lambda: (recon.restore_dev(ps[i], slab, base, W, maps[i][0].data_ptr() + wb * 4,
+                                                                     maps[i][1].data_ptr() + wb * 4, [out[c].data_ptr() for c in range(3)]),
+                                                   recon.sync()))
+            if stage2 in FORCED:
+                assert_stage2_kernel(kernels, FORCED[stage2], ps[i])
             got[:, y0:y0 + rows] = out.cpu().numpy()
     finally:
         recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
@@ -88,13 +94,16 @@ def test_batch_of_stacked_frames_matches_single_frames(recon, orc, cfg, stage2):
     out = torch.full((3, H * n, W), np.nan, dtype=torch.float32, device=dev)
     recon.set_option(_lib.OPT_STAGE2, stage2)      # the stack goes through the stream kernel as one launch when forced (or large enough)
     try:
-        recon.reconstruct_batch_dev(p, n, [d["qcoeff"][c].data_ptr() for c in range(3)], [d["lf"][c].data_ptr() for c in range(3)],
-                                    d["dct_select"].data_ptr(), d["block_origin"].data_ptr(), d["hf_mul"].data_ptr(),
-                                    d["x_from_y"].data_ptr(), d["b_from_y"].data_ptr(), d["sharpness"].data_ptr(),
-                                    [out[c].data_ptr() for c in range(3)])
-        recon.sync()
+        _, kernels = launched_kernels(lambda: (
+            recon.reconstruct_batch_dev(p, n, [d["qcoeff"][c].data_ptr() for c in range(3)], [d["lf"][c].data_ptr() for c in range(3)],
+                                        d["dct_select"].data_ptr(), d["block_origin"].data_ptr(), d["hf_mul"].data_ptr(),
+                                        d["x_from_y"].data_ptr(), d["b_from_y"].data_ptr(), d["sharpness"].data_ptr(),
+                                        [out[c].data_ptr() for c in range(3)]),
+            recon.sync()))
     finally:
         recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
+    if stage2 == _lib.STAGE2_STREAM:
+        assert_stage2_kernel(kernels, "stream", p)
     got = out.cpu().numpy()
     for f in range(n):
         assert np.array_equal(got[:, f * H:(f + 1) * H], singles[f]), "frame %d of the stack differs" % f

@@ -12,6 +12,7 @@ from jxlatte_b200 import synth, default_frame_params
 from jxlatte_b200 import _lib
 from jxlatte_b200.host import InvalidBitstreamError, qm_generate
 from jxlatte_b200.params import TRANSFORM_TYPES, TRANSFORM_NAMES
+from kernel_trace import assert_stage2_kernel, launched_kernels
 
 pytestmark = pytest.mark.gpu
 
@@ -121,17 +122,17 @@ def test_epf_with_non_positive_hf_multipliers(recon, orc, iters, stage2):
     assert np.isfinite(ref).all()
     recon.set_option(_lib.OPT_STAGE2, {"stream": _lib.STAGE2_STREAM, "tile": _lib.STAGE2_TILE, "staged": _lib.STAGE2_STAGED}[stage2])
     try:
-        got = recon.performEdgePreservingFilter(p, planes, hm, sh)
+        got, kernels = launched_kernels(lambda: recon.performEdgePreservingFilter(p, planes, hm, sh))
     finally:
         recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
+    assert_stage2_kernel(kernels, stage2, p)
     assert np.array_equal(got, ref), "max abs err %g" % np.abs(got - ref).max()
 
 
-def test_stream_kernel_random_shapes(recon):
-    """The stream kernel (forced) against the staged kernels on thirty random frame shapes and filter settings, through the whole
+def test_stream_kernel_random_shapes(recon, orc):
+    """The stream kernel (forced) against the oracle on thirty random frame shapes and filter settings, through the whole
     reconstruction: widths from one 8-pixel block to several column strips with a ragged last strip, heights from one block row to several
-    chunks, every (gab, epf_iters >= 1).  The staged kernels are the simple form the fused ones are checked against; they are held to the
-    oracle elsewhere in this file."""
+    chunks, every (gab, epf_iters >= 1).  The kernel trace shows that k2_stream, not its fallback, made each result."""
     rng = np.random.default_rng(20261017)
     qw, qo = qm_generate()
     recon.setWeights(qw, qo)
@@ -141,15 +142,14 @@ def test_stream_kernel_random_shapes(recon):
         iters, gab = int(rng.integers(1, 4)), bool(rng.integers(0, 2))
         p = default_frame_params(W, H, epf_iters=iters, gab=gab)
         st = synth.make_state(W, H, seed=7000 + k, params=p, qm_weights=qw, qm_offsets=qo)
-        out = {}
-        for name, opt in (("stream", _lib.STAGE2_STREAM), ("staged", _lib.STAGE2_STAGED)):
-            recon.set_option(_lib.OPT_STAGE2, opt)
-            try:
-                out[name] = recon.reconstruct(p, st)
-            finally:
-                recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
-        assert np.array_equal(out["stream"], out["staged"]), "%dx%d gab %d epf %d: max abs diff %g" % (
-            W, H, gab, iters, np.abs(out["stream"] - out["staged"]).max())
+        recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_STREAM)
+        try:
+            got, kernels = launched_kernels(lambda: recon.reconstruct(p, st))
+        finally:
+            recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
+        assert_stage2_kernel(kernels, "stream", p)
+        want = orc.vardct_reconstruct(p, st, nthreads=8)
+        assert np.array_equal(got, want), "%dx%d gab %d epf %d: max abs err %g" % (W, H, gab, iters, np.abs(got - want).max())
 
 
 def test_epf_rejects_bad_sharpness(recon):
@@ -206,9 +206,11 @@ def test_full_reconstruction(recon, orc, cfg, stage2):
     except NotImplementedError:
         pytest.skip("library built without this opt-in stage-2 variant (-DJXLB200_WITH_PAIR)")
     try:
-        got = recon.reconstruct(p, st)
+        got, kernels = launched_kernels(lambda: recon.reconstruct(p, st))
     finally:
         recon.set_option(_lib.OPT_STAGE2, _lib.STAGE2_AUTO)
+    if stage2 in ("stream", "tile", "staged"):
+        assert_stage2_kernel(kernels, stage2, p)
     if stage2 != "fast":
         assert np.array_equal(got, ref), "%s path must be bit-identical; max abs err %g" % (stage2, np.abs(got - ref).max())
     err = np.abs(got - ref).max()
