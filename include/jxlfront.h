@@ -26,6 +26,12 @@ typedef struct jxlf_image jxlf_image;
 
 #define JXLF_HOST_TRANSFORMS 1 /* also undo the frame-level Modular transforms on the host (tests / cross-checks only) */
 #define JXLF_HEADERS_ONLY 2    /* stop after the first frame header + TOC */
+/* Parse every frame up to its LF image: LfGlobal and, in each LF group, the LF coefficients and the LF-group Modular channels.
+ * HF metadata, HfGlobal and the pass groups are skipped unread.  "lf", "lf_quant" and "lf_extra_precision" are what the full
+ * parse gives; the HF arrays ("qcoeff", "dct_select", "block_origin", "hf_mul", "sharpness", "x_from_y", "b_from_y") are
+ * not found; jxlf_describe adds "lf_only": true and leaves out the HfGlobal fields "quant_all_default" / "quant_params".
+ * Modular channels that pass groups fill stay empty, so JXLF_HOST_TRANSFORMS cannot be combined with it (status -1). */
+#define JXLF_LF_ONLY 4
 
 /* JXLDecoder(InputStream) + decode() up to the end of the codestream (J/JXLCodestreamDecoder.java:547-626): every frame is
  * entropy-decoded; nothing is rendered. */
@@ -37,6 +43,8 @@ const char *jxlf_error(const jxlf_image *image);
 const char *jxlf_describe(const jxlf_image *image);
 /* Arrays by name; *ptr stays owned by the image.  dtype: 0 int32, 1 float32, 2 uint8.
  *   "qcoeff", "lf"            index = channel (X, Y, B); frame-level planes, passes summed
+ *   "lf_quant"                index = channel (X, Y, B); the quantised LF before LFCoefficients' arithmetic, (hb >> sy) x (wb >> sx)
+ *   "lf_extra_precision"      one byte per LF group
  *   "dct_select", "block_origin", "hf_mul", "sharpness", "x_from_y", "b_from_y"
  *   "modular"                 index = channel of the frame-level modular stream (before its transforms are undone)
  *   "qraw"                    index = 3 * parameter set + channel (MODE_RAW quant tables)

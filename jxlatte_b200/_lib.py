@@ -94,6 +94,10 @@ SYMBOLS = {
     "jxlb200_pack_samples_dev": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "jxlb200_cast_to_float_dev": (_i32, [_vp, _vp, C.c_int64, C.c_float, _vp]),
     "jxlb200_modular_xyb_dev": (_i32, [_vp, _P3, C.c_int64, _vp, _P3]),
+    "jxlb200_lf_preview": (_i32, [_vp, _FP, _vp, C.c_float, C.c_float, _i32, _P3, _vp, _i32, _i32, _i32, _P3]),
+    "jxlb200_lf_preview_dev": (_i32, [_vp, _FP, _vp, C.c_float, C.c_float, _i32, _P3, _vp, _i32, _i32, _i32, _P3]),
+    "jxlb200_area_mean8": (_i32, [_vp, _i32, _P3, _vp, _vp, _i32, _i32, _P3]),
+    "jxlb200_area_mean8_dev": (_i32, [_vp, _i32, _P3, _vp, _vp, _i32, _i32, _P3]),
 }
 
 

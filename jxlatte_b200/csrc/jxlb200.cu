@@ -26,6 +26,7 @@
 #include "k7_blend.cuh"
 #include "k8_features.cuh"
 #include "k9_device.cuh"
+#include "k10_preview.cuh"
 #include "splines_host.cuh"
 #include "qm_tables.cuh"
 #include "split_nccl.cuh"
@@ -1948,6 +1949,139 @@ int32_t jxlb200_lf_dequant_dev(jxlb200_ctx *ctx, int32_t hb, int32_t wb, const f
     if (rc) return rc;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     return lf_enqueue(ctx, hb, wb, scaled_dequant, k_x, k_b, cfl, adaptive_smoothing, lf_quant, extra_precision, out);
+}
+
+
+// ---- 1:8 previews (k10_preview.cuh) ----
+static int preview_check(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float scaled_dequant[3], int32_t adaptive_smoothing,
+    const int32_t *const lf_quant[3], const uint8_t *extra_precision, int32_t n_extra_precision, int32_t out_h, int32_t out_w,
+    float *const out[3]) {
+    int rc = check_params(ctx, p);
+    if (rc) return rc;
+    if (!scaled_dequant || !lf_quant || !extra_precision || !out) return ctx->fail(JXLB200_E_ARG, "NULL pointer");
+    for (int c = 0; c < 3; c++)
+        if (!lf_quant[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+    const int hb = p->height >> 3, wb = p->width >> 3;
+    if (out_h < 1 || out_w < 1 || out_h > hb || out_w > wb) return ctx->fail(JXLB200_E_ARG, "preview size outside the frame's LF grid");
+    const int ng = ((wb + 255) >> 8) * ((hb + 255) >> 8);
+    if (n_extra_precision != ng) return ctx->fail(JXLB200_E_ARG, "extra_precision must hold one byte per LF group");
+    for (int g = 0; g < ng; g++)
+        if (extra_precision[g] > 3) return ctx->fail(JXLB200_E_STREAM, "extraPrecision is a 2-bit field");
+    const bool subsampled = p->shift_x[0] | p->shift_x[1] | p->shift_x[2] | p->shift_y[0] | p->shift_y[1] | p->shift_y[2];
+    if (subsampled && adaptive_smoothing) return ctx->fail(JXLB200_E_STREAM, "adaptive LF smoothing with chroma subsampling");
+    return 0;
+}
+static int preview_enqueue(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float scaled_dequant[3], float k_x, float k_b,
+    int32_t adaptive_smoothing, const int32_t *const d_q[3], const uint8_t *extra_precision, int32_t out_h, int32_t out_w,
+    float *const d_out[3]) {
+    PreviewArgs A;
+    LfArgs &L = A.lf;
+    L.hb = p->height >> 3; L.wb = p->width >> 3;
+    L.gcols = (L.wb + 255) >> 8;
+    const int ng = L.gcols * ((L.hb + 255) >> 8);
+    cudaStream_t st = ctx->stream;
+    CUDA_TRY(ctx, ctx->dtab.ensure(ng));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->dtab.p, extra_precision, ng, cudaMemcpyHostToDevice, st));
+    L.ep = ctx->dtab.as<uint8_t>();
+    A.subsampled = 0;
+    for (int c = 0; c < 3; c++) {
+        L.q[c] = d_q[c]; L.out[c] = nullptr; L.sd[c] = scaled_dequant[c];
+        A.sy[c] = p->shift_y[c]; A.sx[c] = p->shift_x[c];
+        A.subsampled |= A.sy[c] | A.sx[c];
+        A.out[c] = d_out[c];
+    }
+    L.cfl = !A.subsampled; L.smooth = adaptive_smoothing ? 1 : 0; L.kx = k_x; L.kb = k_b;
+    A.out_h = out_h; A.out_w = out_w;
+    fill_k2(A.P, p, nullptr);
+    const long long n = (long long)out_h * out_w;
+    k10_lf_preview<<<(int)std::min<long long>((long long)ctx->sms * 8, (n + 255) / 256), 256, 0, st>>>(A);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+int32_t jxlb200_lf_preview(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float scaled_dequant[3], float k_x, float k_b,
+    int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, int32_t n_extra_precision,
+    int32_t out_h, int32_t out_w, float *const out[3]) {
+    int rc = preview_check(ctx, p, scaled_dequant, adaptive_smoothing, lf_quant, extra_precision, n_extra_precision, out_h, out_w, out);
+    if (rc) return rc;
+    Staged r[6];
+    for (int c = 0; c < 3; c++) {
+        r[c] = {&ctx->blend, lf_quant[c], nullptr, sizeof(int32_t) * (size_t)((p->height >> 3) >> p->shift_y[c]) * ((p->width >> 3) >> p->shift_x[c])};
+        r[3 + c] = {&ctx->blend, nullptr, out[c], sizeof(float) * (size_t)out_h * out_w};
+    }
+    if ((rc = stage_in(ctx, r, 6))) return rc;
+    if ((rc = preview_enqueue(ctx, p, scaled_dequant, k_x, k_b, adaptive_smoothing, planes_of<const int32_t>(r).data(), extra_precision,
+                              out_h, out_w, planes_of<float>(r + 3).data())))
+        return rc;
+    return stage_out(ctx, r, 6);
+}
+int32_t jxlb200_lf_preview_dev(jxlb200_ctx *ctx, const jxlb200_frame_params *p, const float scaled_dequant[3], float k_x, float k_b,
+    int32_t adaptive_smoothing, const int32_t *const lf_quant[3], const uint8_t *extra_precision, int32_t n_extra_precision,
+    int32_t out_h, int32_t out_w, float *const out[3]) {
+    int rc = preview_check(ctx, p, scaled_dequant, adaptive_smoothing, lf_quant, extra_precision, n_extra_precision, out_h, out_w, out);
+    if (rc) return rc;
+    for (int c = 0; c < 3; c++)
+        for (int d = 0; d < 3; d++)
+            if ((const void *)lf_quant[c] == (const void *)out[d]) return ctx->fail(JXLB200_E_ARG, "an output plane aliases an input plane");
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return preview_enqueue(ctx, p, scaled_dequant, k_x, k_b, adaptive_smoothing, lf_quant, extra_precision, out_h, out_w, out);
+}
+
+static int area_check(jxlb200_ctx *ctx, int32_t n_channels, const void *const planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t h, int32_t w, float *const out[]) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!planes || !is_int || !depth || !out || n_channels < 1 || h <= 0 || w <= 0) return ctx->fail(JXLB200_E_ARG, "bad arguments");
+    for (int c = 0; c < n_channels; c++) {
+        if (!planes[c] || !out[c]) return ctx->fail(JXLB200_E_ARG, "NULL plane pointer");
+        if (is_int[c] && (depth[c] < 1 || depth[c] > 31)) return ctx->fail(JXLB200_E_ARG, "bit depth outside 1..31");
+    }
+    return 0;
+}
+static int area_enqueue(jxlb200_ctx *ctx, int32_t n_channels, const void *const d_planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t h, int32_t w, float *const d_out[]) {
+    AreaArgs A;
+    A.h = h; A.w = w; A.oh = (h + 7) >> 3; A.ow = (w + 7) >> 3;
+    const long long n = (long long)A.oh * A.ow;
+    for (int c0 = 0; c0 < n_channels; c0 += kAreaChannels) {
+        const int nc = std::min(kAreaChannels, n_channels - c0);
+        for (int k = 0; k < nc; k++) {
+            const int c = c0 + k;
+            A.plane[k] = d_planes[c]; A.out[k] = d_out[c]; A.is_int[k] = is_int[c] ? 1 : 0;
+            A.scale[k] = is_int[c] ? 1.0f / (float)((1u << depth[c]) - 1u) : 1.0f;      // ImageBuffer.castToFloat
+        }
+        const dim3 grid((unsigned)std::min<long long>((long long)ctx->sms * 8, (n + 255) / 256), (unsigned)nc);
+        k10_area_mean8<<<grid, 256, 0, ctx->stream>>>(A);
+        ctx->launches++;
+    }
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+int32_t jxlb200_area_mean8(jxlb200_ctx *ctx, int32_t n_channels, const void *const planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t h, int32_t w, float *const out[]) {
+    int rc = area_check(ctx, n_channels, planes, is_int, depth, h, w, out);
+    if (rc) return rc;
+    const size_t in_bytes = 4 * (size_t)h * w, out_bytes = sizeof(float) * (size_t)((h + 7) >> 3) * ((w + 7) >> 3);
+    std::vector<Staged> r(2 * (size_t)n_channels);
+    for (int c = 0; c < n_channels; c++) {
+        r[c] = {&ctx->blend, planes[c], nullptr, in_bytes};
+        r[n_channels + c] = {&ctx->blend, nullptr, out[c], out_bytes};
+    }
+    if ((rc = stage_in(ctx, r.data(), 2 * n_channels))) return rc;
+    std::vector<const void *> d(n_channels);
+    std::vector<float *> o(n_channels);
+    for (int c = 0; c < n_channels; c++) { d[c] = r[c].dev; o[c] = (float *)r[n_channels + c].dev; }
+    if ((rc = area_enqueue(ctx, n_channels, d.data(), is_int, depth, h, w, o.data()))) return rc;
+    return stage_out(ctx, r.data(), 2 * n_channels);
+}
+int32_t jxlb200_area_mean8_dev(jxlb200_ctx *ctx, int32_t n_channels, const void *const planes[], const int32_t is_int[], const int32_t depth[],
+    int32_t h, int32_t w, float *const out[]) {
+    int rc = area_check(ctx, n_channels, planes, is_int, depth, h, w, out);
+    if (rc) return rc;
+    for (int c = 0; c < n_channels; c++)
+        for (int d = 0; d < n_channels; d++)
+            if (planes[c] == (const void *)out[d]) return ctx->fail(JXLB200_E_ARG, "an output plane aliases an input plane");
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return area_enqueue(ctx, n_channels, planes, is_int, depth, h, w, out);
 }
 
 

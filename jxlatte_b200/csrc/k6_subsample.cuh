@@ -25,6 +25,10 @@ __global__ void k6_submap(const uint8_t *__restrict__ ds, const int32_t *__restr
     }
 }
 
+// one output sample of a doubling: .75 of the input sample it lies on (c75 = __fmul_rn(0.75f, centre), shared by the two outputs of
+// that sample) + .25 of the input neighbour on its side (clamped at the edge)
+__device__ __forceinline__ float double_px(float c75, float side) { return __fadd_rn(c75, __fmul_rn(0.25f, side)); }
+
 // one horizontal doubling: out[y][2x] = .75 in[y][x] + .25 in[y][max(x-1,0)], out[y][2x+1] = .75 in[y][x] + .25 in[y][min(x+1,w-1)]
 __global__ void k6_upsample_h(const float *__restrict__ in, int h, int w, float *__restrict__ out) {
     const long long n = (long long)h * w;
@@ -32,8 +36,8 @@ __global__ void k6_upsample_h(const float *__restrict__ in, int h, int w, float 
         const int y = (int)(i / w), x = (int)(i - (long long)y * w);
         const float *row = in + (size_t)y * w;
         const float b75 = __fmul_rn(0.75f, row[x]);
-        const float l = __fadd_rn(b75, __fmul_rn(0.25f, row[x == 0 ? 0 : x - 1]));
-        const float r = __fadd_rn(b75, __fmul_rn(0.25f, row[x + 1 == w ? w - 1 : x + 1]));
+        const float l = double_px(b75, row[x == 0 ? 0 : x - 1]);
+        const float r = double_px(b75, row[x + 1 == w ? w - 1 : x + 1]);
         *reinterpret_cast<float2 *>(out + (size_t)y * 2 * w + 2 * x) = make_float2(l, r);
     }
 }
@@ -45,7 +49,7 @@ __global__ void k6_upsample_v(const float *__restrict__ in, int h, int w, float 
         const int y = (int)(i / w), x = (int)(i - (long long)y * w);
         const float b75 = __fmul_rn(0.75f, in[(size_t)y * w + x]);
         const float up = in[(size_t)(y == 0 ? 0 : y - 1) * w + x], dn = in[(size_t)(y + 1 == h ? h - 1 : y + 1) * w + x];
-        out[(size_t)(2 * y) * w + x] = __fadd_rn(b75, __fmul_rn(0.25f, up));
-        out[(size_t)(2 * y + 1) * w + x] = __fadd_rn(b75, __fmul_rn(0.25f, dn));
+        out[(size_t)(2 * y) * w + x] = double_px(b75, up);
+        out[(size_t)(2 * y + 1) * w + x] = double_px(b75, dn);
     }
 }

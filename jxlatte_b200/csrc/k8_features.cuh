@@ -368,39 +368,43 @@ __device__ __forceinline__ void lf_value(const LfArgs &A, size_t o, const float 
         v[2] = __fadd_rn(v[2], __fmul_rn(A.kb, v[1]));
     }
 }
+// the value of LF sample i (row-major over hb x wb): dequantised, LF chroma-from-luma, adaptively smoothed inside its LF group
+__device__ __forceinline__ void lf_sample(const LfArgs &A, long long i, float (&c)[3]) {
+    const int y = (int)(i / A.wb), x = (int)(i - (long long)y * A.wb);
+    const int gy = y >> 8, gx = x >> 8, ly = y & 255, lx = x & 255;
+    const int h = min(256, A.hb - (gy << 8)), w = min(256, A.wb - (gx << 8));
+    const float div = (float)(1 << A.ep[gy * A.gcols + gx]);
+    const float sdg[3] = {__fdiv_rn(A.sd[0], div), __fdiv_rn(A.sd[1], div), __fdiv_rn(A.sd[2], div)};
+    lf_value(A, (size_t)i, sdg, c);
+    const bool interior = A.smooth && h >= 3 && w >= 3 && ly >= 1 && ly + 1 < h && lx >= 1 && lx + 1 < w;
+    if (interior) {
+        float nb[8][3];     // W, E, N, S, NW, NE, SW, SE
+        const long long wb = A.wb;
+        lf_value(A, (size_t)(i - 1), sdg, nb[0]); lf_value(A, (size_t)(i + 1), sdg, nb[1]);
+        lf_value(A, (size_t)(i - wb), sdg, nb[2]); lf_value(A, (size_t)(i + wb), sdg, nb[3]);
+        lf_value(A, (size_t)(i - wb - 1), sdg, nb[4]); lf_value(A, (size_t)(i - wb + 1), sdg, nb[5]);
+        lf_value(A, (size_t)(i + wb - 1), sdg, nb[6]); lf_value(A, (size_t)(i + wb + 1), sdg, nb[7]);
+        float wv[3], gap = 0.5f;
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+            const float adjacent = __fadd_rn(__fadd_rn(__fadd_rn(nb[0][k], nb[1][k]), nb[2][k]), nb[3][k]);
+            const float diag = __fadd_rn(__fadd_rn(__fadd_rn(nb[4][k], nb[5][k]), nb[6][k]), nb[7][k]);
+            wv[k] = __fadd_rn(__fadd_rn(__fmul_rn(0.05226273532324128f, c[k]), __fmul_rn(0.20345139757231578f, adjacent)),
+                              __fmul_rn(0.0334829185968739f, diag));
+            const float g = __fmul_rn(fabsf(__fsub_rn(c[k], wv[k])), A.sd[k]);
+            if (g > gap) gap = g;
+        }
+        gap = __fsub_rn(3.0f, __fmul_rn(4.0f, gap));
+        gap = gap > 0.0f ? gap : 0.0f;
+#pragma unroll
+        for (int k = 0; k < 3; k++) c[k] = __fadd_rn(__fmul_rn(__fsub_rn(c[k], wv[k]), gap), wv[k]);
+    }
+}
 __global__ void k8_lf_dequant(LfArgs A) {
     const long long n = (long long)A.hb * A.wb;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const int y = (int)(i / A.wb), x = (int)(i - (long long)y * A.wb);
-        const int gy = y >> 8, gx = x >> 8, ly = y & 255, lx = x & 255;
-        const int h = min(256, A.hb - (gy << 8)), w = min(256, A.wb - (gx << 8));
-        const float div = (float)(1 << A.ep[gy * A.gcols + gx]);
-        const float sdg[3] = {__fdiv_rn(A.sd[0], div), __fdiv_rn(A.sd[1], div), __fdiv_rn(A.sd[2], div)};
         float c[3];
-        lf_value(A, (size_t)i, sdg, c);
-        const bool interior = A.smooth && h >= 3 && w >= 3 && ly >= 1 && ly + 1 < h && lx >= 1 && lx + 1 < w;
-        if (interior) {
-            float nb[8][3];     // W, E, N, S, NW, NE, SW, SE
-            const long long wb = A.wb;
-            lf_value(A, (size_t)(i - 1), sdg, nb[0]); lf_value(A, (size_t)(i + 1), sdg, nb[1]);
-            lf_value(A, (size_t)(i - wb), sdg, nb[2]); lf_value(A, (size_t)(i + wb), sdg, nb[3]);
-            lf_value(A, (size_t)(i - wb - 1), sdg, nb[4]); lf_value(A, (size_t)(i - wb + 1), sdg, nb[5]);
-            lf_value(A, (size_t)(i + wb - 1), sdg, nb[6]); lf_value(A, (size_t)(i + wb + 1), sdg, nb[7]);
-            float wv[3], gap = 0.5f;
-#pragma unroll
-            for (int k = 0; k < 3; k++) {
-                const float adjacent = __fadd_rn(__fadd_rn(__fadd_rn(nb[0][k], nb[1][k]), nb[2][k]), nb[3][k]);
-                const float diag = __fadd_rn(__fadd_rn(__fadd_rn(nb[4][k], nb[5][k]), nb[6][k]), nb[7][k]);
-                wv[k] = __fadd_rn(__fadd_rn(__fmul_rn(0.05226273532324128f, c[k]), __fmul_rn(0.20345139757231578f, adjacent)),
-                                  __fmul_rn(0.0334829185968739f, diag));
-                const float g = __fmul_rn(fabsf(__fsub_rn(c[k], wv[k])), A.sd[k]);
-                if (g > gap) gap = g;
-            }
-            gap = __fsub_rn(3.0f, __fmul_rn(4.0f, gap));
-            gap = gap > 0.0f ? gap : 0.0f;
-#pragma unroll
-            for (int k = 0; k < 3; k++) c[k] = __fadd_rn(__fmul_rn(__fsub_rn(c[k], wv[k]), gap), wv[k]);
-        }
+        lf_sample(A, i, c);
         A.out[0][i] = c[0]; A.out[1][i] = c[1]; A.out[2][i] = c[2];
     }
 }

@@ -23,7 +23,7 @@ import zlib
 import numpy as np
 
 from . import frontend, host
-from .params import STATE_MAPS, FrameParams, check_planes, check_state_shapes
+from .params import STATE_MAPS, FrameParams, check_channels, check_lf_planes, check_planes, check_state_shapes
 from .upsampling import up_weights
 
 ENC_VARDCT, ENC_MODULAR = 0, 1
@@ -144,13 +144,30 @@ def _arrays(engine):
     return getattr(engine, "arrays", None) or _NUMPY
 
 
+def preview_route(info):
+    """How JXLOptions(preview=True) renders a stream, from its headers (a parse with frontend.FLAG_LF_ONLY has them all): "lf" when
+    every frame's 1:8 image is its LF image -- VarDCT, type 0 or 3, no LF frame used or present, no patches, splines or noise, no
+    upsampling, no extra channels in the image, blend mode REPLACE and an origin on the 8 x 8 grid -- else "full"."""
+    if info["extra_channels"]:
+        return "full"
+    for f in info["frames"]:
+        if (f["encoding"] != ENC_VARDCT or f["type"] not in (0, 3) or f["flags"] & (FLAG_USE_LF_FRAME | FLAG_PATCHES | FLAG_SPLINES | FLAG_NOISE)
+                or f["upsampling"] != 1 or f["blend_mode"] != 0 or f["x0"] % 8 or f["y0"] % 8):
+            return "full"
+    return "lf"
+
+
 class JXLOptions:
     """The reference's JXLOptions (J/JXLOptions.java:7-50), the fields that reach the reconstruction path."""
     OUTPUT_DEFAULT, OUTPUT_PNG, OUTPUT_PFM = -1, 0, 1
 
-    def __init__(self, outputFormat=-1, outputDepth=-1):
+    def __init__(self, outputFormat=-1, outputDepth=-1, preview=False):
         self.outputFormat = outputFormat    # OUTPUT_PNG: the caller will quantise with PNGWriter; OUTPUT_PFM / default: float samples
         self.outputDepth = outputDepth      # -1: PNGWriter picks 8 for images of up to 8 bits per sample, else 16
+        # preview: every displayed image at 1:8, ceil(H / 8) x ceil(W / 8) before orientation, as float32 channels (linear when
+        # xyb_encoded).  Streams preview_route() accepts are rendered from the frames' LF images without decoding any HF data; the
+        # others are decoded in full and each channel is averaged over 8 x 8 areas.
+        self.preview = preview
 
     def quantises_to_8_bits(self, bits_per_sample):
         """True when the only consumer of the planes is PNGWriter at 8 bits: the tolerance "<= 1e-4 and <= 1 LSB" of the north
@@ -219,6 +236,12 @@ class CudaEngine:
 
     def lf_dequant(self, q, ep, scaled_dequant, kx, kb, smooth):
         return self.rec.dequantLF(q, ep, scaled_dequant, kx, kb, cfl=True, smooth=smooth)
+
+    def lf_preview(self, p, q, ep, scaled_dequant, kx, kb, smooth, out_h, out_w):
+        return self.rec.lfPreview(p, q, ep, scaled_dequant, kx, kb, smooth, out_h, out_w)
+
+    def area_mean8(self, channels, depths):
+        return self.rec.areaMean8(channels, depths)
 
     # ---- compositing: the blends of a frame are queued and run in ONE device call (jxlb200_blend_batch) ----
     def _locate(self, v):
@@ -386,6 +409,19 @@ class DeviceEngine(CudaEngine):
         out = self.empty((3, hb, wb))
         self.rec.lf_dequant_dev(hb, wb, scaled_dequant, kx, kb, True, smooth, [a.data_ptr() for a in qd], ep, [out[c].data_ptr() for c in range(3)])
         return out
+
+    def lf_preview(self, p, q, ep, scaled_dequant, kx, kb, smooth, out_h, out_w):
+        qd = check_lf_planes(p, [self.upload(q[c], np.int32) for c in range(3)])
+        out = self.empty((3, out_h, out_w))
+        self.rec.lf_preview_dev(p, scaled_dequant, kx, kb, smooth, [a.data_ptr() for a in qd], ep, out_h, out_w, [out[c].data_ptr() for c in range(3)])
+        return out
+
+    def area_mean8(self, channels, depths):
+        ch = [c.contiguous() for c in channels]
+        h, w = check_channels(ch)
+        out = self.empty((len(ch), (h + 7) // 8, (w + 7) // 8))
+        self.rec.area_mean8_dev([c.data_ptr() for c in ch], [not self.is_float(c) for c in ch], depths, h, w, [o.data_ptr() for o in out])
+        return list(out)
 
     def modular(self, channels, transforms, bit_depth):
         return _DeviceModularTransforms(_DeviceModularOps(self), bit_depth).applyTransforms([self.upload(c, np.int32) for c in channels], transforms)
@@ -679,6 +715,7 @@ class JXLDecoder:
         self._own = engine is None
         self.engine = engine
         self.timings = {}
+        self.preview_route = None           # JXLOptions(preview=True): "lf" or "full" (preview_route()) once the stream is parsed
         self._images = None
         self._next = None
         self._buffered = False
@@ -969,10 +1006,20 @@ class JXLDecoder:
         """Generator over the displayed images: JXLCodestreamDecoder.decode's frame loop for the features this build renders."""
         import time
         t0 = time.perf_counter()
-        parsed = frontend.parse(self.data)
+        if self.options.preview:
+            parsed = frontend.parse(self.data, frontend.FLAG_LF_ONLY)
+            self.preview_route = preview_route(parsed.info)
+            if self.preview_route == "full":
+                parsed.close()
+                parsed = frontend.parse(self.data)
+        else:
+            parsed = frontend.parse(self.data)
         self.timings["front_end_s"] = time.perf_counter() - t0
         if self.engine is None:
             self.engine = CudaEngine()
+        if self.preview_route == "lf":
+            yield from self._compose_lf(parsed)
+            return
         info = parsed.info
         xp, buf = self._xp, self._buf
         sync = getattr(self.engine, "sync", None)
@@ -1070,9 +1117,56 @@ class JXLDecoder:
             if f["is_last"] or f["duration"] != 0:
                 if sync is None:
                     self.timings["reconstruct_s"] = time.perf_counter() - t1
-                img = self._finish(canvas, info, linear, copy=not f["is_last"], xp=xp, engine=self.engine if xp is not _NUMPY else None)
+                shown, copy = canvas, not f["is_last"]
+                if self.options.preview:
+                    shown, copy = self._area_mean8(canvas, info), False
+                img = self._finish(shown, info, linear, copy=copy, xp=xp, engine=self.engine if xp is not _NUMPY else None)
                 if sync is not None:
                     sync()                  # device engines: the image is complete, and stream errors surface here
+                    self.timings["reconstruct_s"] = time.perf_counter() - t1
+                yield img
+                t1 = time.perf_counter()
+        parsed.close()
+
+    def _area_mean8(self, canvas, info):
+        """The preview of a composed canvas: each channel's 8 x 8 area means (float32; int32 channels cast by their bit depth first)."""
+        depths = [info["bits_per_sample"]] * info["color_channels"] + [e["bits_per_sample"] for e in info["extra_channels"]]
+        return [self._buf(a) for a in self.engine.area_mean8([b.a for b in canvas], depths[:len(canvas)])]
+
+    def _compose_lf(self, parsed):
+        """The displayed images of a stream preview_route() sends to "lf", at 1:8: each frame rendered from its LF image by the engine's
+        lf_preview (one kernel), REPLACEd into a ceil(H / 8) x ceil(W / 8) canvas at (y0 / 8, x0 / 8) with blendFrame's crop clipping,
+        and shown when it is the last or has a duration, as _compose shows frames."""
+        import time
+        info, xp, buf = parsed.info, self._xp, self._buf
+        sync = getattr(self.engine, "sync", None)
+        colors = info["color_channels"]
+        ih, iw = -(-info["height"] // 8), -(-info["width"] // 8)
+        canvas = None
+        t1 = time.perf_counter()
+        for k, f in enumerate(parsed.frames):
+            fh, fw, fy0, fx0 = -(-f["height"] // 8), -(-f["width"] // 8), f["y0"] // 8, f["x0"] // 8
+            q, ep, sd, kx, kb, smooth = parsed.lf_state(k)
+            planes = self.engine.lf_preview(self.frame_params(info, f), q, ep, sd, kx, kb, smooth, fh, fw)
+            chans = [planes[1]] if colors == 1 else [planes[c] for c in range(3)]      # a grey image shows Y, as blendBuffers picks it
+            if canvas is None and (fy0, fx0, fh, fw) == (0, 0, ih, iw):
+                canvas = chans                          # fresh planes nobody else holds
+            else:
+                if canvas is None:
+                    canvas = [xp.zeros((ih, iw)) for _ in range(colors)]
+                ps = (min(max(fy0, 0), ih), min(max(fx0, 0), iw))
+                fo = (ps[0] - fy0, ps[1] - fx0)
+                size = (min(fy0 + fh, ih) - ps[0], min(fx0 + fw, iw) - ps[1])
+                if size[0] > 0 and size[1] > 0:
+                    for c in range(colors):
+                        canvas[c][ps[0]:ps[0] + size[0], ps[1]:ps[1] + size[1]] = chans[c][fo[0]:fo[0] + size[0], fo[1]:fo[1] + size[1]]
+            if f["is_last"] or f["duration"] != 0:
+                if sync is None:
+                    self.timings["reconstruct_s"] = time.perf_counter() - t1
+                img = self._finish([buf(a) for a in canvas], info, bool(info["xyb_encoded"]), copy=not f["is_last"], xp=xp,
+                                   engine=self.engine if xp is not _NUMPY else None)
+                if sync is not None:
+                    sync()
                     self.timings["reconstruct_s"] = time.perf_counter() - t1
                 yield img
                 t1 = time.perf_counter()

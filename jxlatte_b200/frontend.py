@@ -23,7 +23,7 @@ class InvalidBitstreamError(IOError):
 
 
 def build(force=False):
-    srcs = [os.path.join(SRC_DIR, f) for f in sorted(os.listdir(SRC_DIR))]
+    srcs = [os.path.join(SRC_DIR, f) for f in sorted(os.listdir(SRC_DIR))] + [os.path.join(_HERE, "..", "include", "jxlfront.h")]
     if not force and os.path.exists(SO_PATH) and all(os.path.getmtime(s) <= os.path.getmtime(SO_PATH) for s in srcs):
         return SO_PATH
     r = subprocess.run([CXX] + CXXFLAGS + ["-o", SO_PATH, os.path.join(SRC_DIR, "api.cpp")], capture_output=True, text=True)
@@ -56,6 +56,7 @@ def lib():
 
 FLAG_HOST_TRANSFORMS = 1     # also undo the frame-level modular transforms on the host (tests / cross-checks)
 FLAG_HEADERS_ONLY = 2
+FLAG_LF_ONLY = 4             # parse each frame up to its LF groups only (include/jxlfront.h JXLF_LF_ONLY)
 _DTYPES = {0: np.int32, 1: np.float32, 2: np.uint8}
 
 
@@ -130,14 +131,21 @@ class ParsedImage:
         f = self.frames[frame]
         if f["flags"] & 32 or any(f["shift_x"]) or any(f["shift_y"]):
             return None
-        hb, wb = f["padded_height"] // 8, f["padded_width"] // 8
         try:
-            q = np.stack([self.array(frame, "lf_quant", c, (hb, wb)) for c in range(3)])
-            ep = self.array(frame, "lf_extra_precision", 0)
+            q, ep, sd, kx, kb, smooth = self.lf_state(frame)
         except Exception:
             return None
+        return np.stack(q), ep, sd, kx, kb, smooth
+
+    def lf_state(self, frame):
+        """The quantised LF image of a VarDCT frame, chroma-subsampled or not: ([lf_quant int32 (hb >> sy[c], wb >> sx[c]) for X, Y, B],
+        extraPrecision per LF group, scaledDequant[3], kX, kB, adaptive smoothing?).  hb, wb are the padded frame size in blocks."""
+        f = self.frames[frame]
+        hb, wb = f["padded_height"] // 8, f["padded_width"] // 8
+        q = [self.array(frame, "lf_quant", c, (hb >> f["shift_y"][c], wb >> f["shift_x"][c])) for c in range(3)]
+        ep = self.array(frame, "lf_extra_precision", 0)
         if ep.size != ((hb + 255) // 256) * ((wb + 255) // 256):
-            return None
+            raise InvalidBitstreamError("frame %d has no extraPrecision for every LF group" % frame)
         f32 = np.float32
         kx = f32(f["base_corr_x"]) + (f32(f["x_factor_lf"]) - f32(128.0)) / f32(f["color_factor"])     # LFCoefficients.java:81-82
         kb = f32(f["base_corr_b"]) + (f32(f["b_factor_lf"]) - f32(128.0)) / f32(f["color_factor"])

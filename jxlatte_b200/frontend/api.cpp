@@ -7,6 +7,7 @@
 #include <sstream>
 
 #include "frame.hpp"
+#include "../../include/jxlfront.h"
 
 using namespace jxlf;
 
@@ -16,6 +17,7 @@ struct jxlf_image {
     std::vector<std::unique_ptr<FrameData>> frames;
     std::string json, error;
     int status = 0;
+    bool lf_only = false;
 };
 
 namespace {
@@ -147,9 +149,9 @@ void describe(jxlf_image &im) {
             j.close(']');
         }
         j.close(']');
-        j.boolean("decoded", !f.dct_select.empty() || f.has_modular || h.encoding == ENC_MODULAR);
-        j.boolean("quant_all_default", f.quant_all_default);
-        if (!f.quant_all_default) {
+        j.boolean("decoded", !f.dct_select.empty() || !f.lf[0].empty() || f.has_modular || h.encoding == ENC_MODULAR);
+        if (!f.lf_only) j.boolean("quant_all_default", f.quant_all_default);      // HfGlobal: not read by an LF-only parse
+        if (!f.lf_only && !f.quant_all_default) {
             j.open("quant_params", '[');
             for (const QuantParams &q : f.qparams) {
                 j.open(nullptr, '{');
@@ -191,6 +193,7 @@ void describe(jxlf_image &im) {
         j.close('}');
     }
     j.close(']');
+    if (im.lf_only) j.boolean("lf_only", true);
     j.close('}');
     im.json = j.o.str();
 }
@@ -200,12 +203,15 @@ void describe(jxlf_image &im) {
 extern "C" {
 
 // flags: bit 0 = also undo the frame-level modular transforms on the host (tests / cross-checks; the product path
-// leaves them to the GPU), bit 1 = stop after the headers of the first frame.
+// leaves them to the GPU), bit 1 = stop after the headers of the first frame, bit 2 = parse every frame up to its LF groups only.
 int32_t jxlf_decode(const uint8_t *data, uint64_t size, int32_t flags, jxlf_image **out) {
     if (!data || !out) return -1;
     auto im = std::make_unique<jxlf_image>();
     coverage().reset();
+    im->lf_only = (flags & JXLF_LF_ONLY) != 0;
     try {
+        // the host transforms need every channel, and an LF-only parse leaves the pass groups' channels empty
+        if ((flags & JXLF_HOST_TRANSFORMS) && im->lf_only) throw std::invalid_argument("JXLF_HOST_TRANSFORMS with JXLF_LF_ONLY");
         std::vector<uint8_t> file(data, data + size);
         const int level = extract_codestream(file, im->codestream);
         BitReader br(im->codestream.data(), im->codestream.size());
@@ -216,7 +222,7 @@ int32_t jxlf_decode(const uint8_t *data, uint64_t size, int32_t flags, jxlf_imag
             FrameDecoder dec(br, im->ih);
             dec.read_header(*f);
             if (flags & 2) { im->frames.push_back(std::move(f)); break; }
-            dec.decode(*f);
+            dec.decode(*f, im->lf_only);
             if (flags & 1) f->modular.apply_transforms();
             const bool last = f->hdr.is_last;
             im->frames.push_back(std::move(f));
@@ -252,6 +258,9 @@ int32_t jxlf_array(const jxlf_image *im, int32_t frame, const char *name, int32_
     if (frame < 0 || frame >= (int)im->frames.size()) return -1;
     const FrameData &f = *im->frames[frame];
     auto give = [&](const auto &v, int dt) { *ptr = v.data(); *count = (int64_t)v.size(); *dtype = dt; return 0; };
+    if (f.lf_only && (n == "qcoeff" || n == "dct_select" || n == "block_origin" || n == "hf_mul" || n == "sharpness" || n == "x_from_y" ||
+                      n == "b_from_y"))
+        return -1;                                       // HF state: an LF-only parse never read it
     if (n == "qcoeff" && index >= 0 && index < 3) return give(f.qcoeff[index], 0);
     if (n == "lf" && index >= 0 && index < 3) return give(f.lf[index], 1);
     if (n == "lf_quant" && index >= 0 && index < 3) return give(f.lf_quant[index], 0);

@@ -69,6 +69,7 @@ struct FrameData {
     // frame-level modular stream
     ModularStream modular;
     bool has_modular = false;
+    bool lf_only = false;                        // parsed up to the LF groups only (JXLF_LF_ONLY): no HF state was read
 };
 
 class FrameDecoder {
@@ -103,7 +104,10 @@ class FrameDecoder {
     size_t frame_bytes() const { size_t n = 0; for (auto l : toc_len_) n += l; return n; }
     void skip(FrameData &) { br_.seek_bytes(toc_start_ + frame_bytes()); }
 
-    void decode(FrameData &f) {
+    // lf_only: stop after LfGlobal and the LF groups' LF coefficients and Modular channels.  HF metadata, HfGlobal and the pass
+    // groups are never read, so their sections may hold anything.
+    void decode(FrameData &f, bool lf_only = false) {
+        f.lf_only = lf_only;
         open_sections();
         fc_.group_dim = f.hdr.group_dim;
         fc_.modular_h = f.hdr.height;
@@ -114,10 +118,12 @@ class FrameDecoder {
         read_lf_global(f, section(0));
         allocate_vardct(f);
         decode_lf_groups(f);
-        BitReader &hg = section(1 + f.num_lf_groups);
-        if (f.hdr.encoding == ENC_VARDCT) read_hf_global(f, hg);
-        read_passes(f, hg);
-        decode_pass_groups(f);
+        if (!lf_only) {
+            BitReader &hg = section(1 + f.num_lf_groups);
+            if (f.hdr.encoding == ENC_VARDCT) read_hf_global(f, hg);
+            read_passes(f, hg);
+            decode_pass_groups(f);
+        }
         br_.seek_bytes(toc_start_ + frame_bytes());
     }
 
@@ -364,10 +370,11 @@ class FrameDecoder {
         if (f.hdr.encoding != ENC_VARDCT) return;
         const int bh = f.padded_h >> 3, bw = f.padded_w >> 3;
         for (int c = 0; c < 3; c++) {
-            f.qcoeff[c].assign((size_t)(f.padded_h >> f.hdr.shift_y[c]) * (f.padded_w >> f.hdr.shift_x[c]), 0);
             f.lf[c].assign((size_t)(bh >> f.hdr.shift_y[c]) * (bw >> f.hdr.shift_x[c]), 0.0f);
             f.lf_quant[c].assign((size_t)(bh >> f.hdr.shift_y[c]) * (bw >> f.hdr.shift_x[c]), 0);
         }
+        if (f.lf_only) return;
+        for (int c = 0; c < 3; c++) f.qcoeff[c].assign((size_t)(f.padded_h >> f.hdr.shift_y[c]) * (f.padded_w >> f.hdr.shift_x[c]), 0);
         f.dct_select.assign((size_t)bh * bw, 0);
         f.block_origin.assign((size_t)bh * bw, 0);
         f.hf_mul.assign((size_t)bh * bw, 1);
@@ -434,7 +441,7 @@ class FrameDecoder {
             ms.init(br, fc_, 1 + f.num_lf_groups + g, cut_channels(f, lf_channels, g, lf_dim));
             ms.decode_channels(br);
             paste_channels(f, lf_channels, ms);
-            if (h.encoding == ENC_VARDCT) read_hf_metadata(f, br, g, st);
+            if (h.encoding == ENC_VARDCT && !f.lf_only) read_hf_metadata(f, br, g, st);
         });
     }
 

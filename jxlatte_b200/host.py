@@ -21,7 +21,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import QmParams, Slab  # noqa: F401
-from .params import STATE_MAPS, FrameParams, check_planes, check_state_shapes
+from .params import STATE_MAPS, FrameParams, check_channels, check_lf_planes, check_planes, check_state_shapes
 
 
 class InvalidBitstreamError(IOError):
@@ -75,6 +75,16 @@ def _extra_precision(extra_precision, hb, wb):
     if ep.size != ((hb + 255) // 256) * ((wb + 255) // 256):
         raise ValueError("extra_precision must hold one byte per LF group")
     return ep
+
+
+def _preview_args(scaled_dequant, extra_precision):
+    """The scaledDequant array and the flat extraPrecision bytes of jxlb200_lf_preview[_dev] (the library checks their count)."""
+    return (C.c_float * 3)(*[float(v) for v in scaled_dequant]), _c(np.asarray(extra_precision).reshape(-1), np.uint8)
+
+
+def _area_args(is_int, depths):
+    """The is_int and depth arrays of jxlb200_area_mean8[_dev]."""
+    return np.array([1 if v else 0 for v in is_int], np.int32), np.array(depths, np.int32)
 
 
 def _upsampling_weights(weights, k):
@@ -392,6 +402,29 @@ class Reconstructor:
                                                _lib.planes([_ptr(a) for a in q]), _ptr(ep), _lib.planes([_ptr(out[c]) for c in range(3)])))
         return out
 
+    # -- 1:8 previews (k10_preview.cuh) --
+    def lfPreview(self, p, lf_quant, extra_precision, scaled_dequant, kx, kb, smooth, out_h, out_w):
+        """A VarDCT frame rendered from its LF image alone (jxlb200_lf_preview): the quantised LF planes X, Y, B (each of its
+        state_shapes(p)["lf"] shape) + extraPrecision per LF group -> the frame at 1:8 after p's colour transform, f32[3, out_h, out_w]."""
+        q = check_lf_planes(p, [_c(lf_quant[c], np.int32) for c in range(3)])
+        sd, ep = _preview_args(scaled_dequant, extra_precision)
+        out = np.empty((3, out_h, out_w), np.float32)
+        self._check(self._L.jxlb200_lf_preview(self._h, C.byref(p), sd, C.c_float(float(kx)), C.c_float(float(kb)), 1 if smooth else 0,
+                                               _lib.planes([_ptr(a) for a in q]), _ptr(ep), ep.size, int(out_h), int(out_w),
+                                               _lib.planes([_ptr(out[c]) for c in range(3)])))
+        return out
+
+    def areaMean8(self, channels, depths):
+        """The 8x8 area mean of equally sized float32 / int32 channels (jxlb200_area_mean8; int32 ones cast by castToFloat(depth) first)
+        -> one float32 plane of ceil(h / 8) x ceil(w / 8) per channel."""
+        ch = [np.ascontiguousarray(c if c.dtype == np.float32 else c.astype(np.int32)) for c in channels]
+        h, w = check_channels(ch)
+        ii, dep = _area_args([c.dtype != np.float32 for c in ch], depths)
+        out = [np.empty(((h + 7) // 8, (w + 7) // 8), np.float32) for _ in ch]
+        self._check(self._L.jxlb200_area_mean8(self._h, len(ch), _lib.planes([_ptr(a) for a in ch]), _ptr(ii), _ptr(dep), h, w,
+                                               _lib.planes([_ptr(a) for a in out])))
+        return out
+
     def blend_batch(self, planes, writable, items):
         """A frame's whole compositing in one call (jxlb200_blend_batch).  planes: 2-D C-contiguous 4-byte numpy arrays (written in
         place when writable[i]); items: (op dict, (h, w), [(plane index, y, x) or None] * 5) in the order canvas, `frame`, `ref`,
@@ -414,6 +447,16 @@ class Reconstructor:
         sd = (C.c_float * 3)(*[float(v) for v in scaled_dequant])
         self._check(self._L.jxlb200_lf_dequant_dev(self._h, int(hb), int(wb), sd, C.c_float(float(kx)), C.c_float(float(kb)), 1 if cfl else 0,
                                                    1 if smooth else 0, _lib.planes(lf_quant), _ptr(ep), _lib.planes(out)))
+
+    def lf_preview_dev(self, p, scaled_dequant, kx, kb, smooth, lf_quant, extra_precision, out_h, out_w, out):
+        """jxlb200_lf_preview_dev: lf_quant / out are three device pointers each; extra_precision a host array."""
+        sd, ep = _preview_args(scaled_dequant, extra_precision)
+        self._check(self._L.jxlb200_lf_preview_dev(self._h, C.byref(p), sd, C.c_float(float(kx)), C.c_float(float(kb)), 1 if smooth else 0,
+                                                   _lib.planes(lf_quant), _ptr(ep), ep.size, int(out_h), int(out_w), _lib.planes(out)))
+
+    def area_mean8_dev(self, planes, is_int, depths, h, w, out):
+        ii, dep = _area_args(is_int, depths)
+        self._check(self._L.jxlb200_area_mean8_dev(self._h, len(planes), _lib.planes(planes), _ptr(ii), _ptr(dep), int(h), int(w), _lib.planes(out)))
 
     def restore_uniform_dev(self, p, epf_sigma_for_modular, planes_in, out):
         self._check(self._L.jxlb200_restore_uniform_dev(self._h, C.byref(p), C.c_float(float(epf_sigma_for_modular)), _lib.planes(planes_in),

@@ -109,6 +109,23 @@ def check_state_shapes(p, arrays, subsampled=True):
             raise ValueError("%s has shape %s, expected %s" % (k, tuple(a.shape), want[k]))
 
 
+def check_lf_planes(p, planes):
+    """The three quantised LF planes of a frame (numpy or torch), each of its state_shapes(p)["lf"] shape; ValueError otherwise."""
+    want = state_shapes(p)["lf"]
+    for c in range(3):
+        if tuple(planes[c].shape) != want[c]:
+            raise ValueError("lf_quant[%d] has shape %s, expected %s" % (c, tuple(planes[c].shape), want[c]))
+    return planes
+
+
+def check_channels(channels):
+    """Equally sized 2-D channels (numpy or torch) -> their (h, w); ValueError otherwise."""
+    shapes = {tuple(a.shape) for a in channels}
+    if not channels or len(shapes) != 1 or len(next(iter(shapes))) != 2:
+        raise ValueError("channels must be 2-D and of one size, got %s" % sorted(shapes))
+    return next(iter(shapes))
+
+
 def check_planes(p, planes):
     """The three colour planes of a frame, each p.height x p.width (numpy or torch); ValueError otherwise."""
     for a in planes:
