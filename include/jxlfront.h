@@ -50,6 +50,10 @@ const char *jxlf_describe(const jxlf_image *image);
  *   "qraw"                    index = 3 * parameter set + channel (MODE_RAW quant tables)
  *   "icc"                     the still-encoded ICC stream (frame ignored) */
 int32_t jxlf_array(const jxlf_image *image, int32_t frame, const char *name, int32_t index, const void **ptr, int64_t *count, int32_t *dtype);
+/* The number of OpenMP threads the calling thread's later jxlf_decode calls spread a frame's sections over (omp_set_num_threads:
+ * the setting belongs to the calling thread, so threads that parse files side by side can each take a share of the cores).
+ * n < 1 is ignored. */
+void jxlf_set_threads(int32_t n);
 
 #ifdef __cplusplus
 }

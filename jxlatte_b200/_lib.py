@@ -98,6 +98,7 @@ SYMBOLS = {
     "jxlb200_lf_preview_dev": (_i32, [_vp, _FP, _vp, C.c_float, C.c_float, _i32, _P3, _vp, _i32, _i32, _i32, _P3]),
     "jxlb200_area_mean8": (_i32, [_vp, _i32, _P3, _vp, _vp, _i32, _i32, _P3]),
     "jxlb200_area_mean8_dev": (_i32, [_vp, _i32, _P3, _vp, _vp, _i32, _i32, _P3]),
+    "jxlb200_pack_batch_dev": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp]),
 }
 
 
@@ -107,6 +108,11 @@ class BlendOp(C.Structure):
 
 class BlendItem(C.Structure):
     _fields_ = [("op", BlendOp), ("h", C.c_int32), ("w", C.c_int32), ("plane", C.c_int32 * 5), ("y", C.c_int32 * 5), ("x", C.c_int32 * 5)]
+
+
+class BatchItem(C.Structure):
+    _fields_ = [("plane", _vp * 4), ("is_int", C.c_int32 * 4), ("depth", C.c_int32 * 4), ("h", C.c_int32), ("w", C.c_int32),
+                ("pitch", C.c_int32 * 4), ("orientation", C.c_int32), ("linear", C.c_int32)]
 
 
 _LIB = None

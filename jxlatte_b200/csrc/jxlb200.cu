@@ -27,6 +27,7 @@
 #include "k8_features.cuh"
 #include "k9_device.cuh"
 #include "k10_preview.cuh"
+#include "k11_batch.cuh"
 #include "splines_host.cuh"
 #include "qm_tables.cuh"
 #include "split_nccl.cuh"
@@ -2128,6 +2129,44 @@ int32_t jxlb200_pack_samples_dev(jxlb200_ctx *ctx, const void *const planes[], c
     if (layout != 0 && layout != 1) return ctx->fail(JXLB200_E_ARG, "layout must be 0 (PNG bytes) or 1 (planar samples)");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     return pack_enqueue(ctx, planes, is_int, depth, n_channels, n_color, linear, h, w, bits, layout, out);
+}
+
+// ---- batch output (k11_pack_batch) ----
+int32_t jxlb200_pack_batch_dev(jxlb200_ctx *ctx, const jxlb200_batch_item *items, int32_t n, int32_t c, int32_t bits, int32_t out_h,
+    int32_t out_w, void *out) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!items || !out || n < 1) return ctx->fail(JXLB200_E_ARG, "NULL pointer or an empty batch");
+    if (c != 1 && c != 3 && c != 4) return ctx->fail(JXLB200_E_ARG, "c must be 1, 3 or 4");
+    if (bits != 8 && bits != 16) return ctx->fail(JXLB200_E_ARG, "bits must be 8 or 16");
+    if (out_h < 1 || out_w < 1) return ctx->fail(JXLB200_E_ARG, "slot smaller than 1 x 1");
+    const size_t bytes = bits > 8 ? 2 : 1;
+    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + (size_t)n * c * out_h * out_w * bytes;
+    for (int i = 0; i < n; i++) {
+        const jxlb200_batch_item &I = items[i];
+        if (I.orientation < 1 || I.orientation > 8) return ctx->fail(JXLB200_E_ARG, "orientation outside 1..8");
+        if (I.h < 1 || I.w < 1) return ctx->fail(JXLB200_E_ARG, "image smaller than 1 x 1");
+        const int oh = I.orientation >= 5 ? I.w : I.h, ow = I.orientation >= 5 ? I.h : I.w;
+        if (oh > out_h || ow > out_w) return ctx->fail(JXLB200_E_ARG, "oriented image larger than its slot");
+        for (int k = 0; k < c; k++) {
+            if (!I.plane[k]) continue;
+            if (I.pitch[k] < I.w) return ctx->fail(JXLB200_E_ARG, "plane pitch below the image width");
+            if (I.is_int[k] && (I.depth[k] < 1 || I.depth[k] > 31)) return ctx->fail(JXLB200_E_ARG, "bit depth outside 1..31");
+            const uintptr_t p0 = (uintptr_t)I.plane[k], p1 = p0 + 4 * ((size_t)(I.h - 1) * I.pitch[k] + I.w);
+            if (p0 < o1 && o0 < p1) return ctx->fail(JXLB200_E_ARG, "the output overlaps an input plane");
+        }
+    }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t tab = sizeof(jxlb200_batch_item) * (size_t)n;
+    CUDA_TRY(ctx, ctx->dtab.ensure(tab));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->dtab.p, items, tab, cudaMemcpyHostToDevice, ctx->stream));
+    const int px = 16 / (int)bytes;                                     // samples per thread: one 16-byte store per channel
+    const int vec = (o0 % 16) == 0 && ((size_t)out_w * bytes) % 16 == 0;
+    const dim3 block(32, 8), grid((unsigned)ceil_div(out_w, 32 * px), (unsigned)ceil_div(out_h, 8), (unsigned)std::min(n, 65535));
+    if (bits == 8) k11_pack_batch<8><<<grid, block, 0, ctx->stream>>>(ctx->dtab.as<jxlb200_batch_item>(), n, c, out_h, out_w, vec, out);
+    else k11_pack_batch<16><<<grid, block, 0, ctx->stream>>>(ctx->dtab.as<jxlb200_batch_item>(), n, c, out_h, out_w, vec, out);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
 }
 
 

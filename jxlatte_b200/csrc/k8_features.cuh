@@ -218,26 +218,34 @@ __device__ __forceinline__ int java_f2i(float v) {        // (int) cast of the J
     return (int)v;
 }
 
+// One sample of the pipeline: channel c of plane[] at i (int32 when is_int[c], else float32) -> its `bits`-bit value, clamped to
+// [0, maxv].  An int channel whose depth is `bits` is only clamped; TF_SRGB.fromLinearF comes first when `oetf` (a colour channel of
+// a linear image).  The per-channel arrays are read where the reference reads them, so k8_pack_samples keeps its instructions.
+__device__ __forceinline__ int pack_sample(const void *const *plane, const int *is_int, const int *depth, int c, long long i, int bits, int maxv,
+                                           bool oetf) {
+    int q;
+    if (is_int[c] && depth[c] == bits) {
+        q = ((const int *)plane[c])[i];
+    } else {
+        float v;
+        if (is_int[c]) v = __fmul_rn((float)((const int *)plane[c])[i], __fdiv_rn(1.0f, (float)((1 << depth[c]) - 1)));
+        else v = ((const float *)plane[c])[i];
+        if (oetf) {
+            if (v < 0.00313066844250063f) v = __fmul_rn(v, 12.92f);
+            else v = __fadd_rn(__fmul_rn(1.055f, (float)pow((double)v, 0.4166666666666667)), -0.055f);
+        }
+        q = java_f2i(__fadd_rn(__fmul_rn(v, (float)maxv), 0.5f));
+    }
+    return q < 0 ? 0 : (q > maxv ? maxv : q);
+}
+
 __global__ void k8_pack_samples(PackArgs A) {
     const long long n = (long long)A.h * A.w;
     const int maxv = (1 << A.bits) - 1, bytes = A.bits > 8 ? 2 : 1;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         unsigned char *o = A.out + i * A.n_channels * bytes;
         for (int c = 0; c < A.n_channels; c++) {
-            int q;
-            if (A.is_int[c] && A.depth[c] == A.bits) {
-                q = ((const int *)A.plane[c])[i];
-            } else {
-                float v;
-                if (A.is_int[c]) v = __fmul_rn((float)((const int *)A.plane[c])[i], __fdiv_rn(1.0f, (float)((1 << A.depth[c]) - 1)));
-                else v = ((const float *)A.plane[c])[i];
-                if (A.linear && c < A.n_color) {
-                    if (v < 0.00313066844250063f) v = __fmul_rn(v, 12.92f);
-                    else v = __fadd_rn(__fmul_rn(1.055f, (float)pow((double)v, 0.4166666666666667)), -0.055f);
-                }
-                q = java_f2i(__fadd_rn(__fmul_rn(v, (float)maxv), 0.5f));
-            }
-            q = q < 0 ? 0 : (q > maxv ? maxv : q);
+            const int q = pack_sample(A.plane, A.is_int, A.depth, c, i, A.bits, maxv, A.linear && c < A.n_color);
             if (A.layout == 1) {
                 if (bytes == 2) reinterpret_cast<unsigned short *>(A.out)[c * n + i] = (unsigned short)q;
                 else A.out[c * n + i] = (unsigned char)q;

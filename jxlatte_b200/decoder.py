@@ -17,6 +17,7 @@ The frame loop is written once.  Where it creates, copies or casts a buffer it g
 for engines that work on host arrays, the DeviceEngine itself for CUDA tensors), so the same loop runs on either.
 """
 import ctypes as C
+import os
 import struct
 import zlib
 
@@ -157,6 +158,22 @@ def preview_route(info):
     return "lf"
 
 
+def parse_stream(data, preview, threads=None):
+    """The front end of a decode: .jxl bytes -> (ParsedImage, preview route or None).  A preview parses up to the LF images
+    (frontend.FLAG_LF_ONLY) and, when preview_route() sends the stream to "full", parses it again in full.  threads: OpenMP threads
+    of the calling thread's parses (frontend.parse)."""
+    def parse(flags):
+        return frontend.parse(data, flags, threads=threads) if threads else frontend.parse(data, flags)
+    if not preview:
+        return parse(0), None
+    parsed = parse(frontend.FLAG_LF_ONLY)
+    route = preview_route(parsed.info)
+    if route == "full":
+        parsed.close()
+        parsed = parse(0)
+    return parsed, route
+
+
 class JXLOptions:
     """The reference's JXLOptions (J/JXLOptions.java:7-50), the fields that reach the reconstruction path."""
     OUTPUT_DEFAULT, OUTPUT_PNG, OUTPUT_PFM = -1, 0, 1
@@ -284,6 +301,22 @@ class CudaEngine:
 
     def pack(self, channels, depths, n_color, linear, bits):
         return self.rec.packSamples(channels, depths, n_color, linear, bits)
+
+    def pack_batch(self, items, c, bits, out_h, out_w):
+        """DeviceEngine.pack_batch's contract on host arrays -> numpy [len(items), c, out_h, out_w] uint8 / uint16.  The samples of
+        each image come from the pack kernel's host form (jxlb200_pack_samples), so both engines agree byte for byte; orientation,
+        channel expansion and placement are numpy (NumpyArrays.orient)."""
+        maxv = (1 << bits) - 1
+        out = np.zeros((len(items), c, out_h, out_w), np.uint16 if bits > 8 else np.uint8)
+        for i, (planes, depths, o, linear) in enumerate(items):
+            k = sum(p is not None for p in planes)        # the planes present come first: only a missing alpha is filled
+            raw = self.pack(planes[:k], depths[:k], min(c, 3), linear, bits)
+            samples = raw.view(">u2") if bits > 8 else raw
+            for ch in range(c):
+                a = samples[:, :, ch] if ch < k else np.full(planes[0].shape, maxv, out.dtype)
+                a = NumpyArrays.orient(a, o) if o != 1 else a
+                out[i, ch, :a.shape[0], :a.shape[1]] = a
+        return out
 
     def noise(self, planes, group_dim, seed0, lut, base_x, base_b):
         return self.rec.synthesizeNoise(planes, group_dim, seed0, lut, base_x, base_b)
@@ -475,6 +508,25 @@ class DeviceEngine(CudaEngine):
             out = torch.empty((h, w, n * (2 if bits > 8 else 1)), dtype=torch.uint8, device=self.device)
         self.rec.pack_samples_dev([c.data_ptr() for c in ch], [not self.is_float(c) for c in ch], depths, n_color, linear, h, w, bits, layout,
                                   out.data_ptr())
+        return out
+
+    def pack_batch(self, items, c, bits, out_h, out_w):
+        """Every image of a batch into one CUDA [len(items), c, out_h, out_w] uint8 / uint16 tensor, in one launch (k11_pack_batch):
+        oriented, each sample through to_int's pipeline, at the top-left of its slot, the rest of the slot 0.  items: (planes, depths,
+        orientation, linear) per image; planes: c stored-orientation 2-D tensors (repeats allowed), None for a channel filled with the
+        maximum sample value; depths: the bit depth of each."""
+        torch = self._torch
+        self._on_stream()
+        out = torch.empty((len(items), c, out_h, out_w), dtype=torch.uint16 if bits > 8 else torch.uint8, device=self.device)
+        keep, args = [], []
+        for planes, depths, o, linear in items:
+            planes = [p if p is None or p.stride(1) == 1 else p.contiguous() for p in planes]
+            keep.append(planes)
+            h, w = next(p for p in planes if p is not None).shape
+            args.append(([0 if p is None else p.data_ptr() for p in planes], [p is not None and not self.is_float(p) for p in planes],
+                         [d if p is not None else 0 for p, d in zip(planes, depths)], h, w, [w if p is None else p.stride(0) for p in planes],
+                         o, linear))
+        self.rec.pack_batch_dev(args, c, bits, out_h, out_w, out.data_ptr())
         return out
 
     # ---- compositing: the rectangles of a frame are queued and blended in one call on the device planes ----
@@ -719,6 +771,17 @@ class JXLDecoder:
         self._images = None
         self._next = None
         self._buffered = False
+        self._parsed = None                 # _from_parsed: the stream, already through the front end
+        self._batch = False
+
+    @classmethod
+    def _from_parsed(cls, parsed, route, engine, options):
+        """decode_batch's decoder: `parsed` (and, with JXLOptions(preview=True), its preview `route`) came from parse_stream.  Its
+        images are left in stored orientation (info["orientation"] still to apply) and are not synchronised: the batch's pack
+        kernel orients them, and the batch synchronises once at its end."""
+        d = cls(b"", engine, options)
+        d._parsed, d.preview_route, d._batch = parsed, route, True
+        return d
 
     def close(self):
         if self._own and self.engine is not None:
@@ -1005,16 +1068,12 @@ class JXLDecoder:
     def _compose(self):
         """Generator over the displayed images: JXLCodestreamDecoder.decode's frame loop for the features this build renders."""
         import time
-        t0 = time.perf_counter()
-        if self.options.preview:
-            parsed = frontend.parse(self.data, frontend.FLAG_LF_ONLY)
-            self.preview_route = preview_route(parsed.info)
-            if self.preview_route == "full":
-                parsed.close()
-                parsed = frontend.parse(self.data)
+        if self._parsed is None:
+            t0 = time.perf_counter()
+            parsed, self.preview_route = parse_stream(self.data, self.options.preview)
+            self.timings["front_end_s"] = time.perf_counter() - t0
         else:
-            parsed = frontend.parse(self.data)
-        self.timings["front_end_s"] = time.perf_counter() - t0
+            parsed, self._parsed = self._parsed, None
         if self.engine is None:
             self.engine = CudaEngine()
         if self.preview_route == "lf":
@@ -1022,7 +1081,7 @@ class JXLDecoder:
             return
         info = parsed.info
         xp, buf = self._xp, self._buf
-        sync = getattr(self.engine, "sync", None)
+        sync = None if self._batch else getattr(self.engine, "sync", None)
         _Buf.before_mutation = staticmethod(self._flush_blends)
         if hasattr(self.engine, "tolerance_mode"):
             self.engine.tolerance_mode = self.options.quantises_to_8_bits(info["bits_per_sample"])
@@ -1120,7 +1179,7 @@ class JXLDecoder:
                 shown, copy = canvas, not f["is_last"]
                 if self.options.preview:
                     shown, copy = self._area_mean8(canvas, info), False
-                img = self._finish(shown, info, linear, copy=copy, xp=xp, engine=self.engine if xp is not _NUMPY else None)
+                img = self._finish(shown, info, linear, copy=copy, xp=xp, engine=self.engine if xp is not _NUMPY else None, orient=not self._batch)
                 if sync is not None:
                     sync()                  # device engines: the image is complete, and stream errors surface here
                     self.timings["reconstruct_s"] = time.perf_counter() - t1
@@ -1139,7 +1198,7 @@ class JXLDecoder:
         and shown when it is the last or has a duration, as _compose shows frames."""
         import time
         info, xp, buf = parsed.info, self._xp, self._buf
-        sync = getattr(self.engine, "sync", None)
+        sync = None if self._batch else getattr(self.engine, "sync", None)
         colors = info["color_channels"]
         ih, iw = -(-info["height"] // 8), -(-info["width"] // 8)
         canvas = None
@@ -1164,7 +1223,7 @@ class JXLDecoder:
                 if sync is None:
                     self.timings["reconstruct_s"] = time.perf_counter() - t1
                 img = self._finish([buf(a) for a in canvas], info, bool(info["xyb_encoded"]), copy=not f["is_last"], xp=xp,
-                                   engine=self.engine if xp is not _NUMPY else None)
+                                   engine=self.engine if xp is not _NUMPY else None, orient=not self._batch)
                 if sync is not None:
                     sync()
                     self.timings["reconstruct_s"] = time.perf_counter() - t1
@@ -1173,8 +1232,8 @@ class JXLDecoder:
         parsed.close()
 
     @staticmethod
-    def _finish(canvas, info, linear, copy, xp=_NUMPY, engine=None):
-        o = info["orientation"]
+    def _finish(canvas, info, linear, copy, xp=_NUMPY, engine=None, orient=True):
+        o = info["orientation"] if orient else 1
         out = []
         for b in canvas:
             a = xp.copy(b.a) if copy else b.a
@@ -1182,3 +1241,185 @@ class JXLDecoder:
                 a = xp.orient(a, o)
             out.append(a)
         return JXLImage(out, info, linear, engine=engine)
+
+
+# ---- batch decode ----
+BATCH_MODES = {"rgb": 3, "rgba": 4, "grey": 1}
+
+
+class BatchResult:
+    """decode_batch's result.  images: [N, C, H, W] uint8 / uint16 (a CUDA tensor from DeviceEngine, numpy from CudaEngine);
+    sizes: [N, 2] int64 (h, w) of each image as displayed, after orientation (a CPU tensor, or numpy); routes: each file's preview
+    route ("lf" / "full") with JXLOptions(preview=True), else None for each; timings: parse_s (front-end time summed over files),
+    parse_wall_s (first parse start to last parse end), device_wall_s (first composition start to the end of the batch's
+    synchronise), total_s (the whole call)."""
+
+    def __init__(self, images, sizes, routes, timings):
+        self.images, self.sizes, self.routes, self.timings = images, sizes, routes, timings
+
+
+def _source_name(src):
+    if isinstance(src, (str, os.PathLike)):
+        return os.fspath(src)
+    if isinstance(src, (bytes, bytearray, memoryview)):
+        return "<%d bytes>" % len(src)
+    return str(getattr(src, "name", type(src).__name__))
+
+
+def _read_source(src):
+    if isinstance(src, (str, os.PathLike)):
+        with open(src, "rb") as f:
+            return f.read()
+    return bytes(src)
+
+
+def _attributed(e, i, name):
+    """e, re-raised as its own type with the source it came from in front of its message."""
+    try:
+        return type(e)("source %d (%s): %s" % (i, name, e))
+    except Exception:
+        return e
+
+
+def _slot_channels(info, mode):
+    """The image channel each output channel shows, None for one filled with the maximum sample value.  A grey image is
+    replicated into R, G and B; "rgba" takes the first alpha channel (a missing one is filled); other extra channels are dropped."""
+    ncol = info["color_channels"]
+    if mode == "grey":
+        if ncol != 1:
+            raise ValueError("mode 'grey' needs a grey image; this one has %d colour channels" % ncol)
+        return [0]
+    slots = [0, 0, 0] if ncol == 1 else [0, 1, 2]
+    if mode == "rgba":
+        slots.append(next((ncol + k for k, e in enumerate(info["extra_channels"]) if e["type"] == 0), None))
+    return slots
+
+
+def _compose_first(parsed, route, engine, options):
+    """The first displayed image of a parsed stream, composed on `engine`, in stored orientation and not synchronised."""
+    d = JXLDecoder._from_parsed(parsed, route, engine, options)
+    img = d.decode()
+    d._images.close()                   # later frames of an animation are not decoded
+    if img is None:
+        raise frontend.InvalidBitstreamError("the stream has no displayed image")
+    return img
+
+
+def decode_batch(sources, engine, *, bits=8, mode="rgb", size=None, workers=None, options=None):
+    """Decode many JPEG XL files into one [N, C, H, W] batch.
+
+    sources: paths, bytes or binary file objects (file objects are read on the calling thread, paths by the parsing threads).
+    engine: a DeviceEngine (images: a CUDA tensor) or a CudaEngine (numpy, the same bytes).  bits: 8 or 16 -> uint8 / uint16
+    samples, each through JXLImage.to_int's pipeline.  mode: "rgb", "rgba" or "grey" -> C = 3, 4 or 1 (see _slot_channels; a
+    colour image in "grey" is a ValueError: no luma formula is applied).  A missing alpha is the maximum sample value.
+    size: (H, W) of every slot; by default the largest displayed size in the batch.  Each image sits at the top-left of its slot
+    after orientation, and the rest of the slot is 0.  Nothing is resampled or cropped: an image larger than `size` is a
+    ValueError naming it.  options: a JXLOptions; preview=True gives the 1:8 previews (BatchResult.routes says which route each
+    took), and outputFormat / outputDepth keep their meaning.
+
+    Only the first displayed image of each file is decoded: a still image, or an animation's first frame.  Frames are not
+    batched across files (their quantisation tables and filters differ) and nothing is colour managed beyond to_int.
+
+    Pipelining: `workers` threads (default min(len(sources), os.cpu_count() // 2)) run the front end, each parse with
+    os.cpu_count() // workers OpenMP threads for the sections of a frame, so parsing threads times OpenMP threads stays within the
+    cores.  The calling thread composes the files in order on the engine's stream while later files parse; at most 2 * workers
+    parsed files are alive at once, and each is closed as soon as its image is composed.  All device work, one pack launch and
+    one synchronise for the batch, runs on the calling thread: composition must stay single-threaded, because _Buf.before_mutation
+    is a class-level hook that points at the composing decoder's blend queue.
+
+    A failure names the index and source it came from and fails the whole call; stream errors found at the batch's synchronise
+    name the batch.  Returns a BatchResult."""
+    import time
+    from concurrent.futures import ThreadPoolExecutor
+    t_start = time.perf_counter()
+    sources = list(sources)
+    n = len(sources)
+    if n == 0:
+        raise ValueError("decode_batch needs at least one source")
+    if bits not in (8, 16):
+        raise ValueError("bits must be 8 or 16, not %r" % (bits,))
+    if mode not in BATCH_MODES:
+        raise ValueError("mode must be one of %s, not %r" % (", ".join(BATCH_MODES), mode))
+    if size is not None and (len(size) != 2 or any(int(v) < 1 for v in size)):
+        raise ValueError("size must be (H, W) with H, W >= 1, not %r" % (size,))
+    if engine is None or not hasattr(engine, "pack_batch"):
+        raise ValueError("decode_batch needs a DeviceEngine or a CudaEngine")
+    options = options if options is not None else JXLOptions()
+    cores = os.cpu_count() or 1
+    workers = max(1, min(n, cores // 2)) if workers is None else int(workers)
+    if workers < 1:
+        raise ValueError("workers must be >= 1")
+    threads = max(1, cores // workers)
+    c = BATCH_MODES[mode]
+    names = [_source_name(s) for s in sources]
+    datas = [s if isinstance(s, (str, os.PathLike, bytes, bytearray, memoryview)) else s.read() for s in sources]
+    frontend.lib()                      # loaded (and built if need be) here, not by the parsing threads at once
+
+    def parse(i):
+        t = time.perf_counter()
+        parsed, route = parse_stream(_read_source(datas[i]), options.preview, threads)
+        return parsed, route, t, time.perf_counter()
+
+    futures = {}
+    items, sizes, routes, spans = [], [], [], []
+    t_dev = None
+    pool = ThreadPoolExecutor(workers)
+    try:
+        submitted = 0
+        for i in range(n):
+            while submitted < min(n, i + 2 * workers):
+                futures[submitted] = pool.submit(parse, submitted)
+                submitted += 1
+            try:
+                parsed, route, t0, t1 = futures.pop(i).result()
+            except Exception as e:
+                raise _attributed(e, i, names[i]) from e
+            spans.append((t0, t1))
+            try:
+                t_dev = t_dev or time.perf_counter()
+                img = _compose_first(parsed, route, engine, options)
+                slots = _slot_channels(img.info, mode)
+                o = img.info["orientation"]
+                h, w = img.height, img.width
+                shown = (w, h) if o >= 5 else (h, w)
+                if size is not None and (shown[0] > size[0] or shown[1] > size[1]):
+                    raise ValueError("image is %d x %d, larger than the batch size %d x %d" % (shown[0], shown[1], size[0], size[1]))
+            except Exception as e:
+                raise _attributed(e, i, names[i]) from e
+            finally:
+                parsed.close()
+            items.append(([None if k is None else img.channels[k] for k in slots], [None if k is None else img._depth(k) for k in slots],
+                          o, img.linear))
+            sizes.append(shown)
+            routes.append(route)
+        out_h, out_w = (int(size[0]), int(size[1])) if size is not None else tuple(max(v) for v in zip(*sizes))
+        images = engine.pack_batch(items, c, bits, out_h, out_w)
+        del items
+        sync = getattr(engine, "sync", None)
+        if sync is not None:
+            try:
+                sync()
+            except Exception as e:
+                raise _attributed(e, -1, "the batch of %d sources" % n) from e
+    except BaseException:
+        pool.shutdown(wait=True, cancel_futures=True)
+        for f in futures.values():              # parses that finished before the failure
+            if not f.cancelled() and f.exception() is None:
+                f.result()[0].close()
+        sync = getattr(engine, "sync", None)
+        if sync is not None:
+            try:
+                sync()                          # drain the batch's device work; the failure being raised is the one to report
+            except Exception:
+                pass
+        raise
+    pool.shutdown(wait=True)
+    t_end = time.perf_counter()
+    timings = dict(parse_s=sum(b - a for a, b in spans), parse_wall_s=max(b for _, b in spans) - min(a for a, _ in spans),
+                   device_wall_s=t_end - t_dev, total_s=t_end - t_start)
+    if isinstance(images, np.ndarray):
+        sizes = np.array(sizes, np.int64)
+    else:
+        import torch
+        sizes = torch.tensor(sizes, dtype=torch.int64)
+    return BatchResult(images, sizes, routes, timings)

@@ -50,6 +50,8 @@ def lib():
         L.jxlf_describe.restype = C.c_char_p
         L.jxlf_array.argtypes = [C.c_void_p, C.c_int32, C.c_char_p, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32)]
         L.jxlf_array.restype = C.c_int32
+        L.jxlf_set_threads.argtypes = [C.c_int32]
+        L.jxlf_set_threads.restype = None
         _lib = L
     return _lib
 
@@ -61,8 +63,10 @@ _DTYPES = {0: np.int32, 1: np.float32, 2: np.uint8}
 
 
 class ParsedImage:
-    def __init__(self, data, flags=0, strict=True):
+    def __init__(self, data, flags=0, strict=True, threads=None):
         L = lib()
+        if threads is not None:
+            L.jxlf_set_threads(int(threads))        # this thread's OpenMP team size for the sections of each frame
         buf = (C.c_uint8 * len(data)).from_buffer_copy(data)
         h = C.c_void_p()
         self.status = L.jxlf_decode(buf, len(data), flags, C.byref(h))
@@ -156,8 +160,10 @@ class ParsedImage:
         return [self.array(frame, "modular", i, (c["h"], c["w"])) for i, c in enumerate(m["channels"])]
 
 
-def parse(data, flags=0, strict=True):
-    return ParsedImage(data, flags, strict)
+def parse(data, flags=0, strict=True, threads=None):
+    """threads: OpenMP threads for the sections of each frame, for this and later parses on the calling thread (jxlf_set_threads);
+    None leaves the thread's setting as it is."""
+    return ParsedImage(data, flags, strict, threads)
 
 
 def parse_file(path, flags=0, strict=True):

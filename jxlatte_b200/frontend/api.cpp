@@ -6,6 +6,8 @@
 #include <cstdio>
 #include <sstream>
 
+#include <omp.h>
+
 #include "frame.hpp"
 #include "../../include/jxlfront.h"
 
@@ -245,6 +247,7 @@ int32_t jxlf_decode(const uint8_t *data, uint64_t size, int32_t flags, jxlf_imag
 }
 
 void jxlf_free(jxlf_image *im) { delete im; }
+void jxlf_set_threads(int32_t n) { if (n >= 1) omp_set_num_threads(n); }
 const char *jxlf_error(const jxlf_image *im) { return im ? im->error.c_str() : "null image"; }
 const char *jxlf_describe(const jxlf_image *im) { return im ? im->json.c_str() : "{}"; }
 

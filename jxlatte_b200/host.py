@@ -494,6 +494,17 @@ class Reconstructor:
         self._check(self._L.jxlb200_pack_samples_dev(self._h, ptrs, _ptr(ii), _ptr(dep), n, int(n_color), int(bool(linear)), int(h), int(w),
                                                      int(bits), int(layout), out))
 
+    def pack_batch_dev(self, items, c, bits, out_h, out_w, out):
+        """jxlb200_pack_batch_dev.  items: one (planes, is_int, depths, h, w, pitches, orientation, linear) per image, planes as
+        device pointers (0: filled with the maximum sample value), one entry per output channel; out: the device pointer of
+        [len(items)][c][out_h][out_w] samples."""
+        arr = (_lib.BatchItem * len(items))()
+        for it, (planes, is_int, depths, h, w, pitches, orientation, linear) in zip(arr, items):
+            for k in range(len(planes)):
+                it.plane[k], it.is_int[k], it.depth[k], it.pitch[k] = int(planes[k]) or None, int(bool(is_int[k])), int(depths[k]), int(pitches[k])
+            it.h, it.w, it.orientation, it.linear = int(h), int(w), int(orientation), int(bool(linear))
+        self._check(self._L.jxlb200_pack_batch_dev(self._h, arr, len(items), int(c), int(bits), int(out_h), int(out_w), out))
+
     def cast_to_float_dev(self, src, n, scale, out):
         self._check(self._L.jxlb200_cast_to_float_dev(self._h, src, int(n), C.c_float(float(scale)), out))
 
