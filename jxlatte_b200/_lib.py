@@ -50,6 +50,7 @@ SYMBOLS = {
     "jxlb200_host_register": (_i32, [_vp, _vp, C.c_uint64]),
     "jxlb200_host_unregister": (_i32, [_vp, _vp]),
     "jxlb200_selftest_divide": (_i32, [_vp, C.c_int64, _i32, C.POINTER(C.c_int64)]),
+    "jxlb200_stage1_plan": (_i32, [_vp, _vp, _vp]),
     "jxlb200_qm_default_params": (_i32, [C.POINTER(QmParams)]),
     "jxlb200_qm_generate": (_i32, [C.POINTER(QmParams), _vp, _vp]),
     "jxlb200_set_qm_weights": (_i32, [_vp, _vp, _vp]),

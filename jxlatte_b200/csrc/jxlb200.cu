@@ -744,6 +744,22 @@ int32_t jxlb200_selftest_divide(jxlb200_ctx *ctx, int64_t n, int32_t seed, int64
     return 0;
 }
 
+int32_t jxlb200_stage1_plan(jxlb200_ctx *ctx, int32_t counts[27], int32_t work[10]) {
+    if (!ctx) return JXLB200_E_ARG;
+    if (!counts || !work) return ctx->fail(JXLB200_E_ARG, "bad arguments");
+    if (!ctx->sched.p) return ctx->fail(JXLB200_E_ARG, "no stage-1 call has run on this context");
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    Sched h;
+    CUDA_TRY(ctx, cudaMemcpyAsync(&h, ctx->sched.p, sizeof(Sched), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    for (int t = 0; t < 27; t++) counts[t] = h.cnt[t];
+    work[0] = h.small_cum[N_SMALL];
+    work[1] = h.med_cum[N_MED];
+    for (int pass = 0; pass < 2; pass++)
+        for (int k = 0; k < N_BIGC; k++) work[2 + N_BIGC * pass + k] = h.big_cum[pass][k][3];
+    return 0;
+}
+
 int32_t jxlb200_qm_default_params(jxlb200_qm_params out[17]) {
     if (!out) return JXLB200_E_ARG;
     qm::default_params(out);

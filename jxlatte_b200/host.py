@@ -199,6 +199,14 @@ class Reconstructor:
         self._check(self._L.jxlb200_selftest_divide(self._h, int(n), int(seed), C.byref(bad)))
         return int(bad.value)
 
+    def stage1_plan(self):
+        """-> (varblocks per TransformType [27], work per stage-1 kernel {"k1_small", "k1_medium", "k1_big<N,PASS>": items}) of the
+        last stage-1 call on this context (jxlb200_stage1_plan)."""
+        counts, work = np.zeros(27, np.int32), np.zeros(10, np.int32)
+        self._check(self._L.jxlb200_stage1_plan(self._h, _ptr(counts), _ptr(work)))
+        names = ["k1_small", "k1_medium"] + ["k1_big<%d,%d>" % (32 << k, pas) for pas in (0, 1) for k in range(4)]
+        return counts, dict(zip(names, work.tolist()))
+
     def set_option(self, option, value):
         self._check(self._L.jxlb200_set_option(self._h, int(option), int(value)))
 

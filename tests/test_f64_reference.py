@@ -1,4 +1,4 @@
-"""Float64 references for the stages after stage 1, each compared with the CPU oracle (no GPU needed) and with the CUDA kernel.
+"""Float64 references for the stages after stage 1 (stage 1 itself: test_stage1_f64.py), each compared with the CPU oracle and the kernel.
 
 The oracle was written from the same reading of the Java as the kernels, so "bit-identical to the oracle" cannot catch a misreading
 the two share.  Each reference below restates one stage as mathematics -- whole-plane shifts of a mirror-padded float64 array, no
