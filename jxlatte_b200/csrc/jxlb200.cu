@@ -201,7 +201,9 @@ template <int N, int PASS> void launch_big(jxlb200_ctx *ctx, const K1Params &P, 
     if (per_sm == 0) {
         int n = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k1_big<N, PASS>, Cfg::kThreads, Cfg::kBytes) != cudaSuccess || n < 1) n = 1;
-        per_sm = min(n, 16);
+        // 32 = the SM's CTA limit; it only binds for the one-warp CTAs of the 32-line class, every other class is held
+        // lower by its threads, registers or shared memory
+        per_sm = min(n, 32);
     }
     k1_big<N, PASS><<<ctx->sms * per_sm, Cfg::kThreads, Cfg::kBytes, st>>>(P, ctx->sched.as<Sched>(), ctx->items.as<int>(), cls,
                                                                                      &ctx->sched.as<Sched>()->ticket[PASS][cls]);

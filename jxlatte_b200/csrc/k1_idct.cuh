@@ -66,62 +66,6 @@ __device__ __forceinline__ VB make_vb(const K1Params &P, int item, int type) {
     return v;
 }
 
-// dequantise + CfL the coefficient at local (ly, lx) of varblock v for the three channels (X, Y, B order).
-// Caller guarantees (ly, lx) is outside the LLF corner.
-__device__ __forceinline__ void dequant3(const K1Params &P, const VB &v, int ly, int lx, float &X, float &Y, float &B) {
-    const int py = v.by * 8 + ly, px = v.bx * 8 + lx;
-    const size_t gi = (size_t)py * P.W + px;
-    const int wi = ly * v.W + lx;
-    const int q0 = __ldg(P.q[0] + gi), q1 = __ldg(P.q[1] + gi), q2 = __ldg(P.q[2] + gi);
-    X = dequant_one(q0, P.qb[0], P.qbn, v.sfc[0], __ldg(v.w[0] + wi));
-    Y = dequant_one(q1, P.qb[1], P.qbn, v.sfc[1], __ldg(v.w[1] + wi));
-    B = dequant_one(q2, P.qb[2], P.qbn, v.sfc[2], __ldg(v.w[2] + wi));
-    // chromaFromLuma :172-188.  A tile's factor is only "cached" once the varblock covering the tile's top-left
-    // pixel has been visited (raster order of origins); before that the Java reads 0.0f from its fresh arrays.
-    const int tile = (py >> 6) * P.tw + (px >> 6);
-    float kX = 0.0f, kB = 0.0f;
-    if (__ldg(P.cfl_gate + tile) <= v.origin) {
-        kX = __fadd_rn(P.base_x, __fdiv_rn((float)__ldg(P.xfy + tile), P.color_factor));
-        kB = __fadd_rn(P.base_b, __fdiv_rn((float)__ldg(P.bfy + tile), P.color_factor));
-    }
-    X = __fadd_rn(X, __fmul_rn(kX, Y));
-    B = __fadd_rn(B, __fmul_rn(kB, Y));
-}
-
-// One LLF coefficient (ky, kx) of HFCoefficients.finalizeLLF :218-226 for a dsH x dsW corner with dsH, dsW <= 4:
-// forwardDCT2D = rows, then columns, each output * 1/N, same accumulation order; then * llfScale.
-__device__ __forceinline__ float llf_small(const float *lf, int wb, int dsH, int dsW, int ky, int kx) {
-    const int lw = ilog2_pow2(dsW), lh = ilog2_pow2(dsH);
-    const float invW = 1.0f / (float)dsW, invH = 1.0f / (float)dsH;
-    float col[4];
-    for (int y = 0; y < dsH; y++) {
-        const float *src = lf + (size_t)y * wb;
-        float d2;
-        if (kx == 0) {
-            d2 = src[0];
-            for (int n = 1; n < dsW; n++) d2 = __fadd_rn(d2, src[n]);
-        } else {
-            const float *lut = c_cos + c_cos_off[lw] + (kx - 1) * dsW;
-            d2 = __fmul_rn(src[0], lut[0]);
-            for (int n = 1; n < dsW; n++) d2 = __fadd_rn(d2, __fmul_rn(src[n], lut[n]));
-        }
-        col[y] = __fmul_rn(d2, invW);
-    }
-    float d2;
-    if (ky == 0) {
-        d2 = col[0];
-        for (int n = 1; n < dsH; n++) d2 = __fadd_rn(d2, col[n]);
-    } else {
-        const float *lut = c_cos + c_cos_off[lh] + (ky - 1) * dsH;
-        d2 = __fmul_rn(col[0], lut[0]);
-        for (int n = 1; n < dsH; n++) d2 = __fadd_rn(d2, __fmul_rn(col[n], lut[n]));
-    }
-    d2 = __fmul_rn(d2, invH);
-    // TransformType ctor :158-165: llfScale[y][x] = SCALE_F[y << (5 - yll)] * SCALE_F[x << (5 - xll)]
-    const float sc = __fmul_rn(c_llf_scale[ky << (5 - lh)], c_llf_scale[kx << (5 - lw)]);
-    return __fmul_rn(d2, sc);
-}
-
 // ------------------------------------------------------------------------------------------------------------
 // k1_small: 8x8-class
 // ------------------------------------------------------------------------------------------------------------
@@ -175,7 +119,7 @@ __global__ void __launch_bounds__(128) k1_small(K1Params P, const Sched *__restr
                     const float4 wa = __ldg(reinterpret_cast<const float4 *>(v.w[c] + y * 8)), wb4 = __ldg(reinterpret_cast<const float4 *>(v.w[c] + y * 8) + 1);
                     w[c][0] = wa.x; w[c][1] = wa.y; w[c][2] = wa.z; w[c][3] = wa.w; w[c][4] = wb4.x; w[c][5] = wb4.y; w[c][6] = wb4.z; w[c][7] = wb4.w;
                 }
-                // chromaFromLuma factors of this row's 64x64 tile (dequant3 has the story of the gate)
+                // chromaFromLuma factors of this row's 64x64 tile (MedVB has the story of the gate)
                 const int tile_i = (py >> 6) * P.tw + (px >> 6);
                 float kX = 0.0f, kB = 0.0f;
                 {
@@ -264,27 +208,131 @@ template <int N> __device__ __forceinline__ void line_idct(float *p, int stride)
     for (int i = 0; i < N; i++) p[i * stride] = v[i];
 }
 
-template <int H, int W> __device__ void medium_batch(const K1Params &P, int type, const int *it, int nvb, float *tile, VB *s_vb) {
-    constexpr int PITCH = W + 1;
-    const int tid = threadIdx.x, nt = blockDim.x;
-    if (tid < nvb) s_vb[tid] = make_vb(P, it[tid], type);
-    __syncthreads();
-    // load + dequant + CfL (x fastest -> coalesced rows of W ints)
-    for (int i = tid; i < nvb * H * W; i += nt) {
-        const int vbi = i / (H * W), r = i % (H * W);
-        const int y = r / W, x = r % W;
-        const VB &v = s_vb[vbi];
-        float X = 0.0f, Y = 0.0f, B = 0.0f;
-        if (y < H / 8 && x < W / 8) {
-            const int o = v.origin;
-            X = llf_small(P.lf[0] + o, P.wb, H / 8, W / 8, y, x);
-            Y = llf_small(P.lf[1] + o, P.wb, H / 8, W / 8, y, x);
-            B = llf_small(P.lf[2] + o, P.wb, H / 8, W / 8, y, x);
-        } else {
-            dequant3(P, v, y, x, X, Y, B);
+__host__ __device__ constexpr int cos_off(int l) { return l <= 1 ? 0 : cos_off(l - 1) + ((1 << (l - 1)) - 1) * (1 << (l - 1)); }
+
+// HFCoefficients.finalizeLLF :218-226 for the whole DH x DW corner (DH, DW <= 4) of one varblock-channel, into d (pitch floats
+// per row): forwardDCT2D = rows, then columns, each output * 1/N, in the reference's accumulation order; then * llfScale.  Every
+// table index is a compile-time constant (constant-bank operands, no divergent indexing).
+template <int DH, int DW> __device__ __forceinline__ void llf_corner(const float *lf, int wb, float *d, int pitch) {
+    constexpr int LW = DW == 1 ? 0 : DW == 2 ? 1 : 2, LH = DH == 1 ? 0 : DH == 2 ? 1 : 2;
+    const float invW = 1.0f / (float)DW, invH = 1.0f / (float)DH;
+    float col[DH][DW];
+#pragma unroll
+    for (int y = 0; y < DH; y++) {
+        float src[DW];
+#pragma unroll
+        for (int n = 0; n < DW; n++) src[n] = __ldg(lf + (size_t)y * wb + n);
+#pragma unroll
+        for (int kx = 0; kx < DW; kx++) {
+            float d2;
+            if (kx == 0) {
+                d2 = src[0];
+#pragma unroll
+                for (int n = 1; n < DW; n++) d2 = __fadd_rn(d2, src[n]);
+            } else {
+                d2 = __fmul_rn(src[0], c_cos[cos_off(LW) + (kx - 1) * DW]);
+#pragma unroll
+                for (int n = 1; n < DW; n++) d2 = __fadd_rn(d2, __fmul_rn(src[n], c_cos[cos_off(LW) + (kx - 1) * DW + n]));
+            }
+            col[y][kx] = __fmul_rn(d2, invW);
         }
-        float *d = tile + ((vbi * 3) * H + y) * PITCH + x;
-        d[0] = X; d[H * PITCH] = Y; d[2 * H * PITCH] = B;
+    }
+#pragma unroll
+    for (int ky = 0; ky < DH; ky++)
+#pragma unroll
+        for (int kx = 0; kx < DW; kx++) {
+            float d2;
+            if (ky == 0) {
+                d2 = col[0][kx];
+#pragma unroll
+                for (int n = 1; n < DH; n++) d2 = __fadd_rn(d2, col[n][kx]);
+            } else {
+                d2 = __fmul_rn(col[0][kx], c_cos[cos_off(LH) + (ky - 1) * DH]);
+#pragma unroll
+                for (int n = 1; n < DH; n++) d2 = __fadd_rn(d2, __fmul_rn(col[n][kx], c_cos[cos_off(LH) + (ky - 1) * DH + n]));
+            }
+            d2 = __fmul_rn(d2, invH);
+            // TransformType ctor :158-165: llfScale[y][x] = SCALE_F[y << (5 - yll)] * SCALE_F[x << (5 - xll)]
+            const float sc = __fmul_rn(c_llf_scale[ky << (5 - LH)], c_llf_scale[kx << (5 - LW)]);
+            d[ky * pitch + kx] = __fmul_rn(d2, sc);
+        }
+}
+
+// Per-varblock constants of a k1_medium batch, formed once per varblock: make_vb's scale and the chroma-from-luma factors
+// (HFCoefficients.chromaFromLuma :172-188) of the at most 2 x 2 tiles an 8-aligned varblock of side <= 32 touches, gate
+// applied: a tile's factor is only "cached" once the varblock covering the tile's top-left pixel has been visited (raster
+// order of origins); before that the Java reads 0.0f from its fresh arrays.
+struct MedVB {
+    int by, bx, origin;
+    float sfc[3];
+    float kx[4], kb[4];     // [2 * (tile row - first tile row) + tile column - first tile column]
+};
+
+template <int H, int W> __device__ void medium_batch(const K1Params &P, int type, const int *it, int nvb, float *tile, MedVB *s_vb) {
+    constexpr int PITCH = W + 1, R = W / 4;       // a thread's unit: a run of four coefficients of a row
+    constexpr int DH = H / 8, DW = W / 8;         // LLF corner
+    const int tid = threadIdx.x, nt = blockDim.x;
+    if (tid < 4 * nvb) {                          // four threads per varblock: tile s, and scale s < 3
+        const int vbi = tid >> 2, s = tid & 3;
+        const int item = it[vbi];
+        const int by = item >> 16, bx = item & 0xffff, origin = by * P.wb + bx;
+        MedVB &m = s_vb[vbi];
+        if (s == 0) { m.by = by; m.bx = bx; m.origin = origin; }
+        if (s < 3) m.sfc[s] = __fdiv_rn(P.sf[s], (float)P.hf_mul[origin]);
+        const int ty = ((by * 8) >> 6) + (s >> 1), tx = ((bx * 8) >> 6) + (s & 1);
+        float kX = 0.0f, kB = 0.0f;
+        if (ty <= (by * 8 + H - 1) >> 6 && tx <= (bx * 8 + W - 1) >> 6) {
+            const int t = ty * P.tw + tx;
+            if (__ldg(P.cfl_gate + t) <= origin) {
+                kX = __fadd_rn(P.base_x, __fdiv_rn((float)__ldg(P.xfy + t), P.color_factor));
+                kB = __fadd_rn(P.base_b, __fdiv_rn((float)__ldg(P.bfy + t), P.color_factor));
+            }
+        }
+        m.kx[s] = kX; m.kb[s] = kB;
+    }
+    __syncthreads();
+    // load + dequant + CfL: one run of four per thread, runs fastest along x (coalesced rows), 128-bit loads of the
+    // coefficients when P.vec holds and of the weights always (a run starts at a multiple of 4 of a weight table's row)
+    const float *wt = P.wexp + c_tab.wexp_off[type];
+    for (int i = tid; i < nvb * H * R; i += nt) {
+        const int vbi = i / (H * R), r = i % (H * R);
+        const int y = r / R, x0 = 4 * (r % R);
+        const MedVB &m = s_vb[vbi];
+        const int py = m.by * 8 + y, px = m.bx * 8 + x0;
+        const size_t gi = (size_t)py * P.W + px;
+        int q[3][4];
+        float w[3][4];
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            const int32_t *qp = P.q[c] + gi;
+            if (P.vec) {
+                const int4 a = __ldg(reinterpret_cast<const int4 *>(qp));
+                q[c][0] = a.x; q[c][1] = a.y; q[c][2] = a.z; q[c][3] = a.w;
+            } else {
+#pragma unroll
+                for (int e = 0; e < 4; e++) q[c][e] = __ldg(qp + e);
+            }
+            const float4 b = __ldg(reinterpret_cast<const float4 *>(wt + c * H * W + y * W + x0));
+            w[c][0] = b.x; w[c][1] = b.y; w[c][2] = b.z; w[c][3] = b.w;
+        }
+        const int s = 2 * ((py >> 6) - ((m.by * 8) >> 6)) + (px >> 6) - ((m.bx * 8) >> 6);
+        const float kX = m.kx[s], kB = m.kb[s];
+        float *d = tile + ((vbi * 3) * H + y) * PITCH + x0;
+#pragma unroll
+        for (int e = 0; e < 4; e++) {
+            if (y < DH && x0 + e < DW) continue;   // the LLF corner, written below
+            float X = dequant_one(q[0][e], P.qb[0], P.qbn, m.sfc[0], w[0][e]);
+            const float Y = dequant_one(q[1][e], P.qb[1], P.qbn, m.sfc[1], w[1][e]);
+            float B = dequant_one(q[2][e], P.qb[2], P.qbn, m.sfc[2], w[2][e]);
+            X = __fadd_rn(X, __fmul_rn(kX, Y));
+            B = __fadd_rn(B, __fmul_rn(kB, Y));
+            d[e] = X; d[H * PITCH + e] = Y; d[2 * H * PITCH + e] = B;
+        }
+    }
+    for (int j = tid; j < nvb * 3; j += nt) {
+        const int vbi = j / 3, c = j % 3;
+        const float *lf = c == 0 ? P.lf[0] : (c == 1 ? P.lf[1] : P.lf[2]);
+        llf_corner<DH, DW>(lf + s_vb[vbi].origin, P.wb, tile + (j * H) * PITCH, PITCH);
     }
     __syncthreads();
     // columns (length H), then rows (length W): MathHelper.inverseDCT2D :110-120
@@ -292,20 +340,29 @@ template <int H, int W> __device__ void medium_batch(const K1Params &P, int type
     __syncthreads();
     for (int l = tid; l < nvb * 3 * H; l += nt) line_idct<W>(tile + l * PITCH, 1);
     __syncthreads();
-    for (int i = tid; i < nvb * H * W; i += nt) {
-        const int vbi = i / (H * W), r = i % (H * W);
-        const int y = r / W, x = r % W;
-        const VB &v = s_vb[vbi];
-        const size_t o = (size_t)(v.by * 8 + y) * P.out_pitch + v.bx * 8 + x;
-        const float *s = tile + ((vbi * 3) * H + y) * PITCH + x;
-        P.out[0][o] = s[0]; P.out[1][o] = s[H * PITCH]; P.out[2][o] = s[2 * H * PITCH];
+    for (int i = tid; i < nvb * H * R; i += nt) {
+        const int vbi = i / (H * R), r = i % (H * R);
+        const int y = r / R, x0 = 4 * (r % R);
+        const MedVB &m = s_vb[vbi];
+        const size_t o = (size_t)(m.by * 8 + y) * P.out_pitch + m.bx * 8 + x0;
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            const float *s = tile + ((vbi * 3 + c) * H + y) * PITCH + x0;
+            float *op = P.out[c] + o;
+            if (P.vec) {
+                *reinterpret_cast<float4 *>(op) = make_float4(s[0], s[1], s[2], s[3]);
+            } else {
+#pragma unroll
+                for (int e = 0; e < 4; e++) op[e] = s[e];
+            }
+        }
     }
     __syncthreads();
 }
 
 __global__ void __launch_bounds__(256) k1_medium(K1Params P, const Sched *__restrict__ S, const int *__restrict__ items) {
     __shared__ float tile[3 * MED_COEFFS * 9 / 8];
-    __shared__ VB s_vb[MED_COEFFS / 128];
+    __shared__ MedVB s_vb[MED_COEFFS / 128];
     const int total = S->med_cum[N_MED];
     for (int b = blockIdx.x; b < total; b += gridDim.x) {
         int ti = 0;
@@ -336,12 +393,12 @@ __global__ void __launch_bounds__(256) k1_medium(K1Params P, const Sched *__rest
 // N = line length.  Both passes evaluate MathHelper.inverseDCTHorizontal's recurrence
 //   out[k] = in[0] + sum_n fl(in[n] * lut[n-1][k])   in n order,
 // forming each product once for out[k] and out[N-1-k] (the float table is exactly (anti)symmetric).
-//   PASS 0  load phase: lane = column, a warp per coefficient row (coalesced; X and B items also dequantise Y, which
-//           chroma-from-luma needs).  Walk: one column per warp, lanes = outputs k and their mirrors, over the column's
+//   PASS 0  load phase: a lane takes four adjacent columns of a row, a warp four rows per 128-bit load (X and B items also
+//           dequantise Y, which chroma-from-luma needs).  Walk: one column per warp, lanes = outputs k and their mirrors, over the column's
 //           NON-ZERO coefficients only (ballot + ffs; adding a +-0 product changes no sum and ~95 % are zero): per live n
 //           one shuffle for in[n] and one coalesced table-row read per 32 k.  Outputs replace the column in shared
-//           memory and leave as 128-byte rows.
-//   PASS 1  lane = output index k (and its mirror).  A warp owns 32 k's of 16 rows: per n one coalesced table load
+//           memory and leave as 128-bit stores, four rows per warp.
+//   PASS 1  the strip arrives by 128-bit loads.  lane = output index k (and its mirror).  A warp owns 32 k's of 16 rows: per n one coalesced table load
 //           (issued four n ahead) and four 128-bit shared-memory broadcasts of in[row][n]; results go straight to the
 //           plane, 128 bytes per row.
 // Shared memory per CTA: PASS 0  A float[N][33] + llf scratch float[32][33];  PASS 1  A float[N][36].
@@ -349,11 +406,13 @@ __global__ void __launch_bounds__(256) k1_medium(K1Params P, const Sched *__rest
 #define BIG_PITCH 33
 #define BIG_PITCH1 36
 template <int N, int PASS> struct BigCfg {
-    static constexpr int kThreads = N == 32 ? 128 : (PASS == 0 ? 2 * N : N);
+    // N = 32: one warp per CTA, which transforms its strip with RefIDCT<32> in registers; with more warps per CTA the others
+    // waited at the barrier for it (42 % of those kernels' stall samples)
+    static constexpr int kThreads = N == 32 ? 32 : (PASS == 0 ? 2 * N : N);
     static constexpr int kFloats = PASS == 0 ? N * BIG_PITCH + 32 * BIG_PITCH + N / 4 + 4 : (N == 32 ? N * BIG_PITCH : N * BIG_PITCH1);
     static constexpr int kBytes = kFloats * 4;
     // the column pass is latency-bound: resident warps matter more than registers per thread (48 warps per SM = 42 registers)
-    static constexpr int kMinBlocks = N == 32 ? 6 : (PASS == 0 ? 1536 / kThreads : (N == 64 ? 14 : 1024 / kThreads));
+    static constexpr int kMinBlocks = N == 32 ? 24 : (PASS == 0 ? 1536 / kThreads : (N == 64 ? 14 : 1024 / kThreads));
 };
 __host__ __device__ constexpr int cos_big_off(int n) { return n == 64 ? 0 : n == 128 ? 63 * 64 : 63 * 64 + 127 * 128; }
 #define COS_BIG_FLOATS (63 * 64 + 127 * 128 + 255 * 256)
@@ -396,7 +455,7 @@ __device__ __forceinline__ float dequant_ch(const K1Params &P, const VB &v, cons
     if (k.c == 1) return Y;
     const float C = dequant_one(__ldg(k.qc + gi), k.qb_c, P.qbn, k.sfc_c, __ldg(k.wc + wi));
     const int tile = (py >> 6) * P.tw + (px >> 6);
-    float f = 0.0f;   // chromaFromLuma :172-188, see dequant3
+    float f = 0.0f;   // chromaFromLuma :172-188, see MedVB
     if (__ldg(P.cfl_gate + tile) <= v.origin) f = __fadd_rn(k.base, __fdiv_rn((float)__ldg(k.fy + tile), P.color_factor));
     return __fadd_rn(C, __fmul_rn(f, Y));
 }
@@ -409,9 +468,9 @@ k1_big(K1Params P, const Sched *__restrict__ S, const int *__restrict__ items, i
     float *scr = smem + N * BIG_PITCH;   // PASS 0 only
     const int tid = threadIdx.x, nt = blockDim.x;
     const int lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
-    const int total = S->big_cum[PASS][cls][3];
     // items are handed out through a counter (zeroed with the rest of Sched before K0): a strip with an LLF corner or a dense
     // column costs several times a sparse one, and a static round-robin left the last CTAs running alone
+    const int total = S->big_cum[PASS][cls][3];
     for (;;) {
         if (tid == 0) s_wi = atomicAdd(ticket, 1);
         __syncthreads();
@@ -431,52 +490,68 @@ k1_big(K1Params P, const Sched *__restrict__ S, const int *__restrict__ items, i
         const ChanCtx kc = make_chan(P, v, c);
 
         if (PASS == 0) {
-            // rows i = 0..N-1 of 32 columns: coalesced 128-byte reads of the coefficient plane(s)
-            // in batches of four rows so that up to sixteen loads per lane are in flight (the kernel is latency-bound: a strip is
-            // only 8-32 KB); the coefficient planes are read once (streaming loads, they must not evict the cosine table from
-            // L1), and the chroma-from-luma factor is recomputed only when the lane's 64x64 tile changes
+            // rows 0..N-1 of the strip's 32 columns.  lane = (row rs of a group of four rows, columns cx..cx+3): one 128-bit
+            // streaming load per plane fetches four rows x 128 bytes per warp (X0 is a multiple of 8 and a strip offset a
+            // multiple of 32, so the four columns are 16-byte aligned when P.vec holds and never straddle a 64x64 tile).  The
+            // coefficient planes are read once (streaming: they must not evict the cosine table from L1); the weights are read
+            // only for a run with a non-zero coefficient; the chroma-from-luma factor is formed once per 64-row band.  Staging is
+            // conflict-free: bank = (rs + cx + e) mod 32.  The LLF corner is dequantised like any other run here and overwritten
+            // below, behind a barrier, before anything reads it.
             {
-                const int lx = strip * 32 + lane, px = X0 + lx;
-                int last_tile = -1;
+                constexpr int NG = N / 4;                                // groups of four rows
+                static_assert(NG % (BigCfg<N, PASS>::kThreads / 32) == 0, "row groups must tile the warps");
+                const int rs = lane >> 3, cx = 4 * (lane & 7);
+                const int lx = strip * 32 + cx, px = X0 + lx;
+                const int32_t *qy0 = kc.qy + (size_t)(Y0 + rs) * P.W + px, *qc0 = kc.qc + (size_t)(Y0 + rs) * P.W + px;
+                const float *wy0 = kc.wy + rs * v.W + lx, *wc0 = kc.wc + rs * v.W + lx;
+                int last_band = -1;
                 float f = 0.0f;
-                for (int i0 = warp; i0 < N; i0 += 4 * nwarps) {
-                    int qy[4], qc[4];
-                    float wy[4], wc[4];
-#pragma unroll
-                    for (int u = 0; u < 4; u++) {
-                        const int i = i0 + u * nwarps;
-                        qy[u] = 0; qc[u] = 0; wy[u] = 0.0f; wc[u] = 0.0f;
-                        if (i < N && !(i < v.dsH && lx < v.dsW)) {
-                            const size_t gi = (size_t)(Y0 + i) * P.W + px;
-                            const int wi = i * v.W + lx;
-                            qy[u] = __ldcs(kc.qy + gi);
-                            wy[u] = __ldg(kc.wy + wi);
-                            if (c != 1) { qc[u] = __ldcs(kc.qc + gi); wc[u] = __ldg(kc.wc + wi); }
-                        }
+                // one group per lane and iteration: holding two groups' loads in flight spilled at the 42-register cap
+                for (int g = warp; g < NG; g += nwarps) {
+                    const int i = 4 * g + rs;
+                    const size_t go = (size_t)(4 * g) * P.W;
+                    int4 qy, qc = make_int4(0, 0, 0, 0);
+                    if (P.vec) {
+                        qy = __ldcs(reinterpret_cast<const int4 *>(qy0 + go));
+                        if (c != 1) qc = __ldcs(reinterpret_cast<const int4 *>(qc0 + go));
+                    } else {
+                        qy = make_int4(__ldcs(qy0 + go), __ldcs(qy0 + go + 1), __ldcs(qy0 + go + 2), __ldcs(qy0 + go + 3));
+                        if (c != 1) qc = make_int4(__ldcs(qc0 + go), __ldcs(qc0 + go + 1), __ldcs(qc0 + go + 2), __ldcs(qc0 + go + 3));
                     }
-#pragma unroll
-                    for (int u = 0; u < 4; u++) {
-                        const int i = i0 + u * nwarps;
-                        if (i >= N) break;
-                        float val = 0.0f;
+                    {
+                        const int oy[4] = {qy.x, qy.y, qy.z, qy.w}, oc[4] = {qc.x, qc.y, qc.z, qc.w};
+                        float val[4] = {0.0f, 0.0f, 0.0f, 0.0f};
                         // both coefficients zero (most are): quant = 0, 0 * sfc * w = +0 and +0 + f * +0 = +0 whatever f's
-                        // sign; the LLF corner loaded zeros above and is filled in below.  Whole rows skip the arithmetic.
-                        if ((qy[u] | qc[u]) != 0) {
-                            const float Y = dequant_one(qy[u], kc.qb_y, P.qbn, kc.sfc_y, wy[u]);
-                            if (c == 1) {
-                                val = Y;
-                            } else {
-                                const float C = dequant_one(qc[u], kc.qb_c, P.qbn, kc.sfc_c, wc[u]);
-                                const int tile = ((Y0 + i) >> 6) * P.tw + (px >> 6);
-                                if (tile != last_tile) {      // chromaFromLuma :172-188, see dequant3 for the gate
-                                    last_tile = tile;
+                        // sign, so the weight is not needed.  Whole runs skip the arithmetic.
+                        if ((oy[0] | oy[1] | oy[2] | oy[3] | oc[0] | oc[1] | oc[2] | oc[3]) != 0) {
+                            const float4 wy4 = __ldg(reinterpret_cast<const float4 *>(wy0 + 4 * g * v.W));
+                            const float wy[4] = {wy4.x, wy4.y, wy4.z, wy4.w};
+                            float wc[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+                            if (c != 1) {
+                                const float4 wc4 = __ldg(reinterpret_cast<const float4 *>(wc0 + 4 * g * v.W));
+                                wc[0] = wc4.x; wc[1] = wc4.y; wc[2] = wc4.z; wc[3] = wc4.w;
+                                const int band = (Y0 + i) >> 6;
+                                if (band != last_band) {      // chromaFromLuma :172-188, see MedVB for the gate
+                                    last_band = band;
+                                    const int tile = band * P.tw + (px >> 6);
                                     f = 0.0f;
                                     if (__ldg(P.cfl_gate + tile) <= v.origin) f = __fadd_rn(kc.base, __fdiv_rn((float)__ldg(kc.fy + tile), P.color_factor));
                                 }
-                                val = __fadd_rn(C, __fmul_rn(f, Y));
+                            }
+#pragma unroll
+                            for (int e = 0; e < 4; e++) {
+                                if ((oy[e] | oc[e]) == 0) continue;
+                                const float Y = dequant_one(oy[e], kc.qb_y, P.qbn, kc.sfc_y, wy[e]);
+                                if (c == 1) {
+                                    val[e] = Y;
+                                } else {
+                                    const float C = dequant_one(oc[e], kc.qb_c, P.qbn, kc.sfc_c, wc[e]);
+                                    val[e] = __fadd_rn(C, __fmul_rn(f, Y));
+                                }
                             }
                         }
-                        A[i * BIG_PITCH + lane] = val;
+                        float *a = A + i * BIG_PITCH + cx;
+                        a[0] = val[0]; a[1] = val[1]; a[2] = val[2]; a[3] = val[3];
                     }
                 }
             }
@@ -519,9 +594,22 @@ k1_big(K1Params P, const Sched *__restrict__ S, const int *__restrict__ items, i
         } else {
             // 32 rows x N columns of the intermediate plane into A[n][row]
             constexpr int PT = N == 32 ? BIG_PITCH : BIG_PITCH1;
-            for (int i = tid; i < 32 * N; i += nt) {
-                const int r = i / N, x = i % N;
-                A[x * PT + r] = plane[(size_t)(Y0 + strip * 32 + r) * P.out_pitch + X0 + x];
+            if (N == 64 && P.vec) {
+                // 128-bit loads; a warp takes 16 rows x 8 columns, so that bank = (16 * (x / 4) + 4 * e + r) mod 32 (PT = 36)
+                // differs across the warp for each of the four stores.  N = 128 and 256 keep the scalar loop: their row loops sit
+                // at the 64-register cap, and with this loop beside them ptxas spilled a register (-Xptxas -v), while for N = 64
+                // this loop is what removes the spill
+                for (int w = warp; w < N / 4; w += nwarps) {
+                    const int r = 16 * (w & 1) + (lane & 15), x = 8 * (w >> 1) + 4 * (lane >> 4);
+                    const float4 t = *reinterpret_cast<const float4 *>(plane + (size_t)(Y0 + strip * 32 + r) * P.out_pitch + X0 + x);
+                    A[x * PT + r] = t.x; A[(x + 1) * PT + r] = t.y; A[(x + 2) * PT + r] = t.z; A[(x + 3) * PT + r] = t.w;
+                }
+            } else {
+                // N = 32 stays scalar: with pitch 33 a 128-bit mapping would put two lanes on each bank for every store
+                for (int i = tid; i < 32 * N; i += nt) {
+                    const int r = i / N, x = i % N;
+                    A[x * PT + r] = plane[(size_t)(Y0 + strip * 32 + r) * P.out_pitch + X0 + x];
+                }
             }
         }
         __syncthreads();
@@ -605,8 +693,17 @@ k1_big(K1Params P, const Sched *__restrict__ S, const int *__restrict__ items, i
                 }
             }
             __syncthreads();
-            for (int i = warp; i < N; i += nwarps)             // 128 bytes per row
-                plane[(size_t)(Y0 + i) * P.out_pitch + X0 + strip * 32 + lane] = A[i * BIG_PITCH + lane];
+            if (P.vec) {                                       // four rows x 128 bytes per warp, lanes as in the load phase
+                const int rs = lane >> 3, cx = 4 * (lane & 7);
+                float *o = plane + (size_t)(Y0 + rs) * P.out_pitch + X0 + strip * 32 + cx;
+                for (int g = warp; g < N / 4; g += nwarps) {
+                    const float *a = A + (4 * g + rs) * BIG_PITCH + cx;
+                    *reinterpret_cast<float4 *>(o + (size_t)(4 * g) * P.out_pitch) = make_float4(a[0], a[1], a[2], a[3]);
+                }
+            } else {
+                for (int i = warp; i < N; i += nwarps)         // 128 bytes per row
+                    plane[(size_t)(Y0 + i) * P.out_pitch + X0 + strip * 32 + lane] = A[i * BIG_PITCH + lane];
+            }
         } else {
             const float *__restrict__ lut = P.cos_big + cos_big_off(N);
             constexpr int KCH = N / 64;                 // 32-lane chunks of k in [0, N/2)
